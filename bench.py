@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W        # this repo's CUDA path
     python bench.py --impl reference ...                  # the reference's CPU path (oracle port + sklearn)
+    python bench.py ... --dump-outputs DIR                # also save the last timed step's scores and decisions
 
 Headline workload (BASELINE.json configs[3], the one the metric is quoted on): per GPU, 10 000 test utterances of 3 s @
 16 kHz int16 -> 39-d MFCC+delta+delta-delta with per-utterance CMVN (298 frames each, 2.98 M frames) -> scored against
@@ -76,6 +77,8 @@ def parse_args():
     ap.add_argument("--no-secondary", action="store_true", help="skip the configs 2 / 3 / 5 legs")
     ap.add_argument("--secondary-scale", type=float, default=1.0, help="shrink the secondary legs (smoke runs)")
     ap.add_argument("--oracle-utts", type=int, default=32, help="utterances of the float64 CPU check (0 = skip)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the timed path returned in its last step to DIR/*.npy, to compare two builds")
     ap.add_argument("--oracle-check", default=None, help=argparse.SUPPRESS)   # internal: npz path -> float64 scores
     ap.add_argument("--cpu-legs", default=None, help=argparse.SUPPRESS)       # internal: CPU baselines of the secondary legs
     return ap.parse_args()
@@ -515,6 +518,23 @@ def oracle_check(b: Bench, pcm_dev, fe, gpu_scores, w, var, means, n_check):
     return out
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path, scores, decisions):
+    """--dump-outputs: the last timed step's per-utterance scores against every model (UBM last) and its LLR-argmax
+    decisions, as float64 .npy files.  Where the scores exceed DUMP_BYTES, a fixed, seeded sample of utterances is kept;
+    scores_rows.npy lists which."""
+    os.makedirs(path, exist_ok=True)
+    n, m = scores.shape
+    dec = decisions.cpu().numpy().astype(np.float64)
+    fit = (DUMP_BYTES - dec.nbytes) // (8 * (m + 1))   # a score row plus its index
+    rows = np.arange(n) if fit >= n else np.sort(np.random.RandomState(0).choice(n, fit, replace=False))
+    np.save(os.path.join(path, "decisions.npy"), dec)
+    np.save(os.path.join(path, "scores.npy"), scores.cpu().numpy()[rows])
+    np.save(os.path.join(path, "scores_rows.npy"), rows.astype(np.float64))
+
+
 # ---------------------------------------------------------------------------------------------- secondary legs
 def leg_config2(b: Bench, scale):
     """BASELINE configs[1]: MFCC+delta+delta-delta (39-d, CMVN) over 100 000 x 3 s utterances, sharded over the ranks."""
@@ -754,6 +774,8 @@ def run_b200(a):
             check.update(oracle_check(b, pcm, fe, gpu_scores, w, var, means, min(a.oracle_utts, N)))
         except Exception as e:
             check["oracle_error"] = f"{e!r}"[:300]
+    if rank == 0 and a.dump_outputs:
+        dump_outputs(a.dump_outputs, gpu_scores, dec)
     del gpu_scores
     keep.clear()
 

@@ -93,6 +93,20 @@ def test_scale_matches_sklearn(golden):
     assert np.all(got[:, 3] == 0)  # constant column: std 0 -> divisor 1
 
 
+def pipeline_train_audio(g):
+    """The training half of pipeline.npz's corpus, regenerated from the seeds the fixture was made with and split the way
+    GMM_UBM.py:125 does; the fixture holds its CRC instead of 0.7 MB of PCM."""
+    import zlib
+
+    from sklearn.model_selection import train_test_split
+
+    x, y = synth.synth_corpus(4, 8, 16000)
+    x_tr, _, y_tr, _ = train_test_split(x, y, test_size=0.3, random_state=0)
+    assert zlib.crc32(np.stack(x_tr).tobytes()) == int(g["x_train_crc"]), "synthetic audio differs from the fixture's"
+    assert list(y_tr) == list(g["y_train"])
+    return x_tr
+
+
 def test_extract_feature_matches_reference_pipeline(golden):
     """GMM_UBM.extract_feature (run unmodified with the sidekit restatement as mfcc) vs ONE launch."""
     g = golden("pipeline.npz")
@@ -102,7 +116,7 @@ def test_extract_feature_matches_reference_pipeline(golden):
     for j in range(len(x)):
         assert feature[j].shape == (98, 26)
         np.testing.assert_allclose(feature[j], g["feat_test"][j], atol=2e-4)
-    train, feature, y = ssp.extract_feature(list(g["x_train"]), list(g["y_train"]), is_train=True)
+    train, feature, y = ssp.extract_feature(pipeline_train_audio(g), list(g["y_train"]), is_train=True)
     assert sorted(train) == sorted(set(g["y_train"].tolist()))
     lab0 = int(g["y_train"][0])
     np.testing.assert_allclose(train[lab0][:98], g["feat_train0"], atol=2e-4)

@@ -295,6 +295,30 @@ def test_counter_based_audio_is_a_pure_function_of_its_ids():
     assert torch.equal(pcm.reshape(3, 2000), synth.synth_pcm_torch(spk[:3], utt[:3], 2000, "cpu"))
 
 
+def test_bench_dump_outputs_keeps_to_its_budget(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float64 files, every decision, all score rows when they fit and otherwise the same seeded
+    sample of rows on every run."""
+    import torch
+
+    sys.path.insert(0, ROOT)
+    import bench
+
+    scores = torch.randn((40, 11), dtype=torch.float64)
+    dec = torch.arange(40) % 10
+    bench.dump_outputs(str(tmp_path / "all"), scores, dec)
+    load = lambda d, name: np.load(str(tmp_path / d / f"{name}.npy"))  # noqa: E731
+    assert all(load("all", f).dtype == np.float64 for f in ("scores", "decisions", "scores_rows"))
+    assert np.array_equal(load("all", "scores"), scores.numpy()) and np.array_equal(load("all", "decisions"), dec.numpy())
+    assert np.array_equal(load("all", "scores_rows"), np.arange(40))
+    monkeypatch.setattr(bench, "DUMP_BYTES", 2000)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), scores, dec)
+    rows = load("a", "scores_rows").astype(np.int64)
+    assert 0 < len(rows) < 40 and (np.diff(rows) > 0).all() and np.array_equal(rows, load("b", "scores_rows"))
+    assert np.array_equal(load("a", "scores"), scores.numpy()[rows]) and len(load("a", "decisions")) == 40
+    assert sum(load("a", f).nbytes for f in ("scores", "decisions", "scores_rows")) <= 2000
+
+
 # ------------------------------------------------------------------------------------------------
 # batched WAV ingest (wavio.py) against scipy.io.wavfile.read, the reader the reference uses (utils/tools.py:45-47)
 # ------------------------------------------------------------------------------------------------
