@@ -290,6 +290,36 @@ int ssp_gmm_map_adapt(const double* n, const double* f, const double* s, const i
                       int32_t flags, double* out_weights, double* out_means, double* out_variances,
                       void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Dynamic time warping: the template-matching stage of the MFCC+DTW recogniser (MFCC_DTW.py, dtw 1.4
+ * `accelerated_dtw`).  Symmetric step pattern, no window, no slope weights, no normalisation:
+ *   D[i,j] = C[i,j] + min(D[i-1,j-1], D[i-1,j], D[i,j-1]),  D[-1,-1] = 0, the rest of row / column -1 = +inf,
+ *   distance = D[n-1, m-1];  C = scipy cdist(x, y, metric), computed in FP32 in difference form.
+ * The distance is exactly symmetric in its two arguments; the "column" side (r, y) is staged in shared memory and
+ * bounds the length (ssp_dtw_max_len), the "row" side is unbounded.
+ * ---------------------------------------------------------------------------------------- */
+#define SSP_DTW_EUCLIDEAN 0   /* sqrt(sum (x - y)^2) */
+#define SSP_DTW_SQEUCLIDEAN 1 /* sum (x - y)^2       */
+#define SSP_DTW_CITYBLOCK 2   /* sum |x - y|         */
+
+/* Longest column-side sequence (frames) the kernels accept at this feature width; 0 if dim is outside [1, 64]. */
+int64_t ssp_dtw_max_len(int32_t dim);
+/*
+ * out_dist[a * n_r + b] = DTW distance of q sequence a and r sequence b, every pair in one launch (dtw_kernel).
+ * q, r           device float[total frames * dim], sequences back to back
+ * q_offsets      device int64[n_q + 1]; r_offsets device int64[n_r + 1] (every sequence at least one frame)
+ * max_r_len      host: longest r sequence (sizes the shared memory; <= ssp_dtw_max_len(dim), else SSP_EUNSUP)
+ * out_dist       device float[n_q * n_r]
+ */
+int ssp_dtw_batch(const float* q, const int64_t* q_offsets, int64_t n_q, const float* r, const int64_t* r_offsets,
+                  int64_t n_r, int32_t dim, int32_t metric, int64_t max_r_len, float* out_dist, void* stream);
+/*
+ * One pair with its matrices (dtw_full_kernel): out_cost = C, out_acc = D, both device float[n_x * n_y] row-major.
+ * n_y <= ssp_dtw_max_len(dim), else SSP_EUNSUP.
+ */
+int ssp_dtw_full(const float* x, int64_t n_x, const float* y, int64_t n_y, int32_t dim, int32_t metric,
+                 float* out_cost, float* out_acc, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -73,6 +73,9 @@ PROTOTYPES = {
     "ssp_gmm_stats_workspace_bytes": (_I64, [C.POINTER(GmmDims), _I64, _I64]),
     "ssp_gmm_mstep": (C.c_int, [_P, _P, _P, _I32, _I32, _I32, C.c_double, C.c_double, _P, _P, _P, _P]),
     "ssp_gmm_map_adapt": (C.c_int, [_P, _P, _P, _P, _I64, _P, _P, _P, _I32, _I32, C.c_double, _I32, _P, _P, _P, _P]),
+    "ssp_dtw_max_len": (_I64, [_I32]),
+    "ssp_dtw_batch": (C.c_int, [_P, _P, _I64, _P, _P, _I64, _I32, _I32, _I64, _P, _P]),
+    "ssp_dtw_full": (C.c_int, [_P, _I64, _P, _I64, _I32, _I32, _P, _P, _P]),
 }
 
 _lib = None
