@@ -296,7 +296,8 @@ int ssp_gmm_map_adapt(const double* n, const double* f, const double* s, const i
  *   D[i,j] = C[i,j] + min(D[i-1,j-1], D[i-1,j], D[i,j-1]),  D[-1,-1] = 0, the rest of row / column -1 = +inf,
  *   distance = D[n-1, m-1];  C = scipy cdist(x, y, metric), computed in FP32 in difference form.
  * The distance is exactly symmetric in its two arguments; the "column" side (r, y) is staged in shared memory and
- * bounds the length (ssp_dtw_max_len), the "row" side is unbounded.
+ * bounds the length (ssp_dtw_max_len), the "row" side takes sequences of up to INT32_MAX / 2 frames (a pair with a
+ * longer one comes out NaN).
  * ---------------------------------------------------------------------------------------- */
 #define SSP_DTW_EUCLIDEAN 0   /* sqrt(sum (x - y)^2) */
 #define SSP_DTW_SQEUCLIDEAN 1 /* sum (x - y)^2       */

@@ -88,41 +88,45 @@ __global__ void __launch_bounds__(kWarps * 32) dtw_kernel(const Args a) {
 #pragma unroll
     for (int k = 0; k < DB; ++k) xr[k] = (k < a.dim && i < n) ? x[(int64_t)i * a.dim + k] : 0.f;
     float recv = INF, diag = INF, left = INF;
-    const int steps = ((n + 31) >> 5) * M + 31;
-    for (int t = 0; t < steps; ++t) {
-      const bool col_ok = j >= 0 && j < m;
-      float up = recv;
-      if (lane == 0) up = (col_ok && i >= 32 && i < n) ? rb[j] : INF;
-      float cur = INF;
-      if (col_ok && i < n) {
-        const float* yj = ys + j * S;
-        float s = 0.f;
+    // ceil(n / 32) * M + 31 steps can exceed INT32_MAX (a row of 10 644 257 frames against 6 456): they run in chunks of
+    // at most 2^30, each counted in 32 bits (one chunk for any realistic pair, and the same inner loop as one count)
+    for (int64_t remaining = (int64_t)((n + 31) >> 5) * M + 31; remaining > 0; remaining -= 1 << 30) {
+      const int steps = remaining < (1 << 30) ? (int)remaining : 1 << 30;
+      for (int t = 0; t < steps; ++t) {
+        const bool col_ok = j >= 0 && j < m;
+        float up = recv;
+        if (lane == 0) up = (col_ok && i >= 32 && i < n) ? rb[j] : INF;
+        float cur = INF;
+        if (col_ok && i < n) {
+          const float* yj = ys + j * S;
+          float s = 0.f;
 #pragma unroll
-        for (int k = 0; k < DB; ++k) {
-          const float d = xr[k] - yj[k];
-          s = ABS ? s + fabsf(d) : fmaf(d, d, s);
+          for (int k = 0; k < DB; ++k) {
+            const float d = xr[k] - yj[k];
+            s = ABS ? s + fabsf(d) : fmaf(d, d, s);
+          }
+          if (a.root) s = sqrtf(s);
+          const float dg = j == 0 ? (i == 0 ? 0.f : INF) : diag;
+          const float lf = j == 0 ? INF : left;
+          cur = s + fminf(dg, fminf(up, lf));
+          if (FULL) {
+            a.cost[(int64_t)i * m + j] = s;
+            a.acc[(int64_t)i * m + j] = cur;
+          } else if (i == n - 1 && j == m - 1) {
+            a.out[q * a.n_cols + c] = cur;
+          }
+          if (lane == 31) rb[j] = cur;
         }
-        if (a.root) s = sqrtf(s);
-        const float dg = j == 0 ? (i == 0 ? 0.f : INF) : diag;
-        const float lf = j == 0 ? INF : left;
-        cur = s + fminf(dg, fminf(up, lf));
-        if (FULL) {
-          a.cost[(int64_t)i * m + j] = s;
-          a.acc[(int64_t)i * m + j] = cur;
-        } else if (i == n - 1 && j == m - 1) {
-          a.out[q * a.n_cols + c] = cur;
-        }
-        if (lane == 31) rb[j] = cur;
-      }
-      left = cur;
-      diag = up;
-      __syncwarp();  // orders lane 31's row-buffer store before lane 0's load of it (M >= 32 steps later, or the next)
-      recv = __shfl_up_sync(0xffffffffu, cur, 1);
-      if (++j == M) {
-        j = 0;
-        i += 32;
+        left = cur;
+        diag = up;
+        __syncwarp();  // orders lane 31's row-buffer store before lane 0's load of it (M >= 32 steps later, or the next)
+        recv = __shfl_up_sync(0xffffffffu, cur, 1);
+        if (++j == M) {
+          j = 0;
+          i += 32;
 #pragma unroll
-        for (int k = 0; k < DB; ++k) xr[k] = (k < a.dim && i < n) ? x[(int64_t)i * a.dim + k] : 0.f;
+          for (int k = 0; k < DB; ++k) xr[k] = (k < a.dim && i < n) ? x[(int64_t)i * a.dim + k] : 0.f;
+        }
       }
     }
     __syncwarp();
