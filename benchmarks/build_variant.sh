@@ -1,5 +1,6 @@
-# Build an A/B variant of the library: benchmarks/bin/libssp_NAME.so with extra -D flags on every source.
-#   bash benchmarks/build_variant.sh NAME -DSSP_SV_STAGES=5 ...
+# Build an A/B variant of the library: benchmarks/bin/libssp_NAME.so from the sources of the tree this script is in (further
+# arguments are passed to every nvcc call).  Edit a constant in a copy of the tree, build it there and point SSP_B200_LIB at it:
+#   bash COPY/benchmarks/build_variant.sh NAME && SSP_B200_LIB=COPY/benchmarks/bin/libssp_NAME.so python bench.py ...
 set -e
 cd "$(dirname "$0")/.."
 name=$1; shift

@@ -45,7 +45,7 @@ def timed(fn, steps=3, warmup=2):
 ms_sv, (a, _) = timed(lambda: sms.score(feats, offs))
 flop = 4.0 * d * k * n_utts * t * (n_spk + 1)
 res = {"n_utts": n_utts, "n_models": n_spk + 1, "K": k, "sv_ms": ms_sv, "sv_algorithmic_tflops": flop / ms_sv / 1e9,
-       "sv_frames_per_s": n_utts * t / ms_sv * 1e3, "poly": os.environ.get("SSP_SV_POLY_PAIRS"), "deg": os.environ.get("SSP_SV_POLY_DEG")}
+       "sv_frames_per_s": n_utts * t / ms_sv * 1e3}
 if general:
     gms = sms.expand()
     ms_g, (b, _) = timed(lambda: gms.score(feats, offs, precision="tf32"))

@@ -123,17 +123,6 @@ extern "C" int ssp_gmm_score_shared(const float* feats, const int64_t* frame_off
                               (cudaStream_t)stream);
 }
 
-// The tensor-core kernels serve every feature width they support (D <= 39); the FP32 CUDA-core kernels are the
-// documented path for wider features only (and SSP_STATS_IMPL=simt, an explicit A/B switch).
-static bool stats_want_tc(const ssp::PackLayout& L) {
-  static int impl = -1;
-  if (impl < 0) {
-    const char* e = getenv("SSP_STATS_IMPL");
-    impl = (e && strcmp(e, "simt") == 0) ? 0 : 1;
-  }
-  return impl == 1 && ssp::stats_tc_supported(L);
-}
-
 extern "C" int64_t ssp_gmm_stats_workspace_bytes(const ssp_gmm_dims* dims, int64_t total_frames, int64_t n_segs) {
   ssp::PackLayout L;
   if (!ssp::make_layout(dims, &L) || total_frames < 0 || n_segs < 0) return 0;
@@ -153,7 +142,9 @@ extern "C" int ssp_gmm_stats(const float* feats, const int64_t* seg_offsets, int
   SSP_REQUIRE(n_segs >= 0 && total_frames >= 0, "ssp_gmm_stats: negative size");
   if (n_segs == 0) return SSP_OK;
   cudaStream_t st = (cudaStream_t)stream;
-  if (stats_want_tc(L)) {
+  // The tensor-core kernels serve every feature width they support (D <= 39); the FP32 CUDA-core kernels serve wider
+  // features only.
+  if (ssp::stats_tc_supported(L)) {
     // no silent 10x slower path: a short workspace is the caller's error
     const int64_t need = ssp::stats_tc_workspace_bytes(L, total_frames, n_segs);
     SSP_REQUIRE(need == 0 || (workspace && workspace_bytes >= need),

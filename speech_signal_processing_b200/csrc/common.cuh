@@ -74,10 +74,7 @@ constexpr int kSvMaxKS = 64;
 constexpr int kSvBaseImages = 4;
 constexpr float kSvConstScale = 1024.f;  // second "one" column of the per-model frame operand (range of the model constants)
 // shape of gmm_score_sv_kernel (here because it bounds the feature width the layout accepts)
-#ifndef SSP_SV_STAGES
-#define SSP_SV_STAGES 12
-#endif
-constexpr int kSvStages = SSP_SV_STAGES, kSvSlots = 6, kSvChunk = 32, kSvUnit = 256;
+constexpr int kSvStages = 12, kSvSlots = 6, kSvChunk = 32, kSvUnit = 256;
 constexpr size_t kMaxDynSmem = 232448;  // 227 KB per CTA on sm_100
 constexpr int kSvMaxFeat = 39;          // widest feature vector whose operands fit (sv_smem_bytes)
 struct SvLayout {

@@ -19,19 +19,16 @@
 //     geometry and conventions are compile-time constants, the window, the real-FFT twiddles and the DCT rows live in
 //     registers, samples are read as aligned 8-byte pairs (round 1: 4-byte loads at stride 2 floats, the bulk of the
 //     26 % bank-conflict wavefronts), the DCT runs two lanes per cepstrum, and log is lg2.approx * ln 2 (|error| ~1e-6).
-#include <cstdlib>
 #include <type_traits>
 
 #include "frontend_common.cuh"
 
 namespace ssp {
 
-#ifndef SSP_FE_MIN_CTAS
-#define SSP_FE_MIN_CTAS 2  // CTAs per SM the register allocation aims at.  3 (<= 85 registers: 80 + 292 bytes of spills, and no
-                           // materialised deltas to fit the shared memory) measured 108.6 ms at config 2 against 33.2 ms
-#endif
-
 namespace ff {
+// CTAs per SM the register allocation aims at.  3 (<= 85 registers: 80 + 292 bytes of spills, and no materialised deltas
+// to fit the shared memory) measured 108.6 ms at config 2 against 33.2 ms
+constexpr int kMinCtas = 2;
 constexpr int W = 8;          // warps per CTA == frames per batch
 constexpr int NH = 256;       // complex FFT length
 constexpr int EXS = 36;       // float2 row stride of the transpose buffer (conflict-free for 64-bit accesses)
@@ -86,8 +83,8 @@ __host__ __device__ inline size_t carve_floats(const ssp_frontend_cfg& c, int ma
 constexpr int SK_FL = 400, SK_SH = 160, SK_NF = 24, SK_NC = 13;
 
 template <typename PcmT, bool kSk>
-__global__ void __launch_bounds__(256, SSP_FE_MIN_CTAS) frontend512_kernel(const FrontendArgs a, const int flags, const int64_t n_utts) {
-  const int materialize = flags & 1;  // bit 1: never take the direct-load path (A/B knob SSP_FE_STAGED)
+__global__ void __launch_bounds__(256, kMinCtas) frontend512_kernel(const FrontendArgs a, const int flags, const int64_t n_utts) {
+  const int materialize = flags & 1;  // bit 0: delta / delta-delta are materialised in shared memory
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const ssp_frontend_cfg& cfg = a.cfg;
   const int NC = kSk ? SK_NC : cfg.n_ceps, NF = kSk ? SK_NF : cfg.n_filt, FL = kSk ? SK_FL : cfg.frame_len,
@@ -403,7 +400,7 @@ __global__ void __launch_bounds__(256, SSP_FE_MIN_CTAS) frontend512_kernel(const
   // (a sample is read by the 2.5 frames that cover it, from L1 after the first), the sample before a pair comes from the
   // neighbouring lane by shuffle, and the loads of the warp's NEXT frame are in flight while this one is transformed.  The
   // warps of a CTA run decoupled until the delta / CMVN phase.
-  const bool direct = kSk && sizeof(PcmT) == 2 && ((reinterpret_cast<uintptr_t>(a.pcm) & 3) == 0) && !(flags & 2);
+  const bool direct = kSk && sizeof(PcmT) == 2 && ((reinterpret_cast<uintptr_t>(a.pcm) & 3) == 0);
   if (direct) {
     // an utterance that starts on an odd sample reads the pairs one sample earlier: word = (x[i - 1], x[i]), x[i + 1] comes
     // from the lane above
@@ -661,13 +658,7 @@ size_t frontend_fast_smem(const ssp_frontend_cfg& c, int max_frames, bool mat) {
 int launch_frontend_fast(const FrontendArgs& a, int64_t n_utts, size_t* smem_out, cudaStream_t st) {
   // materialise delta / delta-delta when that still leaves room for two CTAs per SM
   const size_t with = frontend_fast_smem(a.cfg, a.max_frames, true);
-  static int force = -2;
-  if (force == -2) {
-    const char* e = getenv("SSP_FE_MATERIALIZE");  // tuning knob: 0 / 1 force, unset = heuristic
-    force = e ? atoi(e) : -1;
-  }
-  bool mat = a.cfg.delta_order > 0 && with <= 110 * 1024;
-  if (force >= 0) mat = force != 0 && a.cfg.delta_order > 0 && with <= 220 * 1024;
+  const bool mat = a.cfg.delta_order > 0 && with <= 110 * 1024;
   const size_t smem = mat ? with : frontend_fast_smem(a.cfg, a.max_frames, false);
   if (smem_out) *smem_out = smem;
   // persistent CTAs: the per-CTA tables (twiddles, filterbank segments) are built once and amortised over the utterances
@@ -680,23 +671,13 @@ int launch_frontend_fast(const FrontendArgs& a, int64_t n_utts, size_t* smem_out
   }
   const unsigned grid = (unsigned)(n_utts < 16 * (int64_t)sms ? n_utts : 16 * (int64_t)sms);
   const ssp_frontend_cfg& c = a.cfg;
-  static int staged = -1;
-  if (staged < 0) {
-    const char* e = getenv("SSP_FE_STAGED");  // A/B knob: 1 = stage the samples of 8 frames in shared memory (round-1 scheme)
-    staged = e ? atoi(e) : 0;
-  }
-  static int no_sk = -1;
-  if (no_sk < 0) {
-    const char* e = getenv("SSP_FE_GENERIC");  // A/B knob: 1 = never take the compile-time specialisation
-    no_sk = e ? atoi(e) : 0;
-  }
-  const bool sk = !no_sk && c.frame_len == ff::SK_FL && c.frame_shift == ff::SK_SH && c.n_filt == ff::SK_NF && c.n_ceps == ff::SK_NC &&
+  const bool sk = c.frame_len == ff::SK_FL && c.frame_shift == ff::SK_SH && c.n_filt == ff::SK_NF && c.n_ceps == ff::SK_NC &&
                   c.framing == 0 && c.preemph_mode == 1 && c.spec_type == 0 && c.spec_scale == 1.0f && c.log_type == 0 &&
                   c.log_add == 0.0f && c.log_zero_floor == 0.0f && c.energy_mode <= 1;
 #define SSP_FE_LAUNCH(T, SK)                                                                                              \
   do {                                                                                                                    \
     SSP_CUDA_OK(cudaFuncSetAttribute(ff::frontend512_kernel<T, SK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    ff::frontend512_kernel<T, SK><<<grid, 256, smem, st>>>(a, (mat ? 1 : 0) | (staged ? 2 : 0), n_utts);                 \
+    ff::frontend512_kernel<T, SK><<<grid, 256, smem, st>>>(a, mat ? 1 : 0, n_utts);                                       \
   } while (0)
   if (c.pcm_dtype == 0) {
     if (sk) SSP_FE_LAUNCH(int16_t, true); else SSP_FE_LAUNCH(int16_t, false);

@@ -32,8 +32,6 @@
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
-#include <cstdlib>
-
 #include "tc_common.cuh"
 
 namespace ssp {
@@ -143,17 +141,20 @@ __device__ __forceinline__ void tc_ld8(uint32_t taddr, uint32_t (&r)[8]) {
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
-// sum over 32 accumulator columns of 2^(r - cm); kPoly of the 16 column pairs on the FMA pipe (degree-4 minimax
+// share of the LSE pass's exponentials on the FMA pipe (pairs of 16), measured at config 3 (36 M frames, K = 512):
+// 2 / 4 / 6 / 8 pairs -> 30.0 / 27.8 / 26.3 / 27.3 ms per call
+constexpr int kPolyPairs = 6;
+
+// sum over 32 accumulator columns of 2^(r - cm); kPolyPairs of the 16 column pairs on the FMA pipe (degree-4 minimax
 // polynomial after a magic-number range reduction, 2.7e-6 relative), the rest MUFU ex2 (see gmm_score_sv.cu)
-template <int kPoly>
 __device__ __forceinline__ float exp_sum32(const uint32_t (&r)[32], float cm) {
-  static_assert(kPoly % 2 == 0 && kPoly <= 16, "pairs are consumed two at a time");
+  static_assert(kPolyPairs % 2 == 0 && kPolyPairs <= 16, "pairs are consumed two at a time");
   const float MAGIC = 12582912.f;  // 1.5 * 2^23
   const float2 mg = make_float2(MAGIC, MAGIC), nmg = make_float2(-MAGIC, -MAGIC), neg1 = make_float2(-1.f, -1.f);
   const float2 ncm = make_float2(-cm, -cm);
   float2 accp = make_float2(0.f, 0.f), accm0 = accp, accm1 = accp;
 #pragma unroll
-  for (int i = 0; i < kPoly; ++i) {
+  for (int i = 0; i < kPolyPairs; ++i) {
     float2 d = __fadd2_rn(make_float2(__uint_as_float(r[2 * i]), __uint_as_float(r[2 * i + 1])), ncm);
     d.x = fmaxf(d.x, -126.f);
     d.y = fmaxf(d.y, -126.f);
@@ -170,7 +171,7 @@ __device__ __forceinline__ float exp_sum32(const uint32_t (&r)[32], float cm) {
     accp = __fadd2_rn(accp, e);
   }
 #pragma unroll
-  for (int i = kPoly; i < 16; i += 2) {
+  for (int i = kPolyPairs; i < 16; i += 2) {
     const float2 d0 = __fadd2_rn(make_float2(__uint_as_float(r[2 * i]), __uint_as_float(r[2 * i + 1])), ncm);
     const float2 d1 = __fadd2_rn(make_float2(__uint_as_float(r[2 * i + 2]), __uint_as_float(r[2 * i + 3])), ncm);
     accm0 = __fadd2_rn(accm0, make_float2(ex2(d0.x), ex2(d0.y)));
@@ -287,7 +288,6 @@ __global__ void __launch_bounds__(256) em_prep_kernel(const Args a) {
 // ================================================================================================ pass LSE
 // grid = (image chunks, tile pairs).  Shared memory: the pair's model tiles (BF16 hi + lo) + NS_L Fb stages; tensor
 // memory: 2 tiles x 2 buffers of 128 accumulator columns.
-template <int kPoly>
 __global__ void __launch_bounds__(THREADS, 1) gmm_em_lse_kernel(const Args a) {
   extern __shared__ __align__(1024) unsigned char smem[];
   const int KDb = a.KDb;
@@ -409,7 +409,7 @@ __global__ void __launch_bounds__(THREADS, 1) gmm_em_lse_kernel(const Args a) {
 #pragma unroll
         for (int e = 1; e < 31; e += 2) cm = max3(cm, __uint_as_float(rb[e]), __uint_as_float(rb[e + 1]));
         cm = fmaxf(cm, __uint_as_float(rb[31]));
-        const float s = exp_sum32<kPoly>(ra, cm) + exp_sum32<kPoly>(rb, cm);
+        const float s = exp_sum32(ra, cm) + exp_sum32(rb, cm);
         dst[i * IMG] = make_float2(cm, s);
       }
     }
@@ -478,19 +478,10 @@ __global__ void __launch_bounds__(256) em_merge_kernel(const Args a) {
 // GEMM2(k - 1) (statistics); both rings are released by the completion of GEMM2(k), so the loads of step k + 1 are
 // issued two GEMMs before they are needed.
 namespace p3 {
-#ifndef SSP_EM_XT_LO
-#define SSP_EM_XT_LO 1  // 1: the statistics GEMM also multiplies the residual (lo) FP16 piece of the frames.  0 (A/B builds) saves 4 of
-                        // 23 MMAs per step (19.7 vs 21.0 ms per call at config 3) but the 11-bit x and x^2 cancel in S/N - mean^2:
-                        // variances off by up to 60 % in test_em_trajectory_matches_sklearn
-#endif
-#ifndef SSP_EM_NF
-#define SSP_EM_NF 3
-#define SSP_EM_NX 4
-#endif
 // ring depths, measured at config 3 (ms per statistics call, three runs each on one box; single runs scatter by up to 5 ms):
 // (NF, NX) = (3, 2) 21.6 / 21.6 / 22.6, (4, 3) 21.5 / 21.3 / 21.1, (3, 4) 21.0 / 20.8 -- the FP16 Xt images freed the shared
 // memory for the deeper Xt ring
-constexpr int NF = SSP_EM_NF, NX = SSP_EM_NX;
+constexpr int NF = 3, NX = 4;
 constexpr uint32_t COL_LOGIT = 0;    // + 64 * (2 * tile + buffer)
 constexpr uint32_t COL_STAT = 256;   // + KDb * tile
 constexpr int CTRL = 96;             // warp 0: producer; warps 1, 2: MMA issuers of tile 0 / tile 1 (a step's MMAs are 32-40
@@ -614,11 +605,12 @@ __global__ void __launch_bounds__(p3::THREADS_S, 1) gmm_em_stats_kernel(const Ar
 #pragma unroll
           for (int q = 0; q < BLK / 16; ++q)
             mma_f16_ts(t_stat, t_gam + 32u * (q >> 1) + 8u * (q & 1), xhi + (uint64_t)(q * ks_x), idesc2, (first && q == 0) ? 0u : 1u);
-#if SSP_EM_XT_LO
+          // the residual (lo) FP16 piece of the frames too: leaving it out saves 4 of 23 MMAs per step (19.7 vs 21.0 ms per
+          // call at config 3), but the 11-bit x and x^2 cancel in S/N - mean^2: variances off by up to 60 % in
+          // test_em_trajectory_matches_sklearn
 #pragma unroll
           for (int q = 0; q < BLK / 16; ++q)
             mma_f16_ts(t_stat, t_gam + 32u * (q >> 1) + 8u * (q & 1), xlo + (uint64_t)(q * ks_x), idesc2, 1u);
-#endif
           if (flush) tc_commit(st_done + t);
           tc_commit(f_empty + p % NF);
           tc_commit(x_empty + xs);
@@ -792,21 +784,8 @@ int launch_stats_tc(const float* feats, const int64_t* seg_offsets, int64_t n_se
   const size_t TB = w.img_bytes();
   const size_t smem_lse = (2 + NS_L) * TB + 16 * sizeof(uint64_t) + 64;
   const size_t smem_stats = 2 * TB + p3::NF * (TB / 2 + 256) + p3::NX * (TB / 2) + (13 + 2 * p3::NF + 2 * p3::NX) * sizeof(uint64_t) + 64;
-  static int poly = -1;
-  if (poly < 0) {
-    const char* e = getenv("SSP_EM_POLY_PAIRS");  // share of the LSE pass's exponentials on the FMA pipe (pairs of 16)
-    poly = e ? atoi(e) : 6;  // measured at config 3 (36 M frames, K = 512): 2 / 4 / 6 / 8 pairs -> 30.0 / 27.8 / 26.3 / 27.3 ms per call
-  }
-#define SSP_EM_LSE(pp)                                                                                               \
-  case pp:                                                                                                           \
-    SSP_CUDA_OK(cudaFuncSetAttribute(gmm_em_lse_kernel<pp>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_lse)); \
-    gmm_em_lse_kernel<pp><<<dim3((unsigned)gx_l, (unsigned)n_pairs, gz), THREADS, smem_lse, st>>>(a);               \
-    break;
-  switch (poly) {
-    SSP_EM_LSE(0) SSP_EM_LSE(2) SSP_EM_LSE(4) SSP_EM_LSE(6) SSP_EM_LSE(8)
-    default: SSP_REQUIRE(false, "SSP_EM_POLY_PAIRS must be 0, 2, 4, 6 or 8 (got %d)", poly);
-  }
-#undef SSP_EM_LSE
+  SSP_CUDA_OK(cudaFuncSetAttribute(gmm_em_lse_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_lse));
+  gmm_em_lse_kernel<<<dim3((unsigned)gx_l, (unsigned)n_pairs, gz), THREADS, smem_lse, st>>>(a);
   SSP_LAUNCH_CHECK("gmm_em_lse_kernel");
   {
     const int64_t groups = (w.nb_max + 3) / 4, cap = 8 * (int64_t)num_sms;

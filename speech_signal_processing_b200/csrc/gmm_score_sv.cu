@@ -64,23 +64,12 @@ constexpr int CTRL_REGS = 32, EPI_REGS = 112;  // launched at 96: 128 x (96 - 32
 constexpr int NQ = kSvBaseImages;          // ring slots of the common part: B_hi columns [0, KS) and [KS, KQ), B_lo likewise
 constexpr int CHUNK = kSvChunk;                // models per chunk: partial sums [2 column halves][CHUNK][UNIT] fp32 = 64 KB
 constexpr uint32_t ACC_COL0 = 128;       // TMEM: [0, 2 KS) frame operand of the two row blocks, [128, 512) accumulators
-#ifndef SSP_SV_WEIGHTS
-#define SSP_SV_WEIGHTS 1  // 1: the epilogue keeps 2^(q - m_t) as weights; 0: q - m_t is left in the accumulator slots (round-1 scheme)
-#endif
-#ifndef SSP_SV_RELAX_NS
-#define SSP_SV_RELAX_NS 1000  // suspend-time hint of the control warps' mbarrier waits
-#endif
-#ifndef SSP_SV_RSTEPS
-#define SSP_SV_RSTEPS 0  // A/B builds only: K steps issued per model job (0 = all; fewer gives wrong results, for timing)
-#endif
-#ifndef SSP_SV_QMASK
-#define SSP_SV_QMASK 0xf  // which of the NQ images of the common part are multiplied (all; cleared bits are A/B builds)
-#endif
-// Share of the exponentials on the FMA pipe, measured on B200 (bench.py config 4, ms per scoring call, benchmarks/sv_poly_ab.sh;
+constexpr uint32_t kRelaxNs = 1000;      // suspend-time hint of the control warps' mbarrier waits
+// Share of the exponentials on the FMA pipe, measured on B200 (bench.py config 4, ms per scoring call, profiles/r2k_sv_ab.txt E;
 // the float64 oracle check reads 1.35e-5 / 1.36e-5 relative for degree 4 / 3): FP16 kernel, (pairs, degree) = (2,4) 728, (4,4) 711,
 // (6,4) 706, (6,3) 691, (8,3) 720.  (The TF32 kernel of round 1, power-capped and with twice the MMA instructions, was best at (4,4).)
-constexpr int kDefaultPolyPairs = 6;
-constexpr int kDefaultPolyDeg = 3;
+constexpr int kPolyPairs = 6;
+constexpr int kPolyDeg = 3;
 
 struct Args {
   const float* feats;
@@ -114,56 +103,35 @@ __device__ __forceinline__ bool bar_try_wait(uint32_t bar, uint32_t parity) {
       : "memory");
   return ok != 0;
 }
-// spin on an mbarrier phase; a protocol bug must trap (after seconds), not hang the GPU.  The bound is a poll counter:
-// reading clock64() in every iteration was 5 % of the kernel's executed instructions (profiles/r1d_sass_opcode_mix).
+// spin on an mbarrier phase; a protocol bug must trap (after seconds), not hang the GPU.
 // No printf here: a call would cost the control warps more registers than setmaxnreg leaves them.
-// Watchdog of the spin loops: clock64() (default) or a poll counter (SSP_SV_CLOCK_WATCHDOG=0).  The clock reads are 5 % of
-// the kernel's executed instructions, but removing them makes it SLOWER: measured on one box, config 4, ms per call
-// (benchmarks/sv_ab.sh, profiles/r2e_sv_ab.txt): clock64 706 / 708, poll counter 718 / 727, counter + nanosleep(20 / 60)
-// 712 / 713 -- a waiting epilogue warp that polls faster takes issue slots and mbarrier bandwidth from the three working
-// warps of its sub-partition; the clock read is the cheapest throttle found.
-#ifndef SSP_SV_CLOCK_WATCHDOG
-#define SSP_SV_CLOCK_WATCHDOG 1
-#endif
+// The bound is clock64(): its reads are 5 % of the kernel's executed instructions, but a poll counter instead makes it
+// SLOWER: measured on one box, config 4, ms per call (profiles/r2e_sv_ab.txt): clock64 706 / 708, poll counter 718 / 727,
+// counter + nanosleep(20 / 60) 712 / 713 -- a waiting epilogue warp that polls faster takes issue slots and mbarrier
+// bandwidth from the three working warps of its sub-partition; the clock read is the cheapest throttle found.
 __device__ __forceinline__ void bar_spin(uint32_t bar, uint32_t parity) {
   if (bar_try_wait(bar, parity)) return;
-#if SSP_SV_CLOCK_WATCHDOG
   const long long t0 = clock64();
   while (!bar_try_wait(bar, parity)) {
     if (clock64() - t0 > (1ll << 31)) __trap();
   }
-#else
-  uint32_t polls = 0;
-  while (!bar_try_wait(bar, parity)) {
-#ifdef SSP_SV_POLL_SLEEP_NS
-    __nanosleep(SSP_SV_POLL_SLEEP_NS);
-#endif
-    if (++polls > (1u << 26)) __trap();
-  }
-#endif
 }
 // the control warps' version: a failed poll parks the warp in hardware for up to ~1 us instead of re-issuing the wait
 // loop, which would steal issue slots from the four epilogue warps that share the sub-partition
 __device__ __forceinline__ void bar_spin_relaxed(uint32_t bar, uint32_t parity) {
   if (bar_try_wait(bar, parity)) return;
-#if SSP_SV_CLOCK_WATCHDOG
   const long long t0 = clock64();
-#endif
-  for (uint32_t polls = 0;; ++polls) {
+  for (;;) {
     uint32_t ok;
     asm volatile(
         "{\n\t.reg .pred p;\n\t"
         "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
         "selp.u32 %0, 1, 0, p;\n\t}"
         : "=r"(ok)
-        : "r"(bar), "r"(parity), "r"((uint32_t)SSP_SV_RELAX_NS)
+        : "r"(bar), "r"(parity), "r"(kRelaxNs)
         : "memory");
     if (ok) return;
-#if SSP_SV_CLOCK_WATCHDOG
     if (clock64() - t0 > (1ll << 31)) __trap();
-#else
-    if (polls > (1u << 22)) __trap();
-#endif
   }
 }
 __device__ __forceinline__ void bar_arrive(uint32_t bar) {
@@ -181,79 +149,45 @@ __device__ __forceinline__ void bulk_g2s_u32(uint32_t smem_dst, const void* gmem
                : "memory");
 }
 
-__device__ __forceinline__ void tc_st32f(uint32_t taddr, const float (&v)[32]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
-      "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
-      :
-      : "r"(taddr), "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7]), "f"(v[8]), "f"(v[9]),
-        "f"(v[10]), "f"(v[11]), "f"(v[12]), "f"(v[13]), "f"(v[14]), "f"(v[15]), "f"(v[16]), "f"(v[17]), "f"(v[18]), "f"(v[19]),
-        "f"(v[20]), "f"(v[21]), "f"(v[22]), "f"(v[23]), "f"(v[24]), "f"(v[25]), "f"(v[26]), "f"(v[27]), "f"(v[28]), "f"(v[29]),
-        "f"(v[30]), "f"(v[31])
-      : "memory");
-}
 __device__ __forceinline__ void tc_st8(uint32_t taddr, const uint32_t (&r)[8]) {
   asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr), "r"(r[0]),
                "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
                : "memory");
 }
 
-// sum over 32 accumulator columns of 2^(r + qm) (kAdd) or 2^r (the accumulator already held qm when the MMA ran).
-// kPoly of the 16 column pairs go to the FMA pipe:
-// 2^d = 2^n p(f), n = round(d) by the 1.5 * 2^23 magic add, f = d - n in [-0.5, 0.5], p = minimax polynomial
-// (degree 4: 2.7e-6 relative, degree 3: 7.5e-5 -- 3e-5 absolute on a frame's log-likelihood at the default share, 5e-7 of
-// its magnitude), 2^n applied by adding n to the exponent field; the rest is MUFU ex2.
-// kMode 0: the accumulator already holds r + (q - m_t) (the MMA ran on top of it); 1: qm = q - m_t is added here; 2: qm holds
-// the WEIGHTS 2^(q - m_t) and the sum is sum_c qm_c 2^r_c -- same instruction count as mode 0 (the packed add of the running
-// sum becomes a packed FMA), and nothing has to be left in the accumulator slot for a later job.
-template <int kPoly, int kDeg, int kMode>
+// sum_c qm_c 2^r_c over 32 accumulator columns, qm holding the WEIGHTS 2^(q - m_t) of the common part: one packed FMA
+// per column pair.  kPolyPairs of the 16 column pairs go to the FMA pipe:
+// 2^d = 2^n p(f), n = round(d) by the 1.5 * 2^23 magic add, f = d - n in [-0.5, 0.5], p = degree-3 minimax polynomial
+// (7.5e-5 relative -- 3e-5 absolute on a frame's log-likelihood at this share, 5e-7 of its magnitude; degree 4 would be
+// 2.7e-6), 2^n applied by adding n to the exponent field; the rest is MUFU ex2.
 __device__ __forceinline__ float exp_sum32(const uint32_t (&r)[32], const float (&qm)[32]) {
-  constexpr bool kAdd = kMode == 1, kMul = kMode == 2;
-  static_assert(kPoly % 2 == 0 && kPoly <= 16, "pairs are consumed two at a time");
+  static_assert(kPolyPairs % 2 == 0 && kPolyPairs <= 16, "pairs are consumed two at a time");
+  static_assert(kPolyDeg == 3, "the coefficients below are those of the degree-3 polynomial");
   const float MAGIC = 12582912.f;  // 1.5 * 2^23
   const float2 mg = make_float2(MAGIC, MAGIC), nmg = make_float2(-MAGIC, -MAGIC), neg1 = make_float2(-1.f, -1.f);
   float2 accp = make_float2(0.f, 0.f), accm0 = accp, accm1 = accp;
 #pragma unroll
-  for (int i = 0; i < kPoly; ++i) {
+  for (int i = 0; i < kPolyPairs; ++i) {
     float2 d = make_float2(__uint_as_float(r[2 * i]), __uint_as_float(r[2 * i + 1]));
-    if (kAdd) d = __fadd2_rn(d, make_float2(qm[2 * i], qm[2 * i + 1]));
     d.x = fmaxf(d.x, -126.f);
     d.y = fmaxf(d.y, -126.f);
     const float2 t = __fadd2_rn(d, mg);
     const float2 nn = __fadd2_rn(t, nmg);
     const float2 f = __ffma2_rn(nn, neg1, d);
-    float2 p;
-    if (kDeg == 4) {
-      p = __ffma2_rn(make_float2(0.009570102207362652f, 0.009570102207362652f), f, make_float2(0.05591785907745361f, 0.05591785907745361f));
-      p = __ffma2_rn(p, f, make_float2(0.240247443318367f, 0.240247443318367f));
-      p = __ffma2_rn(p, f, make_float2(0.6931217908859253f, 0.6931217908859253f));
-      p = __ffma2_rn(p, f, make_float2(0.9999992847442627f, 0.9999992847442627f));
-    } else {
-      p = __ffma2_rn(make_float2(0.0551716685295105f, 0.0551716685295105f), f, make_float2(0.2426111251115799f, 0.2426111251115799f));
-      p = __ffma2_rn(p, f, make_float2(0.6932609677314758f, 0.6932609677314758f));
-      p = __ffma2_rn(p, f, make_float2(0.9999280571937561f, 0.9999280571937561f));
-    }
+    float2 p = __ffma2_rn(make_float2(0.0551716685295105f, 0.0551716685295105f), f, make_float2(0.2426111251115799f, 0.2426111251115799f));
+    p = __ffma2_rn(p, f, make_float2(0.6932609677314758f, 0.6932609677314758f));
+    p = __ffma2_rn(p, f, make_float2(0.9999280571937561f, 0.9999280571937561f));
     float2 e;
     e.x = __uint_as_float(__float_as_uint(p.x) + (__float_as_uint(t.x) << 23));
     e.y = __uint_as_float(__float_as_uint(p.y) + (__float_as_uint(t.y) << 23));
-    accp = kMul ? __ffma2_rn(e, make_float2(qm[2 * i], qm[2 * i + 1]), accp) : __fadd2_rn(accp, e);
+    accp = __ffma2_rn(e, make_float2(qm[2 * i], qm[2 * i + 1]), accp);
   }
 #pragma unroll
-  for (int i = kPoly; i < 16; i += 2) {
-    float2 d0 = make_float2(__uint_as_float(r[2 * i]), __uint_as_float(r[2 * i + 1]));
-    float2 d1 = make_float2(__uint_as_float(r[2 * i + 2]), __uint_as_float(r[2 * i + 3]));
-    if (kAdd) {
-      d0 = __fadd2_rn(d0, make_float2(qm[2 * i], qm[2 * i + 1]));
-      d1 = __fadd2_rn(d1, make_float2(qm[2 * i + 2], qm[2 * i + 3]));
-    }
-    if (kMul) {
-      accm0 = __ffma2_rn(make_float2(ex2(d0.x), ex2(d0.y)), make_float2(qm[2 * i], qm[2 * i + 1]), accm0);
-      accm1 = __ffma2_rn(make_float2(ex2(d1.x), ex2(d1.y)), make_float2(qm[2 * i + 2], qm[2 * i + 3]), accm1);
-    } else {
-      accm0 = __fadd2_rn(accm0, make_float2(ex2(d0.x), ex2(d0.y)));
-      accm1 = __fadd2_rn(accm1, make_float2(ex2(d1.x), ex2(d1.y)));
-    }
+  for (int i = kPolyPairs; i < 16; i += 2) {
+    const float2 d0 = make_float2(__uint_as_float(r[2 * i]), __uint_as_float(r[2 * i + 1]));
+    const float2 d1 = make_float2(__uint_as_float(r[2 * i + 2]), __uint_as_float(r[2 * i + 3]));
+    accm0 = __ffma2_rn(make_float2(ex2(d0.x), ex2(d0.y)), make_float2(qm[2 * i], qm[2 * i + 1]), accm0);
+    accm1 = __ffma2_rn(make_float2(ex2(d1.x), ex2(d1.y)), make_float2(qm[2 * i + 2], qm[2 * i + 3]), accm1);
   }
   const float2 tot = __fadd2_rn(__fadd2_rn(accm0, accm1), accp);
   return tot.x + tot.y;
@@ -262,7 +196,7 @@ __device__ __forceinline__ float exp_sum32(const uint32_t (&r)[32], const float 
 // kFirst: this launch finds the stabilisers (pre-pass over the reference model) and, if a.stab is set, leaves them for
 // the launches of the other model groups; !kFirst: reads them.  A template flag, so that the control warps (32
 // registers after setmaxnreg) compile exactly as for a single launch.
-template <int kPoly, int kDeg, int KSTEPS, bool kFirst>
+template <int KSTEPS, bool kFirst>
 __global__ void __launch_bounds__(THREADS, 1) gmm_score_sv_kernel(const Args a) {
   extern __shared__ __align__(1024) unsigned char smem[];
   constexpr int KS = KSTEPS * 16;
@@ -356,7 +290,7 @@ __global__ void __launch_bounds__(THREADS, 1) gmm_score_sv_kernel(const Args a) 
     auto next_stage = [&]() { if (++stage == NSTAGE) { stage = 0; bph ^= 1u; } };
     auto next_slot = [&]() { if (++s3 == 3) { s3 = 0; sph ^= 1u; } };
     // one accumulator job of this row block: r part only (frame operand in TMEM)
-    auto job_r = [&](uint32_t preinit) {
+    auto job_r = [&]() {
       bar_spin_relaxed(b_full + 8u * stage, bph);
       const uint32_t slot = (uint32_t)g + 2u * s3;
       bar_spin_relaxed(t_empty + 8u * slot, sph ^ 1u);
@@ -365,7 +299,7 @@ __global__ void __launch_bounds__(THREADS, 1) gmm_score_sv_kernel(const Args a) 
         const uint32_t d_tmem = tmem_base + ACC_COL0 + slot * BN;
         const uint64_t bd = b_desc0 + (uint64_t)(stage * tile_units);
 #pragma unroll
-        for (int k = 0; k < (SSP_SV_RSTEPS ? SSP_SV_RSTEPS : KSTEPS); ++k) mma_f16_ts(d_tmem, at + 8u * k, bd + (uint64_t)(k * ks_b), idesc, k > 0 ? 1u : preinit);
+        for (int k = 0; k < KSTEPS; ++k) mma_f16_ts(d_tmem, at + 8u * k, bd + (uint64_t)(k * ks_b), idesc, k > 0 ? 1u : 0u);
         bar_commit(t_full + 8u * slot);
         bar_commit(b_empty + 8u * stage);
       }
@@ -390,17 +324,15 @@ __global__ void __launch_bounds__(THREADS, 1) gmm_score_sv_kernel(const Args a) 
           const uint64_t bd = b_desc0 + (uint64_t)(stage * tile_units);
           const bool second = (part & 1) != 0;
           const uint64_t a_off = second ? (uint64_t)(KSTEPS * ks_a) : 0ull;
-          if ((SSP_SV_QMASK >> part) & 1) {  // (cleared bits: A/B builds only, benchmarks/sv_ab.sh)
+#pragma unroll
+          for (int k = 0; k < KSTEPS; ++k)
+            if (!second || k < steps_b)
+              mma_f16_ss(d_tmem, ah_desc + a_off + (uint64_t)(k * ks_a), bd + (uint64_t)(k * ks_b), idesc, (part | k) ? 1u : 0u);
+          if (part < 2) {
 #pragma unroll
             for (int k = 0; k < KSTEPS; ++k)
               if (!second || k < steps_b)
-                mma_f16_ss(d_tmem, ah_desc + a_off + (uint64_t)(k * ks_a), bd + (uint64_t)(k * ks_b), idesc, (part | k) ? 1u : 0u);
-            if (part < 2) {
-#pragma unroll
-              for (int k = 0; k < KSTEPS; ++k)
-                if (!second || k < steps_b)
-                  mma_f16_ss(d_tmem, al_desc + a_off + (uint64_t)(k * ks_a), bd + (uint64_t)(k * ks_b), idesc, 1u);
-            }
+                mma_f16_ss(d_tmem, al_desc + a_off + (uint64_t)(k * ks_a), bd + (uint64_t)(k * ks_b), idesc, 1u);
           }
           if (part == NQ - 1) bar_commit(t_full + 8u * slot);
           bar_commit(b_empty + 8u * stage);
@@ -420,7 +352,7 @@ __global__ void __launch_bounds__(THREADS, 1) gmm_score_sv_kernel(const Args a) 
         for (int j = 0; j < NT; ++j) {
           job_q();                                // common part of tile j
 #pragma unroll 1
-          for (int m = 0; m < nm; ++m) job_r(!SSP_SV_WEIGHTS && m >= 2 ? 1u : 0u);
+          for (int m = 0; m < nm; ++m) job_r();
         }
       }
       if (elect_one()) bar_commit(a_empty);
@@ -447,16 +379,11 @@ __global__ void __launch_bounds__(THREADS, 1) gmm_score_sv_kernel(const Args a) 
     const uint32_t my_tmem = tmem_base + lane_addr + ACC_COL0 + (uint32_t)(g * BN + half * 32);  // slot s3 at + 2 BN s3
     const uint32_t my_full = t_full + 8u * g, my_empty = t_empty + 8u * g;                       // slot s3 at + 16 s3
     const bool lane0 = lane == 0;
-    // `init` != nullptr: the job three ahead (same slot) belongs to the same component tile -> leave q - m_t behind
-    auto fetch = [&](uint32_t (&r)[32], const float (*init)[32] = nullptr) {
+    auto fetch = [&](uint32_t (&r)[32]) {
       bar_spin(my_full + 16u * s3, sph);
       tc_fence_after();
       tc_ld32_issue(my_tmem + 2u * BN * s3, r);
       tc_ld_wait(r);
-      if (init) {
-        tc_st32f(my_tmem + 2u * BN * s3, *init);
-        asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-      }
       tc_fence_before();
       __syncwarp();
       if (lane0) bar_arrive(my_empty + 16u * s3);
@@ -552,7 +479,6 @@ __global__ void __launch_bounds__(THREADS, 1) gmm_score_sv_kernel(const Args a) 
       for (int m0 = 0; m0 < S; m0 += CHUNK) {
         const int nm = min(CHUNK, S - m0);
         for (int j = 0; j < NT; ++j) {
-#if SSP_SV_WEIGHTS
           // sum_c 2^(q - m_t + r) = sum_c P_c 2^r_c with the weights P = 2^(q - m_t) of this thread's 32 columns kept in
           // registers for the models of the chunk: one MUFU per column and tile, and a model job is tcgen05.ld, release,
           // 32 x (ex2 | polynomial) and a packed FMA per pair.  (Round 1 left q - m_t in the accumulator slot for the MMA
@@ -571,45 +497,8 @@ __global__ void __launch_bounds__(THREADS, 1) gmm_score_sv_kernel(const Args a) 
           for (int m = 0; m < nm; ++m, dst += UNIT) {
             uint32_t r[32];
             fetch(r);
-            *dst += exp_sum32<kPoly, kDeg, 2>(r, qm);
+            *dst += exp_sum32(r, qm);
           }
-#else
-          // Job i of this tile (i = 0: common part, i = 1 + m: model m) shares its accumulator slot with job i + 3.
-          // If that one is a model of the same tile, q - m_t is left in the slot and the MMA accumulates on top of
-          // it, so the sum needs no add; the first two models of a tile (their slots were last used by the previous
-          // tile) add q - m_t here instead.
-          float qm[32];
-          {
-            uint32_t r[32];
-            bar_spin(my_full + 16u * s3, sph);
-            tc_fence_after();
-            tc_ld32_issue(my_tmem + 2u * BN * s3, r);
-            tc_ld_wait(r);
-#pragma unroll
-            for (int i = 0; i < 32; ++i) qm[i] = __uint_as_float(r[i]) - m_t;
-            if (nm > 2) {
-              tc_st32f(my_tmem + 2u * BN * s3, qm);
-              asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-            }
-            tc_fence_before();
-            __syncwarp();
-            if (lane0) bar_arrive(my_empty + 16u * s3);
-            if (++s3 == 3) { s3 = 0; sph ^= 1u; }
-          }
-          float* dst = my_part;
-#pragma unroll 1
-          for (int m = 0; m < nm && m < 2; ++m, dst += UNIT) {
-            uint32_t r[32];
-            fetch(r, m + 3 < nm ? &qm : nullptr);
-            *dst += exp_sum32<kPoly, kDeg, 1>(r, qm);
-          }
-#pragma unroll 1
-          for (int m = 2; m < nm; ++m, dst += UNIT) {
-            uint32_t r[32];
-            fetch(r, m + 3 < nm ? &qm : nullptr);
-            *dst += exp_sum32<kPoly, kDeg, 0>(r, qm);
-          }
-#endif
         }
         // ---- partial sums of this chunk -> per-frame log-likelihood -> per-utterance score
         named_bar_sync(3, EPI);
@@ -696,25 +585,24 @@ static int num_sms() {
   return g_num_sms;
 }
 
-template <int kPoly, int kDeg, int KSTEPS>
+template <int KSTEPS>
 static int launch_one(const Args& a, unsigned grid, bool first, cudaStream_t st) {
   const size_t smem = sv_smem_bytes(KSTEPS * 16, a.KQ);  // make_sv_layout has checked it against the 227 KB limit
   if (first) {
-    SSP_CUDA_OK(cudaFuncSetAttribute(gmm_score_sv_kernel<kPoly, kDeg, KSTEPS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    gmm_score_sv_kernel<kPoly, kDeg, KSTEPS, true><<<grid, THREADS, smem, st>>>(a);
+    SSP_CUDA_OK(cudaFuncSetAttribute(gmm_score_sv_kernel<KSTEPS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    gmm_score_sv_kernel<KSTEPS, true><<<grid, THREADS, smem, st>>>(a);
   } else {
-    SSP_CUDA_OK(cudaFuncSetAttribute(gmm_score_sv_kernel<kPoly, kDeg, KSTEPS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    gmm_score_sv_kernel<kPoly, kDeg, KSTEPS, false><<<grid, THREADS, smem, st>>>(a);
+    SSP_CUDA_OK(cudaFuncSetAttribute(gmm_score_sv_kernel<KSTEPS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    gmm_score_sv_kernel<KSTEPS, false><<<grid, THREADS, smem, st>>>(a);
   }
   return SSP_OK;
 }
-template <int kPoly, int kDeg>
 static int launch_ks(const Args& a, unsigned grid, bool first, cudaStream_t st) {
   switch (a.KS) {
-    case 16: return launch_one<kPoly, kDeg, 1>(a, grid, first, st);
-    case 32: return launch_one<kPoly, kDeg, 2>(a, grid, first, st);
-    case 48: return launch_one<kPoly, kDeg, 3>(a, grid, first, st);
-    case 64: return launch_one<kPoly, kDeg, 4>(a, grid, first, st);
+    case 16: return launch_one<1>(a, grid, first, st);
+    case 32: return launch_one<2>(a, grid, first, st);
+    case 48: return launch_one<3>(a, grid, first, st);
+    case 64: return launch_one<4>(a, grid, first, st);
   }
   set_error("ssp_gmm_score_shared: contraction length %d is not a multiple of 16 in [16, 64]", a.KS);
   return SSP_EINVAL;
@@ -772,29 +660,12 @@ int launch_score_sv(const float* feats, const int64_t* offsets, int64_t n_utts, 
   a.stab = group < L.n_models ? (float*)workspace : nullptr;
   const int64_t n_units = (total_frames + UNIT - 1) / UNIT;
   const unsigned grid = (unsigned)(n_units < num_sms() ? n_units : num_sms());
-  static int poly = -1, deg = -1;
-  if (poly < 0) {
-    const char* e = getenv("SSP_SV_POLY_PAIRS");  // tuning knobs: share of the exponentials on the FMA pipe, degree
-    poly = e ? atoi(e) : kDefaultPolyPairs;
-    e = getenv("SSP_SV_POLY_DEG");
-    deg = e ? atoi(e) : kDefaultPolyDeg;
-  }
   for (int m0 = 0; m0 < L.n_models; m0 += group) {
     a.n_models = L.n_models - m0 < group ? L.n_models - m0 : group;
     a.tiles_group = a.tiles + (size_t)m0 * BN * L.KS;   // images are BN * KS FP16 values
     a.scores = scores + m0;
     a.frame_lse = frame_lse ? frame_lse + (size_t)m0 * total_frames : nullptr;
-    const bool first = m0 == 0;
-    int rc = SSP_EINVAL;
-    if (deg == 4 && poly == 0) rc = launch_ks<0, 4>(a, grid, first, st);
-    else if (deg == 4 && poly == 2) rc = launch_ks<2, 4>(a, grid, first, st);
-    else if (deg == 4 && poly == 4) rc = launch_ks<4, 4>(a, grid, first, st);
-    else if (deg == 4 && poly == 6) rc = launch_ks<6, 4>(a, grid, first, st);
-    else if (deg == 4 && poly == 8) rc = launch_ks<8, 4>(a, grid, first, st);
-    else if (deg == 3 && poly == 4) rc = launch_ks<4, 3>(a, grid, first, st);
-    else if (deg == 3 && poly == 6) rc = launch_ks<6, 3>(a, grid, first, st);
-    else if (deg == 3 && poly == 8) rc = launch_ks<8, 3>(a, grid, first, st);
-    else set_error("SSP_SV_POLY_PAIRS / SSP_SV_POLY_DEG: unsupported combination (%d, %d)", poly, deg);
+    const int rc = launch_ks(a, grid, m0 == 0, st);
     if (rc != SSP_OK) return rc;
     SSP_LAUNCH_CHECK("gmm_score_sv_kernel");
   }

@@ -24,7 +24,6 @@
 // so the epilogue is max / ex2 / add only.
 #include <cuda_fp16.h>
 
-#include <cstdlib>
 #include <mutex>
 #include <unordered_map>
 
@@ -49,7 +48,7 @@ constexpr int threads_of(int mb) { return 64 + 8 * mb * 32; }
 // Measured on B200 under the 1 kW cap (10k utts x 1001 models): pairs 0/2/4/6/8 -> 523/539/526/496/486 TFLOP/s.
 // The kernel is power-bound, not pipe-bound: a MUFU ex2 costs less energy than the ~7 FMA-pipe instructions that
 // replace it, so only a small share is worth moving.
-constexpr int kDefaultPolyPairs = 2;
+constexpr int kPolyPairs = 2;
 
 // Sum of 2^(v - m_stab) over 32 accumulator columns of one row, plus their maximum.
 //
@@ -62,7 +61,6 @@ constexpr int kDefaultPolyPairs = 2;
 // evaluated on the FMA pipe: 2^x = 2^n * p(f), n = round(x) via the 1.5*2^23 magic add, f = x - n in
 // [-0.5, 0.5], p = degree-4 minimax polynomial (max relative error 2.7e-6), 2^n applied by adding n to the
 // exponent field.  Packed FADD2 / FFMA2 halve the issue slots; FMNMX3 halves the max chain.
-template <int kPolyPairs>
 __device__ __forceinline__ void chunk_sum(const uint32_t (&r)[32], float m_stab, float2& accp, float2& accm0, float2& accm1,
                                           float& cmax) {
   float v[32];
@@ -135,7 +133,7 @@ struct Args {
 
 // kH: FP16 operands (kind::f16, K = 16 per MMA: half the MMA instructions, half the bytes of a model tile and of the frame
 // operand; an FP16 significand has TF32's 11 bits, so every rung keeps its error).  a.KD is then the FP16 contraction length.
-template <int kPolyPairs, int MB, int NPARTS, bool kH = false>
+template <int MB, int NPARTS, bool kH>
 __global__ void __launch_bounds__(threads_of(MB), 1) gmm_score_tc_kernel(const Args a) {
   static_assert(NPARTS >= 1 && NPARTS <= 3 && (MB == 1 || MB == 2) && (NPARTS < 3 || MB == 1), "see the rung table");
   constexpr uint32_t ELT = kH ? 2u : 4u;
@@ -319,8 +317,8 @@ __global__ void __launch_bounds__(threads_of(MB), 1) gmm_score_tc_kernel(const A
           tc_ld32_issue(taddr, ra);
           tc_ld32_issue(taddr + 32, rb);
           tc_ld_wait2(ra, rb);
-          chunk_sum<kPolyPairs>(ra, m_stab, accp, accm0, accm1, cmax);
-          chunk_sum<kPolyPairs>(rb, m_stab, accp, accm0, accm1, cmax);
+          chunk_sum(ra, m_stab, accp, accm0, accm1, cmax);
+          chunk_sum(rb, m_stab, accp, accm0, accm1, cmax);
           const float2 tot = __fadd2_rn(__fadd2_rn(accm0, accm1), accp);
           float s_tile = tot.x + tot.y;
           // stabiliser check: too low (overflow risk) on any tile, too high (underflow of everything) on a
@@ -428,12 +426,7 @@ void note_pack(const void* pack) {
   g_pack_h[pack] = -1;
 }
 static bool pack_h_usable(const void* pack, const PackLayout& L, cudaStream_t st) {
-  static int off = -1;
-  if (off < 0) {
-    const char* e = getenv("SSP_TC_TF32");   // A/B knob: 1 = the single-pass rung always issues kind::tf32
-    off = e ? atoi(e) : 0;
-  }
-  if (off || !L.off_tile_h) return false;
+  if (!L.off_tile_h) return false;
   std::lock_guard<std::mutex> lk(g_pack_mu);
   auto it = g_pack_h.find(pack);
   if (it == g_pack_h.end()) return false;   // a pack this process did not build (copied buffer): TF32 images are always valid
@@ -490,32 +483,19 @@ int launch_score_tc(const float* feats, const int64_t* offsets, int64_t n_utts, 
   }
   const int64_t n_units = (total_frames + unit - 1) / unit;
   const unsigned grid = (unsigned)(n_units < num_sms ? n_units : num_sms);
-  // share of the exponentials evaluated on the FMA pipe (pairs out of 16 per 32 columns); tuning knob of the 1-pass rung
-  static int poly = -1;
-  if (poly < 0) {
-    const char* e = getenv("SSP_TC_POLY_PAIRS");
-    poly = e ? atoi(e) : kDefaultPolyPairs;
-  }
-#define SSP_TC_LAUNCH(pp, MBv, NP)                                                                                              \
+#define SSP_TC_LAUNCH(MBv, NP)                                                                                                  \
   do {                                                                                                                          \
     if (use_h) {                                                                                                                \
-      SSP_CUDA_OK(cudaFuncSetAttribute(gmm_score_tc_kernel<pp, MBv, NP, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-      gmm_score_tc_kernel<pp, MBv, NP, true><<<grid, threads_of(MBv), smem, st>>>(a);                                          \
+      SSP_CUDA_OK(cudaFuncSetAttribute(gmm_score_tc_kernel<MBv, NP, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+      gmm_score_tc_kernel<MBv, NP, true><<<grid, threads_of(MBv), smem, st>>>(a);                                               \
     } else {                                                                                                                    \
-      SSP_CUDA_OK(cudaFuncSetAttribute(gmm_score_tc_kernel<pp, MBv, NP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-      gmm_score_tc_kernel<pp, MBv, NP><<<grid, threads_of(MBv), smem, st>>>(a);                                                \
+      SSP_CUDA_OK(cudaFuncSetAttribute(gmm_score_tc_kernel<MBv, NP, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+      gmm_score_tc_kernel<MBv, NP, false><<<grid, threads_of(MBv), smem, st>>>(a);                                              \
     }                                                                                                                           \
   } while (0)
-  if (parts == 2) SSP_TC_LAUNCH(kDefaultPolyPairs, 2, 2);
-  else if (parts == 3) SSP_TC_LAUNCH(kDefaultPolyPairs, 1, 3);
-  else switch (poly) {
-    case 0: SSP_TC_LAUNCH(0, 2, 1); break;
-    case 2: SSP_TC_LAUNCH(2, 2, 1); break;
-    case 4: SSP_TC_LAUNCH(4, 2, 1); break;
-    case 6: SSP_TC_LAUNCH(6, 2, 1); break;
-    case 8: SSP_TC_LAUNCH(8, 2, 1); break;
-    default: SSP_REQUIRE(false, "SSP_TC_POLY_PAIRS must be 0, 2, 4, 6 or 8 (got %d)", poly);
-  }
+  if (parts == 1) SSP_TC_LAUNCH(2, 1);
+  else if (parts == 2) SSP_TC_LAUNCH(2, 2);
+  else SSP_TC_LAUNCH(1, 3);
 #undef SSP_TC_LAUNCH
   SSP_LAUNCH_CHECK(parts == 1 ? "gmm_score_tc_kernel" : parts == 2 ? "gmm_score_tc_kernel<2 passes>" : "gmm_score_tc_kernel<3 passes>");
   if (use_h) {

@@ -33,20 +33,11 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
 // poll; round 1 read clock64() in every iteration of every spin loop, 5 % of all executed instructions of the scoring
 // kernel and half of those of the EM kernels).  mbarrier.try_wait itself blocks for a hardware-defined time slice,
 // so 2^26 failed polls are seconds.
-#ifndef SSP_CLOCK_WATCHDOG
-#define SSP_CLOCK_WATCHDOG 0
-#endif
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   if (mbar_try_wait(bar, parity)) return;
-#if SSP_CLOCK_WATCHDOG
-  const long long t0 = clock64();
-  while (!mbar_try_wait(bar, parity)) {
-    if (clock64() - t0 > (1ll << 32)) {
-#else
   uint32_t polls = 0;
   while (!mbar_try_wait(bar, parity)) {
     if (++polls > (1u << 26)) {
-#endif
       printf("ssp: mbarrier wait timed out (block %d,%d thread %d bar %u parity %u)\n", blockIdx.x, blockIdx.y, threadIdx.x,
              smem_u32(bar), parity);
       __trap();

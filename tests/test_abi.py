@@ -78,6 +78,24 @@ def test_null_arguments_fail_without_touching_the_gpu(lib):
     assert lib.ssp_delta(None, 10, 13, 0, None, None) == -1
 
 
+def test_library_has_no_hidden_tuning_switches():
+    """The kernels' tuning choices are constants in the sources.  The only environment variable the library reads is
+    SSP_SV_GROUP_MB (the L2 group size of shared-variance scoring, which tests use to reach the multi-launch path), and no
+    SSP_ macro selects code at build time."""
+    import glob
+
+    names, directives = set(), []
+    for path in sorted(glob.glob(os.path.join(ROOT, "speech_signal_processing_b200", "csrc", "*.cu*"))):
+        text = open(path).read()
+        calls = re.findall(r"\bgetenv\s*\(", text)
+        literal = re.findall(r"\bgetenv\s*\(\s*\"([^\"]*)\"\s*\)", text)
+        assert len(literal) == len(calls), f"{os.path.basename(path)}: getenv with a computed name"
+        names.update(literal)
+        directives += [(os.path.basename(path), d) for d in re.findall(r"^[ \t]*#[ \t]*(?:if|ifdef|ifndef|elif)\b.*\bSSP_\w*", text, flags=re.M)]
+    assert names == {"SSP_SV_GROUP_MB"}
+    assert directives == []
+
+
 def test_header_is_plain_c(tmp_path):
     """The boundary is a C ABI: include/ssp_b200.h must compile as C99 (no C++ or torch types in the signatures) and a
     C translation unit that calls the host-only entry points must link against the library."""
