@@ -361,7 +361,6 @@ def levinson(r, order):
 def sidekit_plp(sig, nwin=0.025, fs=16000, plp_order=13, shift=0.01, get_spec=False, get_mspec=False, prefac=0.97,
                 rasta=True):
     """Restatement of SIDEKIT ``plp`` (rastamat ``rastaplp``).  Returns ``[ceps (T, plp_order), log_energy (T,), None, None]``."""
-    order = plp_order - 1
     win = int(round(nwin * fs))
     hop = int(shift * fs)
     nfft = 2 ** int(math.ceil(math.log2(win)))
@@ -375,10 +374,17 @@ def sidekit_plp(sig, nwin=0.025, fs=16000, plp_order=13, shift=0.01, get_spec=Fa
     powspec = mag.real ** 2 + mag.imag ** 2                              # (T, 257)
     wts = fft2barkmx(nfft, fs, 0, 1.0, 0.0, fs / 2.0)                    # (21, 257) at 16 kHz
     asp = powspec @ wts.T                                                # (T, nbands)
+    return [plp_post(asp, plp_order, fs / 2.0, rasta), log_energy, None, None]
+
+
+def plp_post(asp, plp_order, fmax, rasta=True):
+    """The back half of ``rastaplp`` on critical-band energies asp (T, nbands): rasta -> postaud -> dolpc -> lpc2cep ->
+    lifter.  Returns the liftered cepstra (T, plp_order)."""
+    order = plp_order - 1
     nbands = asp.shape[1]
     if rasta:
         asp = np.exp(rasta_filt(np.log(asp)))
-    post = (postaud_weights(nbands, fs / 2.0)[None, :] * asp) ** 0.33
+    post = (postaud_weights(nbands, fmax)[None, :] * asp) ** 0.33
     post[:, 0] = post[:, 1]
     post[:, -1] = post[:, -2]
     # dolpc: autocorrelation = real IDFT of the even-symmetric extension, then Levinson-Durbin
@@ -397,7 +403,7 @@ def sidekit_plp(sig, nwin=0.025, fs=16000, plp_order=13, shift=0.01, get_spec=Fa
             s += (n - m) * norm[:, m] * cep[:, n - m]
         cep[:, n] = -(norm[:, n] + s / n)
     lift = np.concatenate([[1.0], np.arange(1, ncep, dtype=np.float64) ** 0.6])
-    return [cep * lift[None, :], log_energy, None, None]
+    return cep * lift[None, :]
 
 
 # ----------------------------------------------------------------------------

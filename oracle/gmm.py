@@ -98,17 +98,19 @@ def map_adapt(n, f, s, weights, means, variances, n_frames, relevance=16.0,
     alpha_c = n_c / (n_c + r); mu^_c = alpha E_c[x] + (1-alpha) mu_c
     (optionally) w^_c ~ alpha n_c / T + (1-alpha) w_c, renormalised;
     var^_c = alpha E_c[x^2] + (1-alpha)(var_c + mu_c^2) - mu^_c^2.
+    A speaker or component without data keeps the UBM's parameters: alpha = 0 where n_c = 0 (also at relevance 0),
+    and the weight term alpha n_c / T is 0 for a speaker of T = 0 frames.
     The reference has no MAP code (SURVEY F4): parity unpinned, defined by formula.
     """
     n = np.asarray(n, dtype=np.float64)
-    alpha = (n / (n + relevance))[:, None]
+    alpha = np.divide(n, n + relevance, out=np.zeros_like(n), where=n > 0)[:, None]
     safe = np.maximum(n, np.finfo(np.float64).tiny)[:, None]
     ex = f / safe
     ex2 = s / safe
     new_means = alpha * ex + (1.0 - alpha) * means if "means" in adapt else np.array(means, dtype=np.float64)
     new_w = np.array(weights, dtype=np.float64)
     if "weights" in adapt:
-        new_w = alpha[:, 0] * n / n_frames + (1.0 - alpha[:, 0]) * weights
+        new_w = (alpha[:, 0] * n / n_frames if n_frames > 0 else 0.0) + (1.0 - alpha[:, 0]) * weights
         new_w = new_w / new_w.sum()
     new_var = np.array(variances, dtype=np.float64)
     if "variances" in adapt:

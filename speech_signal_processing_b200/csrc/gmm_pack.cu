@@ -276,7 +276,9 @@ __global__ void gmm_mstep_kernel(const double* __restrict__ n, const double* __r
 }
 
 // ------------------------------------------------------------------------------------------ MAP
-// Reynolds, Quatieri, Dunn (2000) eq. 11-14.  One block per speaker.
+// Reynolds, Quatieri, Dunn (2000) eq. 11-14.  One block per speaker.  A speaker or component without data keeps the
+// UBM's parameters: alpha = 0 when n = 0 (also at relevance 0, where n / (n + r) would be 0 / 0), and the weight term
+// alpha n / T is 0 for a speaker of T = 0 frames.
 __global__ void gmm_map_kernel(const double* __restrict__ n, const double* __restrict__ f, const double* __restrict__ s,
                                const int64_t* __restrict__ seg, const double* __restrict__ uw,
                                const double* __restrict__ umu, const double* __restrict__ uvar, int K, int D,
@@ -292,8 +294,9 @@ __global__ void gmm_map_kernel(const double* __restrict__ n, const double* __res
     const double T = (double)(seg[spk + 1] - seg[spk]);
     double part = 0.0;
     for (int c = threadIdx.x; c < K; c += blockDim.x) {
-      double a = n_s[c] / (n_s[c] + relevance);
-      double v = (flags & 2) ? a * n_s[c] / T + (1.0 - a) * uw[c] : uw[c];
+      double a = n_s[c] > 0.0 ? n_s[c] / (n_s[c] + relevance) : 0.0;
+      const double wn = T > 0.0 ? a * n_s[c] / T : 0.0;
+      double v = (flags & 2) ? wn + (1.0 - a) * uw[c] : uw[c];
       ow[(int64_t)spk * K + c] = v;
       part += v;
     }
@@ -312,7 +315,7 @@ __global__ void gmm_map_kernel(const double* __restrict__ n, const double* __res
   for (int i = threadIdx.x; i < K * D; i += blockDim.x) {
     int c = i / D;
     double nc = n_s[c];
-    double a = nc / (nc + relevance);
+    double a = nc > 0.0 ? nc / (nc + relevance) : 0.0;
     double safe = nc > 1e-300 ? nc : 1e-300;
     double m_new = (flags & 1) ? a * (f_s[i] / safe) + (1.0 - a) * umu[i] : umu[i];
     if (omu) omu[(int64_t)spk * K * D + i] = m_new;

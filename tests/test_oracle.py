@@ -144,6 +144,33 @@ def test_map_adapt_limits():
     assert np.isclose(w2.sum(), 1.0) and (v2 > 0).all()
 
 
+def test_map_adapt_without_data_keeps_the_ubm():
+    """A speaker of no frames, and a component no frame reaches (also at relevance 0), keep the UBM's parameters."""
+    from speech_signal_processing_b200 import synth
+
+    every = ("means", "weights", "variances")
+    w, mu, var = synth.synth_ubm(8, 5, seed=4)
+    z = np.zeros(8)
+    for r in (16.0, 0.0):
+        got = ogmm.map_adapt(z, np.zeros((8, 5)), np.zeros((8, 5)), w, mu, var, 0, relevance=r, adapt=every)
+        for g, want in zip(got, (w / w.sum(), mu, var)):
+            assert np.isfinite(g).all()
+            np.testing.assert_allclose(g, want, rtol=1e-12, atol=0)   # var + mu^2 - mu^2 rounds
+    x = synth.sample_gmm(w, mu + 0.5, var, 400, seed=5).astype(np.float64)
+    n, f, s, _ = ogmm.suff_stats(x, w, mu, var)
+    n[3], f[3], s[3] = 0.0, 0.0, 0.0
+    for r in (16.0, 0.0):
+        w2, m2, v2 = ogmm.map_adapt(n, f, s, w, mu, var, 400, relevance=r, adapt=every)
+        assert np.isfinite(w2).all() and np.isfinite(m2).all() and np.isfinite(v2).all()
+        np.testing.assert_array_equal(m2[3], mu[3])
+        np.testing.assert_allclose(v2[3], var[3], rtol=1e-12)
+        a = n / (n + r) if r else (n > 0).astype(float)
+        want_w = a * n / 400 + (1 - a) * w
+        np.testing.assert_allclose(w2, want_w / want_w.sum(), rtol=1e-14)
+    np.testing.assert_allclose(ogmm.map_adapt(n, f, s, w, mu, var, 400, relevance=0.0)[1][n > 0], (f / n[:, None])[n > 0],
+                               rtol=1e-14)
+
+
 def test_vad_matches_reference(golden):
     """oracle.vad against the unmodified VAD.py (framing, ZCR, energy, spectral entropy, both detectors)."""
     from oracle import vad as ov
