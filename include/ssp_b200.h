@@ -271,6 +271,31 @@ int ssp_gmm_stats(const float* feats, const int64_t* seg_offsets, int64_t n_segs
 int64_t ssp_gmm_stats_workspace_bytes(const ssp_gmm_dims* dims, int64_t total_frames, int64_t n_segs);
 
 /*
+ * Frame posteriors (GaussianMixture.predict_proba / predict, sklearn _base.py:552-582 and argmax of it):
+ *   gamma[t, c] = w_c N(x_t; c) / sum_c' w_c' N(x_t; c'),  label[t] = lowest c maximising log w_c + log N(x_t; c)
+ *   (numpy's argmax rule on ties).
+ * Models and segments as in ssp_gmm_stats: dims->n_models == 1 puts every segment under the one model,
+ * dims->n_models == n_segs puts segment s under model s (D <= 39 only; SSP_EUNSUP above).
+ * Always FP32 grade: for D <= 39 the logits are the 3 x BF16 tcgen05 products of ssp_gmm_stats (same frame images,
+ * same per-frame log-likelihood), for 40 <= D <= 80 the FP32 CUDA-core kernels of SSP_PREC_FP32.
+ * out_resp       device float[total_frames * K] (row-major, K unpadded) or NULL
+ * out_label      device int64[total_frames] or NULL; at least one of the two (both NULL is SSP_EINVAL).  Labels alone
+ *                skip the log-sum-exp pass.
+ * out_frame_lse  device float[total_frames] or NULL: per-frame log-likelihood (computed when out_resp or this is set)
+ * workspace      device, ssp_gmm_posteriors_workspace_bytes() bytes, 1024-byte aligned.  For D <= 39 it has the layout
+ *                of the ssp_gmm_stats workspace (same size, frame images at the same place), so one workspace serves both
+ *                calls on the same frames and reuse_images works across them (label the frames of an EM run
+ *                without preparing them again).
+ * reuse_images   nonzero: the workspace still holds the images of THIS feats / seg_offsets (see ssp_gmm_stats).
+ */
+int ssp_gmm_posteriors(const float* feats, const int64_t* seg_offsets, int64_t n_segs, int64_t total_frames,
+                       const void* pack, const ssp_gmm_dims* dims, float* out_resp, int64_t* out_label,
+                       float* out_frame_lse, void* workspace, int64_t workspace_bytes, int32_t reuse_images,
+                       void* stream);
+/* Scratch bytes ssp_gmm_posteriors needs for these dims, frames and segments (0: unsupported dims). */
+int64_t ssp_gmm_posteriors_workspace_bytes(const ssp_gmm_dims* dims, int64_t total_frames, int64_t n_segs);
+
+/*
  * M-step on device (sklearn _gaussian_mixture.py:312-313,250-252,898): from (all-reduced)
  * statistics to weights/means/variances, double precision, for n_models models at once (arrays [n_models][K](xD)).
  * nk = N + 10*eps_of(stat_dtype); mu = F/nk; var = S/nk - mu^2 + reg_covar; w = nk/sum(nk).

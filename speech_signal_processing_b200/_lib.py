@@ -71,6 +71,8 @@ PROTOTYPES = {
     "ssp_gmm_score_shared": (C.c_int, [_P, _P, _I64, _I64, _P, C.POINTER(GmmDims), _P, _P, _P, _I64, _P]),
     "ssp_gmm_stats": (C.c_int, [_P, _P, _I64, _I64, _P, C.POINTER(GmmDims), _P, _P, _P, _P, _P, _P, _I64, _I32, _P]),
     "ssp_gmm_stats_workspace_bytes": (_I64, [C.POINTER(GmmDims), _I64, _I64]),
+    "ssp_gmm_posteriors": (C.c_int, [_P, _P, _I64, _I64, _P, C.POINTER(GmmDims), _P, _P, _P, _P, _I64, _I32, _P]),
+    "ssp_gmm_posteriors_workspace_bytes": (_I64, [C.POINTER(GmmDims), _I64, _I64]),
     "ssp_gmm_mstep": (C.c_int, [_P, _P, _P, _I32, _I32, _I32, C.c_double, C.c_double, _P, _P, _P, _P]),
     "ssp_gmm_map_adapt": (C.c_int, [_P, _P, _P, _P, _I64, _P, _P, _P, _I32, _I32, C.c_double, _I32, _P, _P, _P, _P]),
     "ssp_dtw_max_len": (_I64, [_I32]),

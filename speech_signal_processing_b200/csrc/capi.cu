@@ -163,3 +163,45 @@ extern "C" int ssp_gmm_stats(const float* feats, const int64_t* seg_offsets, int
   if (rc != SSP_OK) return rc;
   return ssp::launch_stats_simt(feats, seg_offsets, n_segs, total_frames, pack, L, frame_lse, out_n, out_f, out_s, st);
 }
+
+extern "C" int64_t ssp_gmm_posteriors_workspace_bytes(const ssp_gmm_dims* dims, int64_t total_frames, int64_t n_segs) {
+  ssp::PackLayout L;
+  if (!ssp::make_layout(dims, &L) || total_frames < 0 || n_segs < 0) return 0;
+  if (ssp::stats_tc_supported(L)) return ssp::stats_tc_workspace_bytes(L, total_frames, n_segs);
+  return L.n_models == 1 ? ssp::posteriors_simt_workspace_bytes(total_frames, n_segs) : 0;
+}
+
+extern "C" int ssp_gmm_posteriors(const float* feats, const int64_t* seg_offsets, int64_t n_segs, int64_t total_frames,
+                                  const void* pack, const ssp_gmm_dims* dims, float* out_resp, int64_t* out_label,
+                                  float* out_frame_lse, void* workspace, int64_t workspace_bytes, int32_t reuse_images,
+                                  void* stream) {
+  ssp::PackLayout L;
+  SSP_REQUIRE(ssp::make_layout(dims, &L), "ssp_gmm_posteriors: unsupported dims");
+  SSP_REQUIRE(dims->n_models == 1 || dims->n_models == n_segs,
+              "ssp_gmm_posteriors: %d models for %lld segments (one model for all segments, or one per segment)",
+              dims->n_models, (long long)n_segs);
+  SSP_REQUIRE(out_resp || out_label, "ssp_gmm_posteriors: out_resp and out_label are both NULL (nothing to compute)");
+  SSP_REQUIRE(seg_offsets && pack && (feats || total_frames == 0), "ssp_gmm_posteriors: null pointer");
+  SSP_REQUIRE(n_segs >= 0 && total_frames >= 0, "ssp_gmm_posteriors: negative size");
+  if (n_segs == 0 || total_frames == 0) return SSP_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (ssp::stats_tc_supported(L)) {
+    const int64_t need = ssp::stats_tc_workspace_bytes(L, total_frames, n_segs);
+    SSP_REQUIRE(workspace && workspace_bytes >= need,
+                "ssp_gmm_posteriors: workspace of %lld bytes, need %lld (ssp_gmm_posteriors_workspace_bytes)",
+                (long long)(workspace ? workspace_bytes : 0), (long long)need);
+    return ssp::launch_posteriors_tc(feats, seg_offsets, n_segs, total_frames, pack, L, out_resp, out_label, out_frame_lse,
+                                     workspace, reuse_images != 0, st);
+  }
+  if (dims->n_models != 1) {
+    ssp::set_error("ssp_gmm_posteriors: per-segment models need the tensor-core path (D <= 39, n_models <= %d)",
+                   ssp::kMaxTrainModels);
+    return SSP_EUNSUP;
+  }
+  const int64_t need = ssp::posteriors_simt_workspace_bytes(total_frames, n_segs);
+  SSP_REQUIRE(workspace && workspace_bytes >= need,
+              "ssp_gmm_posteriors: workspace of %lld bytes, need %lld (ssp_gmm_posteriors_workspace_bytes)",
+              (long long)(workspace ? workspace_bytes : 0), (long long)need);
+  return ssp::launch_posteriors_simt(feats, seg_offsets, n_segs, total_frames, pack, L, out_resp, out_label, out_frame_lse,
+                                     workspace, st);
+}

@@ -217,6 +217,17 @@ int64_t score_sv_workspace_bytes(const SvLayout& L, int64_t total_frames);
 int launch_score_sv(const float* feats, const int64_t* offsets, int64_t n_utts, int64_t total_frames, const void* pack,
                     const SvLayout& L, bool normalize, double* scores, float* frame_lse, void* workspace, cudaStream_t st);
 int64_t stats_tc_workspace_bytes(const PackLayout& L, int64_t total_frames, int64_t n_segs);
+int launch_posteriors_tc(const float* feats, const int64_t* seg_offsets, int64_t n_segs, int64_t total_frames, const void* pack,
+                         const PackLayout& L, float* out_resp, int64_t* out_label, float* out_frame_lse, void* workspace,
+                         bool reuse_images, cudaStream_t st);
+// workspace of the CUDA-core posterior path: per-segment sums of the scoring kernel, then the per-frame lse
+inline int64_t posteriors_simt_lse_offset(int64_t n_segs) { return (8 * n_segs + 255) / 256 * 256; }
+inline int64_t posteriors_simt_workspace_bytes(int64_t total_frames, int64_t n_segs) {
+  return posteriors_simt_lse_offset(n_segs) + 4 * total_frames;
+}
+int launch_posteriors_simt(const float* feats, const int64_t* seg_offsets, int64_t n_segs, int64_t total_frames,
+                           const void* pack, const PackLayout& L, float* out_resp, int64_t* out_label, float* out_frame_lse,
+                           void* workspace, cudaStream_t st);
 int launch_stats_simt(const float* feats, const int64_t* seg_offsets, int64_t n_segs, int64_t total_frames,
                       const void* pack, const PackLayout& L, const float* frame_lse, double* out_n, double* out_f,
                       double* out_s, cudaStream_t st);

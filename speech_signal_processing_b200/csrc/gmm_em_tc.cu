@@ -95,11 +95,14 @@ struct Args {
   int K, D, KDb, n_tiles;
   int per_seg_model;           // 1: segment s is scored under model s (grid z = segment; segments padded to whole Fb images)
   // outputs
-  float* frame_lse;
+  float* frame_lse;          // may be NULL (ssp_gmm_posteriors)
   double* out_n;
   double* out_f;
   double* out_s;
-  double* out_loglik;
+  double* out_loglik;        // may be NULL (ssp_gmm_posteriors)
+  float* out_resp;           // [total_frames][K] (posterior pass)
+  int64_t* out_label;        // [total_frames]    (posterior pass)
+  int resp_vec;              // out_resp rows are 16-byte aligned (K % 4 == 0 and an aligned base): float4 stores
 };
 
 // ------------------------------------------------------------------------------------------------ PTX helpers
@@ -285,10 +288,18 @@ __global__ void __launch_bounds__(256) em_prep_kernel(const Args a) {
   }
 }
 
-// ================================================================================================ pass LSE
+// ================================================================================================ pass LSE / posteriors
 // grid = (image chunks, tile pairs).  Shared memory: the pair's model tiles (BF16 hi + lo) + NS_L Fb stages; tensor
-// memory: 2 tiles x 2 buffers of 128 accumulator columns.
-__global__ void __launch_bounds__(THREADS, 1) gmm_em_lse_kernel(const Args a) {
+// memory: 2 tiles x 2 buffers of 128 accumulator columns.  The epilogue is chosen at compile time:
+//   kEpiLse    (gmm_em_lse_kernel)   (max, sum 2^x) of each 64-component half tile -> partial
+//   kEpiResp   (gmm_em_post_kernel)  gamma = 2^(L - lse2) -> out_resp[frame][comp], live frames and components only
+//   kEpiLabel  (gmm_em_post_kernel)  (max logit, lowest component reaching it) of each half tile -> partial, in the
+//                                    slots of the LSE partials (em_label_merge_kernel reduces them)
+constexpr int kEpiLse = 0, kEpiResp = 1, kEpiLabel = 2;
+
+template <int kEpi>
+__device__ __forceinline__ void logit_pass(const Args& a) {
+  constexpr bool kResp = (kEpi & kEpiResp) != 0, kLabel = (kEpi & kEpiLabel) != 0;
   extern __shared__ __align__(1024) unsigned char smem[];
   const int KDb = a.KDb;
   const uint32_t TB = 512u * (uint32_t)KDb;  // bytes of one image (hi + lo)
@@ -391,8 +402,19 @@ __global__ void __launch_bounds__(THREADS, 1) gmm_em_lse_kernel(const Args a) {
     const uint32_t lane_addr = (uint32_t)(quad * 32) << 16;
     if (t < ntl && i0 < i1) {
       float2* dst = a.partial + (size_t)(2 * (tile0 + t) + half) * a.P + row;
+      const int comp0 = (2 * (tile0 + t) + half) * 64;  // component of column 0 of this thread's half tile
       uint32_t k = 0;
       for (int64_t i = i0; i < i1; ++i, ++k) {
+        // posteriors: the row's frame and merged lse2, loaded before the wait for the logits
+        int live = 0;
+        int64_t frame = 0;
+        float l2 = 0.f;
+        if constexpr (kResp) {
+          const int64_t b = 2 * i + (row >> 6);
+          live = (row & 63) < __ldg(a.blk_nt + b);
+          frame = __ldg(a.blk_t0 + b) + (row & 63);
+          l2 = __ldg(a.lse2 + i * IMG + row) + 12.f;  // undo the gamma scale of the statistics pass: log2(kGammaScale) = 12
+        }
         const uint32_t slot = 2u * (k & 1u) + (uint32_t)t;
         mbar_wait(t_full + slot, (k >> 1) & 1u);
         tc_fence_after();
@@ -403,20 +425,87 @@ __global__ void __launch_bounds__(THREADS, 1) gmm_em_lse_kernel(const Args a) {
         tc_ld_wait2(ra, rb);
         tc_fence_before();
         mbar_arrive(t_empty + slot);
-        float cm = max3(__uint_as_float(ra[0]), __uint_as_float(ra[1]), __uint_as_float(rb[0]));
+        if constexpr (kEpi == kEpiLse) {
+          float cm = max3(__uint_as_float(ra[0]), __uint_as_float(ra[1]), __uint_as_float(rb[0]));
 #pragma unroll
-        for (int e = 2; e < 32; e += 2) cm = max3(cm, __uint_as_float(ra[e]), __uint_as_float(ra[e + 1]));
+          for (int e = 2; e < 32; e += 2) cm = max3(cm, __uint_as_float(ra[e]), __uint_as_float(ra[e + 1]));
 #pragma unroll
-        for (int e = 1; e < 31; e += 2) cm = max3(cm, __uint_as_float(rb[e]), __uint_as_float(rb[e + 1]));
-        cm = fmaxf(cm, __uint_as_float(rb[31]));
-        const float s = exp_sum32(ra, cm) + exp_sum32(rb, cm);
-        dst[i * IMG] = make_float2(cm, s);
+          for (int e = 1; e < 31; e += 2) cm = max3(cm, __uint_as_float(rb[e]), __uint_as_float(rb[e + 1]));
+          cm = fmaxf(cm, __uint_as_float(rb[31]));
+          const float s = exp_sum32(ra, cm) + exp_sum32(rb, cm);
+          dst[i * IMG] = make_float2(cm, s);
+        }
+        if constexpr (kLabel) {
+          // strict > in component order: the lowest index wins a tie (numpy's argmax); padded components never compete
+          const int n_live = a.K - comp0;  // columns of real components (may be <= 0: a half tile of padding)
+          float bm = -3.0e38f;
+          int bi = 0;
+#pragma unroll
+          for (int e = 0; e < 32; ++e) {
+            const float v = __uint_as_float(ra[e]);
+            if (e < n_live && v > bm) { bm = v; bi = e; }
+          }
+#pragma unroll
+          for (int e = 0; e < 32; ++e) {
+            const float v = __uint_as_float(rb[e]);
+            if (32 + e < n_live && v > bm) { bm = v; bi = 32 + e; }
+          }
+          dst[i * IMG] = make_float2(bm, __int_as_float(comp0 + bi));
+        }
+        if constexpr (kResp) {
+          if (live) {
+            float* out = a.out_resp + frame * a.K + comp0;
+            if (a.resp_vec && comp0 + 64 <= a.K) {
+              float4* o4 = reinterpret_cast<float4*>(out);
+#pragma unroll
+              for (int q = 0; q < 8; ++q)
+                __stcs(o4 + q, make_float4(ex2(__uint_as_float(ra[4 * q]) - l2), ex2(__uint_as_float(ra[4 * q + 1]) - l2),
+                                           ex2(__uint_as_float(ra[4 * q + 2]) - l2), ex2(__uint_as_float(ra[4 * q + 3]) - l2)));
+#pragma unroll
+              for (int q = 0; q < 8; ++q)
+                __stcs(o4 + 8 + q, make_float4(ex2(__uint_as_float(rb[4 * q]) - l2), ex2(__uint_as_float(rb[4 * q + 1]) - l2),
+                                               ex2(__uint_as_float(rb[4 * q + 2]) - l2), ex2(__uint_as_float(rb[4 * q + 3]) - l2)));
+            } else {
+#pragma unroll
+              for (int e = 0; e < 32; ++e)
+                if (comp0 + e < a.K) __stcs(out + e, ex2(__uint_as_float(ra[e]) - l2));
+#pragma unroll
+              for (int e = 0; e < 32; ++e)
+                if (comp0 + 32 + e < a.K) __stcs(out + 32 + e, ex2(__uint_as_float(rb[e]) - l2));
+            }
+          }
+        }
       }
     }
   }
   tc_fence_before();
   __syncthreads();
   if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+}
+
+__global__ void __launch_bounds__(THREADS, 1) gmm_em_lse_kernel(const Args a) { logit_pass<kEpiLse>(a); }
+
+template <int kEpi>
+__global__ void __launch_bounds__(THREADS, 1) gmm_em_post_kernel(const Args a) { logit_pass<kEpi>(a); }
+
+// label partials -> out_label: thread == padded frame; partial slots ascend with the component index, so strict > keeps
+// the lowest index of a tie
+__global__ void __launch_bounds__(256) em_label_merge_kernel(const Args a) {
+  const int64_t n_rows = ((a.blk_start[a.n_segs] + 1) & ~(int64_t)1) * BLK;
+  const int n_part = 2 * a.n_tiles;
+  for (int64_t p = (int64_t)blockIdx.x * 256 + threadIdx.x; p < n_rows; p += (int64_t)gridDim.x * 256) {
+    const int64_t b = p >> 6;
+    const int r = (int)(p & 63);
+    if (r >= __ldg(a.blk_nt + b)) continue;
+    const float2 q0 = __ldg(a.partial + p);
+    float bm = q0.x, bi = q0.y;
+#pragma unroll 4
+    for (int y = 1; y < n_part; ++y) {
+      const float2 q = __ldg(a.partial + (size_t)y * a.P + p);
+      if (q.x > bm) { bm = q.x; bi = q.y; }
+    }
+    a.out_label[__ldg(a.blk_t0 + b) + r] = __float_as_int(bi);
+  }
 }
 
 // partials -> lse2 per padded frame, frame_lse per frame, log-likelihood per segment.  Persistent CTAs walk groups of 4
@@ -434,7 +523,7 @@ __global__ void __launch_bounds__(256) em_merge_kernel(const Args a) {
     double tot = acc;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) tot += __shfl_xor_sync(0xffffffffu, tot, o);
-    if (lane == 0 && seg_acc >= 0 && tot != 0.0) atomicAdd(a.out_loglik + seg_acc, tot);
+    if (lane == 0 && seg_acc >= 0 && tot != 0.0 && a.out_loglik) atomicAdd(a.out_loglik + seg_acc, tot);
     acc = 0.0;
   };
   for (int64_t b = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 6); b < nb2; b += (int64_t)gridDim.x * 4) {
@@ -459,7 +548,7 @@ __global__ void __launch_bounds__(256) em_merge_kernel(const Args a) {
       }
       lse2 = m + lg2(s);
       ll = lse2 * 0.69314718055994530942f;
-      a.frame_lse[a.blk_t0[b] + r] = ll;
+      if (a.frame_lse) a.frame_lse[a.blk_t0[b] + r] = ll;
     }
     a.lse2[p] = lse2 < 1.0e38f ? lse2 - 12.f : lse2;   // log2(kGammaScale) = 12
     if (seg != seg_acc) {
@@ -727,21 +816,23 @@ int64_t stats_tc_workspace_bytes(const PackLayout& L, int64_t total_frames, int6
   return stats_tc_supported(L) ? (int64_t)em::ws_layout(L, total_frames, n_segs).bytes : 0;
 }
 
-int launch_stats_tc(const float* feats, const int64_t* seg_offsets, int64_t n_segs, int64_t total_frames, const void* pack,
-                    const PackLayout& L, float* frame_lse, double* out_n, double* out_f, double* out_s, double* out_loglik,
-                    void* workspace, bool reuse_images, cudaStream_t st) {
-  using namespace em;
-  SSP_CUDA_OK(cudaMemsetAsync(out_loglik, 0, sizeof(double) * n_segs, st));
-  if (total_frames == 0) return SSP_OK;
-  static int num_sms = 0;
-  if (num_sms == 0) {
+static int g_num_sms = 0;
+static int query_sms() {
+  if (g_num_sms == 0) {
     int dev = 0;
     SSP_CUDA_OK(cudaGetDevice(&dev));
-    SSP_CUDA_OK(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev));
+    SSP_CUDA_OK(cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev));
   }
-  const Ws w = ws_layout(L, total_frames, n_segs);
+  return SSP_OK;
+}
+
+// Arguments shared by the statistics and posterior calls: the workspace carve-up (images at the same place for both) and
+// the model.  Outputs are left NULL.
+static em::Args em_args(const float* feats, const int64_t* seg_offsets, int64_t n_segs, int64_t total_frames, const void* pack,
+                        const PackLayout& L, const em::Ws& w, void* workspace) {
+  using namespace em;
   unsigned char* base = (unsigned char*)workspace;
-  Args a;
+  Args a = {};
   a.feats = feats;
   a.seg = seg_offsets;
   a.n_segs = n_segs;
@@ -762,40 +853,78 @@ int launch_stats_tc(const float* feats, const int64_t* seg_offsets, int64_t n_se
   a.KDb = w.KDb;
   a.n_tiles = L.Kp / BN;
   a.per_seg_model = L.n_models > 1 ? 1 : 0;
-  a.frame_lse = frame_lse;
-  a.out_n = out_n;
-  a.out_f = out_f;
-  a.out_s = out_s;
-  a.out_loglik = out_loglik;
+  return a;
+}
+
+// grids of the passes: the number of blocks is a device value (segment padding); size them from its host-side bounds
+struct EmGrid {
+  int n_pairs;
+  unsigned gz;
+  int64_t gx_l, gx_s;  // image chunks of the logit passes, block chunks of the statistics pass
+  size_t smem_lse;
+};
+static int em_grid(const em::Args& a, const em::Ws& w, int64_t n_segs, int64_t total_frames, const char* who, EmGrid* g) {
+  using namespace em;
+  const int rc = query_sms();
+  if (rc != SSP_OK) return rc;
+  const int sms = g_num_sms;
+  g->n_pairs = (a.n_tiles + 1) / 2;
+  const int64_t nb_lo = (total_frames + BLK - 1) / BLK;
+  g->gz = a.per_seg_model ? (unsigned)n_segs : 1u;
+  SSP_REQUIRE(!a.per_seg_model || n_segs <= 65535, "%s: %lld per-segment models (at most 65535)", who, (long long)n_segs);
+  int64_t gx = sms / ((int64_t)g->n_pairs * g->gz);
+  if (gx < 1) gx = 1;
+  g->gx_l = min(gx, (nb_lo + 1) / 2);
+  g->gx_s = min(gx, nb_lo);
+  g->smem_lse = (2 + NS_L) * w.img_bytes() + 16 * sizeof(uint64_t) + 64;
+  return SSP_OK;
+}
+
+// plan + images (skipped on reuse), then the LSE pass and the merge: lse2 per padded frame (+ frame_lse / loglik if set)
+static int em_prepare_and_lse(em::Args& a, const em::Ws& w, const EmGrid& g, bool reuse_images, bool lse, cudaStream_t st) {
+  using namespace em;
   if (!reuse_images) {
     em_plan_kernel<<<1, 1024, 0, st>>>(a);
     SSP_LAUNCH_CHECK("em_plan_kernel");
     em_prep_kernel<<<(unsigned)w.nb_max, 256, 0, st>>>(a);
     SSP_LAUNCH_CHECK("em_prep_kernel");
   }
-  const int n_pairs = (a.n_tiles + 1) / 2;
-  // the number of blocks is a device value (segment padding); size the grids from its host-side bounds
-  const int64_t nb_lo = (total_frames + BLK - 1) / BLK;
-  const unsigned gz = a.per_seg_model ? (unsigned)n_segs : 1u;
-  SSP_REQUIRE(gz <= 65535u, "ssp_gmm_stats: %lld per-segment models (at most 65535)", (long long)n_segs);
-  int64_t gx = num_sms / ((int64_t)n_pairs * gz);
-  if (gx < 1) gx = 1;
-  const int64_t gx_l = min(gx, (nb_lo + 1) / 2), gx_s = min(gx, nb_lo);
-  const size_t TB = w.img_bytes();
-  const size_t smem_lse = (2 + NS_L) * TB + 16 * sizeof(uint64_t) + 64;
-  const size_t smem_stats = 2 * TB + p3::NF * (TB / 2 + 256) + p3::NX * (TB / 2) + (13 + 2 * p3::NF + 2 * p3::NX) * sizeof(uint64_t) + 64;
-  SSP_CUDA_OK(cudaFuncSetAttribute(gmm_em_lse_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_lse));
-  gmm_em_lse_kernel<<<dim3((unsigned)gx_l, (unsigned)n_pairs, gz), THREADS, smem_lse, st>>>(a);
+  if (!lse) return SSP_OK;
+  SSP_CUDA_OK(cudaFuncSetAttribute(gmm_em_lse_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem_lse));
+  gmm_em_lse_kernel<<<dim3((unsigned)g.gx_l, (unsigned)g.n_pairs, g.gz), THREADS, g.smem_lse, st>>>(a);
   SSP_LAUNCH_CHECK("gmm_em_lse_kernel");
   {
-    const int64_t groups = (w.nb_max + 3) / 4, cap = 8 * (int64_t)num_sms;
+    const int64_t groups = (w.nb_max + 3) / 4, cap = 8 * (int64_t)g_num_sms;
     em_merge_kernel<<<(unsigned)(groups < cap ? groups : cap), 256, 0, st>>>(a);
   }
   SSP_LAUNCH_CHECK("em_merge_kernel");
+  return SSP_OK;
+}
+
+int launch_stats_tc(const float* feats, const int64_t* seg_offsets, int64_t n_segs, int64_t total_frames, const void* pack,
+                    const PackLayout& L, float* frame_lse, double* out_n, double* out_f, double* out_s, double* out_loglik,
+                    void* workspace, bool reuse_images, cudaStream_t st) {
+  using namespace em;
+  SSP_CUDA_OK(cudaMemsetAsync(out_loglik, 0, sizeof(double) * n_segs, st));
+  if (total_frames == 0) return SSP_OK;
+  const Ws w = ws_layout(L, total_frames, n_segs);
+  Args a = em_args(feats, seg_offsets, n_segs, total_frames, pack, L, w, workspace);
+  a.frame_lse = frame_lse;
+  a.out_n = out_n;
+  a.out_f = out_f;
+  a.out_s = out_s;
+  a.out_loglik = out_loglik;
+  EmGrid g;
+  int rc = em_grid(a, w, n_segs, total_frames, "ssp_gmm_stats", &g);
+  if (rc != SSP_OK) return rc;
+  rc = em_prepare_and_lse(a, w, g, reuse_images, true, st);
+  if (rc != SSP_OK) return rc;
+  const size_t TB = w.img_bytes();
+  const size_t smem_stats = 2 * TB + p3::NF * (TB / 2 + 256) + p3::NX * (TB / 2) + (13 + 2 * p3::NF + 2 * p3::NX) * sizeof(uint64_t) + 64;
 #define SSP_EM_STATS(ks)                                                                                                  \
   case ks:                                                                                                                \
     SSP_CUDA_OK(cudaFuncSetAttribute(gmm_em_stats_kernel<ks>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_stats)); \
-    gmm_em_stats_kernel<ks><<<dim3((unsigned)gx_s, (unsigned)n_pairs, gz), p3::THREADS_S, smem_stats, st>>>(a);         \
+    gmm_em_stats_kernel<ks><<<dim3((unsigned)g.gx_s, (unsigned)g.n_pairs, g.gz), p3::THREADS_S, smem_stats, st>>>(a);   \
     break;
   switch (w.KDb >> 4) {
     SSP_EM_STATS(1) SSP_EM_STATS(2) SSP_EM_STATS(3) SSP_EM_STATS(4) SSP_EM_STATS(5)
@@ -803,6 +932,45 @@ int launch_stats_tc(const float* feats, const int64_t* seg_offsets, int64_t n_se
   }
 #undef SSP_EM_STATS
   SSP_LAUNCH_CHECK("gmm_em_stats_kernel");
+  return SSP_OK;
+}
+
+int launch_posteriors_tc(const float* feats, const int64_t* seg_offsets, int64_t n_segs, int64_t total_frames, const void* pack,
+                         const PackLayout& L, float* out_resp, int64_t* out_label, float* out_frame_lse, void* workspace,
+                         bool reuse_images, cudaStream_t st) {
+  using namespace em;
+  if (total_frames == 0) return SSP_OK;
+  const Ws w = ws_layout(L, total_frames, n_segs);
+  Args a = em_args(feats, seg_offsets, n_segs, total_frames, pack, L, w, workspace);
+  a.frame_lse = out_frame_lse;
+  a.out_resp = out_resp;
+  a.out_label = out_label;
+  a.resp_vec = (L.K % 4 == 0 && ((uintptr_t)out_resp & 15) == 0) ? 1 : 0;
+  EmGrid g;
+  int rc = em_grid(a, w, n_segs, total_frames, "ssp_gmm_posteriors", &g);
+  if (rc != SSP_OK) return rc;
+  // labels alone need no log-sum-exp: the argmax of the logits is the argmax of the posteriors
+  rc = em_prepare_and_lse(a, w, g, reuse_images, out_resp || out_frame_lse, st);
+  if (rc != SSP_OK) return rc;
+  if (!out_resp && !out_label) return SSP_OK;
+  const dim3 grid((unsigned)g.gx_l, (unsigned)g.n_pairs, g.gz);
+#define SSP_EM_POST(epi, name)                                                                                          \
+  SSP_CUDA_OK(cudaFuncSetAttribute(gmm_em_post_kernel<epi>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem_lse)); \
+  gmm_em_post_kernel<epi><<<grid, THREADS, g.smem_lse, st>>>(a);                                                        \
+  SSP_LAUNCH_CHECK(name);
+  if (out_resp && out_label) {
+    SSP_EM_POST(kEpiResp | kEpiLabel, "gmm_em_post_kernel<resp+labels>")
+  } else if (out_resp) {
+    SSP_EM_POST(kEpiResp, "gmm_em_post_kernel<resp>")
+  } else {
+    SSP_EM_POST(kEpiLabel, "gmm_em_post_kernel<labels>")
+  }
+#undef SSP_EM_POST
+  if (out_label) {
+    const int64_t blocks = (w.P + 255) / 256, cap = 8 * (int64_t)g_num_sms;
+    em_label_merge_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, st>>>(a);
+    SSP_LAUNCH_CHECK("em_label_merge_kernel");
+  }
   return SSP_OK;
 }
 

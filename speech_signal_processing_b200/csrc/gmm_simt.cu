@@ -101,6 +101,100 @@ int launch_score_simt(const float* feats, const int64_t* offsets, int64_t n_utts
 }
 
 // ------------------------------------------------------------------------------------------------
+// Posteriors (D > 39, one model).  Same block shape and logit arithmetic as gmm_score_simt_kernel, whose per-frame lse
+// this pass consumes: gamma[t, c] = exp(L[t, c] - lse_t) is staged per 32 components in shared memory and written as
+// rows of 32 consecutive components (one 128-byte row segment per warp store); the label is the lowest component index
+// reaching the maximum logit.
+// ------------------------------------------------------------------------------------------------
+template <int DP>
+__global__ void __launch_bounds__(128) gmm_post_simt_kernel(const float* __restrict__ feats, int64_t total_frames,
+                                                           const float2* __restrict__ ab, const float* __restrict__ cst,
+                                                           int K, int Kp, int D, const float* __restrict__ frame_lse,
+                                                           float* __restrict__ out_resp, int64_t* __restrict__ out_label) {
+  __shared__ __align__(16) float2 s_ab[kSC * DP];
+  __shared__ float s_c[kSC];
+  __shared__ float s_g[kSF * (kSC + 1)];
+  __shared__ float s_m[kSF];
+  __shared__ int s_i[kSF];
+  const int tid = threadIdx.x, f = tid % kSF, h = tid / kSF;
+  const int64_t f0 = (int64_t)blockIdx.x * kSF, frame = f0 + f;
+  const bool valid = frame < total_frames;
+  float x[DP];
+#pragma unroll
+  for (int d = 0; d < DP; ++d) x[d] = (valid && d < D) ? feats[frame * D + d] : 0.f;
+  const float lse = (valid && out_resp) ? frame_lse[frame] : 0.f;
+  float bm = -3.0e38f;
+  int bi = 0;
+  for (int c0 = 0; c0 < Kp; c0 += kSC) {
+    __syncthreads();
+    for (int i = tid; i < kSC * DP; i += 128) s_ab[i] = ab[(int64_t)c0 * DP + i];
+    if (tid < kSC) s_c[tid] = cst[c0 + tid];
+    __syncthreads();
+#pragma unroll 4
+    for (int j = 0; j < kSC / 2; ++j) {
+      const int c = h * (kSC / 2) + j;
+      const float4* row = reinterpret_cast<const float4*>(s_ab + c * DP);
+      float acc0 = s_c[c], acc1 = 0.f;
+#pragma unroll
+      for (int d = 0; d < DP; d += 2) {
+        float4 p = row[d >> 1];
+        acc0 = fmaf(x[d], fmaf(p.y, x[d], p.x), acc0);
+        acc1 = fmaf(x[d + 1], fmaf(p.w, x[d + 1], p.z), acc1);
+      }
+      const float l = acc0 + acc1;
+      if (c0 + c < K && l > bm) { bm = l; bi = c0 + c; }
+      if (out_resp) s_g[f * (kSC + 1) + c] = expf(l - lse);
+    }
+    if (out_resp) {
+      __syncthreads();
+      // warp w writes rows w, w + 4, ...: 32 lanes = 32 consecutive components of one frame
+      const int lane = tid & 31;
+      for (int r = tid >> 5; r < kSF; r += 4)
+        if (f0 + r < total_frames && c0 + lane < K) __stcs(out_resp + (f0 + r) * K + c0 + lane, s_g[r * (kSC + 1) + lane]);
+    }
+  }
+  if (out_label) {
+    // half 0 holds components [c0, c0 + 16) of every chunk, half 1 [c0 + 16, c0 + 32): on a tie the lower index wins
+    if (h == 1) { s_m[f] = bm; s_i[f] = bi; }
+    __syncthreads();
+    if (h == 0 && valid) {
+      const float m1 = s_m[f];
+      const int i1 = s_i[f];
+      out_label[frame] = (m1 > bm || (m1 == bm && i1 < bi)) ? i1 : bi;
+    }
+  }
+}
+
+int launch_posteriors_simt(const float* feats, const int64_t* seg_offsets, int64_t n_segs, int64_t total_frames,
+                           const void* pack, const PackLayout& L, float* out_resp, int64_t* out_label, float* out_frame_lse,
+                           void* workspace, cudaStream_t st) {
+  if (total_frames == 0) return SSP_OK;
+  const char* base = (const char*)pack;
+  const float2* ab = (const float2*)(base + L.off_ab);
+  const float* cst = (const float*)(base + L.off_cst);
+  // workspace: per-segment sums of gmm_score_simt_kernel (unused), then the per-frame lse unless the caller takes it
+  double* seg_sums = (double*)workspace;
+  float* lse = out_frame_lse ? out_frame_lse : (float*)((char*)workspace + posteriors_simt_lse_offset(n_segs));
+  if (out_resp || out_frame_lse) {
+    const int rc = launch_score_simt(feats, seg_offsets, n_segs, total_frames, pack, L, false, seg_sums, lse, st);
+    if (rc != SSP_OK) return rc;
+  }
+  if (!out_resp && !out_label) return SSP_OK;
+  const unsigned grid = (unsigned)((total_frames + kSF - 1) / kSF);
+#define SSP_CASE(dp)                                                                                                   \
+  case dp:                                                                                                             \
+    gmm_post_simt_kernel<dp><<<grid, 128, 0, st>>>(feats, total_frames, ab, cst, L.K, L.Kp, L.D, lse, out_resp, out_label); \
+    break;
+  switch (L.DP) {  // the tensor-core pass serves D <= 39
+    SSP_CASE(40) SSP_CASE(64) SSP_CASE(80)
+    default: SSP_REQUIRE(false, "unsupported padded feature dim %d", L.DP);
+  }
+#undef SSP_CASE
+  SSP_LAUNCH_CHECK("gmm_post_simt_kernel");
+  return SSP_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
 // Statistics pass.  grid = (frame chunks, component groups of 64), block = 256.
 //   phase A: thread = (frame t = tid%64, quarter q): gamma[t, c] = exp(L[t,c] - lse_t) for 16 components
 //   phase B: thread = (component c = tid%64, quarter q): F/S accumulators for DP/4 dims (+N on q == 0)

@@ -3,9 +3,10 @@
 The reference binds ``sklearn.mixture.GaussianMixture`` at GMM_UBM.py:16 and uses exactly
 ``GaussianMixture(n_components=K, covariance_type='diag').fit(X)`` (:158-160, :169-170) and
 ``.score(X)`` (:185, :194), plus pickling of the fitted objects (:173-179).  :class:`GaussianMixture`
-mirrors that surface (same constructor names, attributes and error behaviour); the arithmetic runs
+mirrors that surface (same constructor names, attributes and error behaviour) and adds the rest of
+sklearn's inference calls (``predict_proba``, ``predict``, ``fit_predict``, ``bic``, ``aic``); the arithmetic runs
 in the CUDA library: ``ssp_gmm_pack_models`` / ``ssp_gmm_score`` / ``ssp_gmm_stats`` /
-``ssp_gmm_mstep``.  :class:`ModelSet` + :func:`score_matrix` are the batched form the reference
+``ssp_gmm_posteriors`` / ``ssp_gmm_mstep``.  :class:`ModelSet` + :func:`score_matrix` are the batched form the reference
 lacks (all utterances x all models in one launch instead of S*N*2 Python calls).
 """
 from __future__ import annotations
@@ -21,6 +22,9 @@ PRECISIONS = {"fp32": _lib.PREC_FP32, "tf32": _lib.PREC_TF32, "tf32x2": _lib.PRE
 # Below this many components the single-pass TF32 rounding no longer averages out to 1e-4 of the utterance score /
 # 1e-3 of an LLR (SURVEY 8(c)); "auto" then takes the 3-pass (FP32-grade) tensor rung.
 SINGLE_PASS_MIN_COMPONENTS = 512
+# GaussianMixture.predict_proba computes the posteriors in frame chunks of at most this many bytes of float32 output, so
+# the device buffer stays bounded whatever the number of frames
+PROBA_CHUNK_BYTES = 1 << 30
 
 
 def resolve_precision(precision: str, n_comp: int, n_feat: int) -> str:
@@ -156,9 +160,51 @@ class ModelSet:
         return n, f, s, ll
 
 
+    @_lib.on_device
+    def posteriors(self, feats, seg_offsets, resp=True, labels=False, workspace=None, reuse_images=False):
+        """(resp (T, K) float32 cuda | None, labels (T,) int64 cuda | None, frame_lse (T,) float32 cuda | None): frame
+        posteriors and/or the most probable component of every frame (lowest index on ties), under this set's single
+        model or -- one model per segment -- segment s under model s, as in :meth:`stats`.  ``frame_lse`` (the per-frame
+        log-likelihood) comes with ``resp``; labels alone skip the log-sum-exp pass and return None there.
+
+        Always FP32 grade (``ssp_gmm_posteriors``): the 3 x BF16 tensor-core logits of :meth:`stats` for D <= 39, the
+        FP32 CUDA-core kernels above.  ``workspace`` / ``reuse_images`` as in :meth:`stats`, whose workspace (and frame
+        images) this call shares."""
+        torch = _lib.require_cuda()
+        seg_offsets = np.asarray(seg_offsets, dtype=np.int64)
+        n_segs, total = len(seg_offsets) - 1, int(seg_offsets[-1])
+        if self.n_models != 1 and self.n_models != n_segs:
+            raise ValueError("posteriors are taken under one model for all segments, or under one model per segment "
+                             f"(got {self.n_models} models for {n_segs} segments)")
+        if feats.shape[1] != self.n_feat:
+            raise ValueError(f"X has {feats.shape[1]} features, but the models expect {self.n_feat}")
+        if not (resp or labels):
+            raise ValueError("posteriors: ask for resp, labels or both")
+        g = torch.empty((total, self.n_comp), dtype=torch.float32, device=self.device) if resp else None
+        lab = torch.empty(total, dtype=torch.int64, device=self.device) if labels else None
+        lse = torch.empty(total, dtype=torch.float32, device=self.device) if resp else None
+        d_off = torch.as_tensor(seg_offsets, device=self.device)
+        ws_bytes = int(self.lib.ssp_gmm_posteriors_workspace_bytes(C.byref(self.dims), total, n_segs))
+        if workspace is None:
+            workspace = getattr(self, "_ws", None)
+            if workspace is None:
+                workspace = self._ws = StatsWorkspace(self.device)
+            reuse_images = False
+        buf = workspace.reserve(ws_bytes)
+        rc = self.lib.ssp_gmm_posteriors(_lib.ptr(feats), _lib.ptr(d_off), n_segs, total, _lib.ptr(self.pack),
+                                         C.byref(self.dims), _lib.ptr(g), _lib.ptr(lab), _lib.ptr(lse),
+                                         _lib.ptr(buf) if ws_bytes else None, ws_bytes,
+                                         int(bool(reuse_images) and workspace.valid), _lib.stream_ptr())
+        _lib.check(rc, "ssp_gmm_posteriors")
+        workspace.valid = True
+        self._keep = d_off
+        return g, lab, lse
+
+
 class StatsWorkspace:
-    """Scratch of ``ssp_gmm_stats`` (operand images of the frames + log-sum-exp partials).  ``valid`` says that it holds
-    the images of the frames it was last used with; growing it invalidates them."""
+    """Scratch of ``ssp_gmm_stats`` and ``ssp_gmm_posteriors`` (operand images of the frames + log-sum-exp partials; the
+    two calls lay it out alike).  ``valid`` says that it holds the images of the frames it was last used with; growing it
+    invalidates them."""
 
     def __init__(self, device):
         self.device, self.buf, self.valid = device, None, False
@@ -274,6 +320,11 @@ class GaussianMixture:
     random frames (sklearn's KMeans++ stream is not reproduced: the reference leaves
     ``random_state=None``, so its own runs are not reproducible either -- SURVEY F7); parity with
     sklearn is defined for given ``weights_init/means_init/precisions_init``.
+
+    Inference beyond ``score`` follows sklearn too: ``predict_proba`` (float64 posteriors), ``predict`` and
+    ``fit_predict`` (int64 labels, the lowest component index on ties), ``bic`` and ``aic``.  Posteriors and labels are
+    always computed at FP32 grade (``ssp_gmm_posteriors``: 3 x BF16 tensor-core logits for D <= 39, FP32 CUDA cores
+    above), whatever ``precision`` says.
 
     ``precision`` selects the scoring kernel of ``score`` / ``score_samples``: ``"fp32"`` (default: CUDA-core
     FMA, ~1e-7 relative, safe for any data) or ``"tf32"`` (tcgen05 tensor cores; meant for CMVN-normalised
@@ -455,6 +506,20 @@ class GaussianMixture:
 
     def fit(self, X, y=None):
         """Estimate parameters with EM (sklearn/mixture/_base.py:203-312)."""
+        self._fit(X)
+        return self
+
+    def fit_predict(self, X, y=None):
+        """``fit(X)``, then the label of every frame from a final E-step under the best parameters (sklearn
+        _base.py ``fit_predict``), so that it equals ``fit(X).predict(X)``.  The final E-step reuses the frames' operand
+        images of the EM run."""
+        feats, workspace = self._fit(X)
+        _, labels, _ = self._model_set().posteriors(feats, np.array([0, feats.shape[0]]), resp=False, labels=True,
+                                                    workspace=workspace, reuse_images=True)
+        return labels.cpu().numpy()
+
+    def _fit(self, X):
+        """EM; returns the device frames and the :class:`StatsWorkspace` holding their operand images."""
         torch = _lib.require_cuda()
         self._check()
         dev = torch.device(f"cuda:{torch.cuda.current_device()}")
@@ -501,7 +566,7 @@ class GaussianMixture:
                              "number of components, increase reg_covar, or scale the input data.")
         self.converged_, self.n_iter_, self.lower_bound_, self.lower_bounds_ = converged, n_iter, lower, bounds
         self._ms = None
-        return self
+        return feats, workspace
 
     # ------------------------------------------------------------------ scoring
     def score_samples(self, X):
@@ -517,6 +582,51 @@ class GaussianMixture:
         feats = _as_feats(X, ms.device)
         scores, _ = ms.score(feats, np.array([0, feats.shape[0]]), precision=self.precision)
         return float(scores[0, 0].item())
+
+    # ------------------------------------------------------------------ posteriors and model selection
+    def _frames(self, X):
+        ms = self._model_set()
+        feats = _as_feats(X, ms.device)
+        if feats.shape[1] != ms.n_feat:
+            raise ValueError(f"X has {feats.shape[1]} features, but GaussianMixture is expecting {ms.n_feat} features as input.")
+        return ms, feats
+
+    def predict_proba(self, X):
+        """Posterior of every component for every frame, float64 (T, K) (sklearn/mixture/_base.py ``predict_proba``).
+        Computed at FP32 grade whatever ``precision`` says (``ssp_gmm_posteriors``), in frame chunks of at most
+        ``PROBA_CHUNK_BYTES`` of device output, each copied into the host result as it completes."""
+        ms, feats = self._frames(X)
+        n, k = feats.shape[0], ms.n_comp
+        out = np.empty((n, k), dtype=np.float64)
+        step = max(1, PROBA_CHUNK_BYTES // (4 * k))
+        workspace = StatsWorkspace(ms.device)
+        for a in range(0, n, step):
+            b = min(n, a + step)
+            g, _, _ = ms.posteriors(feats[a:b], np.array([0, b - a]), resp=True, workspace=workspace)
+            out[a:b] = g.cpu().numpy()
+        return out
+
+    def predict(self, X):
+        """Most probable component of every frame, int64 (T,) (sklearn/mixture/_base.py ``predict``; the lowest index
+        on ties).  FP32 grade whatever ``precision`` says."""
+        ms, feats = self._frames(X)
+        _, labels, _ = ms.posteriors(feats, np.array([0, feats.shape[0]]), resp=False, labels=True)
+        return labels.cpu().numpy()
+
+    def _n_parameters(self):
+        """Free parameters of a diagonal model: K D variances, K D means and K - 1 weights."""
+        k, d = np.shape(self.means_)
+        return int(2 * k * d + k - 1)
+
+    def bic(self, X):
+        """Bayesian information criterion on X (sklearn/mixture/_gaussian_mixture.py ``bic``); lower is better."""
+        n = int(X.shape[0]) if hasattr(X, "shape") else len(X)
+        return -2.0 * self.score(X) * n + self._n_parameters() * np.log(n)
+
+    def aic(self, X):
+        """Akaike information criterion on X (sklearn/mixture/_gaussian_mixture.py ``aic``); lower is better."""
+        n = int(X.shape[0]) if hasattr(X, "shape") else len(X)
+        return -2.0 * self.score(X) * n + 2 * self._n_parameters()
 
     # ------------------------------------------------------------------ interchange (SURVEY 8(f).1)
     @classmethod
