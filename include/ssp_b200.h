@@ -233,7 +233,8 @@ int ssp_gmm_score(const float* feats, const int64_t* frame_offsets, int64_t n_ut
  * dims->n_models = number of mean sets S; weights double[K], variances double[K*D], means double[S*K*D] (device).
  * ref_model      (at pack time) index of the reference member: the UBM's own means if they are part of the set,
  *                else any member.  Its per-frame maximum logit also stabilises the exponentials.
- * workspace      device, ssp_gmm_score_shared_workspace_bytes() bytes; may be NULL when that is 0.  Large model sets
+ * workspace      device, ssp_gmm_score_shared_workspace_bytes() bytes, 16-byte aligned (else SSP_EINVAL); may be NULL
+ *                when that is 0.  Large model sets
  *                are scored in groups whose tile images stay resident in L2 while all frames pass by; the per-frame
  *                exponent stabilisers found while the first group is scored live here (4 bytes per frame).
  */
@@ -255,7 +256,8 @@ int ssp_gmm_score_shared(const float* feats, const int64_t* frame_offsets, int64
  *   GMM_UBM.py:154-165 as one call per EM iteration (D <= 39, n_models <= 1024).
  * Outputs are ACCUMULATED into (caller zeroes them).
  * frame_lse      device float[total_frames]: per-frame log-likelihood under the model (written by this call)
- * workspace      device, ssp_gmm_stats_workspace_bytes() bytes, 1024-byte aligned.  The tensor-core path (tcgen05,
+ * workspace      device, ssp_gmm_stats_workspace_bytes() bytes, 16-byte aligned (else SSP_EINVAL: the frame images
+ *                are written with 16-byte stores and read by cp.async.bulk).  The tensor-core path (tcgen05,
  *                D <= 39) keeps there (a) the tcgen05 operand images of the frames -- [x, x^2, 1, 1] as BF16 hi + lo
  *                rows and as TF32 hi + lo with the frame index contiguous, segments padded to 64 frames: 12 * roundup(2D+2,
  *                16) bytes per frame, 960 at D = 39 -- and (b) per-component-tile log-sum-exp partials.  A NULL or short
@@ -282,7 +284,8 @@ int64_t ssp_gmm_stats_workspace_bytes(const ssp_gmm_dims* dims, int64_t total_fr
  * out_label      device int64[total_frames] or NULL; at least one of the two (both NULL is SSP_EINVAL).  Labels alone
  *                skip the log-sum-exp pass.
  * out_frame_lse  device float[total_frames] or NULL: per-frame log-likelihood (computed when out_resp or this is set)
- * workspace      device, ssp_gmm_posteriors_workspace_bytes() bytes, 1024-byte aligned.  For D <= 39 it has the layout
+ * workspace      device, ssp_gmm_posteriors_workspace_bytes() bytes, 16-byte aligned (else SSP_EINVAL).  For D <= 39 it
+ *                has the layout
  *                of the ssp_gmm_stats workspace (same size, frame images at the same place), so one workspace serves both
  *                calls on the same frames and reuse_images works across them (label the frames of an EM run
  *                without preparing them again).

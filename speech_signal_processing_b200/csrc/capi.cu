@@ -52,6 +52,11 @@ extern "C" const char* ssp_launch_log(void) {
   return ssp::g_log_text;
 }
 
+// Workspaces of the statistics, posterior and shared-variance calls: the tensor-core kernels write the operand images
+// with 16-byte (uint4) stores and stream them into shared memory with cp.async.bulk, whose global source must be 16-byte
+// aligned.  Every section inside a workspace starts at a multiple of 256 bytes from its base, so the base is what counts.
+static constexpr uintptr_t kWorkspaceAlign = 16;
+
 extern "C" int64_t ssp_gmm_pack_bytes(const ssp_gmm_dims* dims) {
   ssp::PackLayout L;
   if (!ssp::make_layout(dims, &L)) return 0;
@@ -115,6 +120,8 @@ extern "C" int ssp_gmm_score_shared(const float* feats, const int64_t* frame_off
   SSP_REQUIRE(ssp::make_sv_layout(dims, &L), "ssp_gmm_score_shared: unsupported dims");
   SSP_REQUIRE(frame_offsets && pack && out_scores && (feats || total_frames == 0), "ssp_gmm_score_shared: null pointer");
   SSP_REQUIRE(workspace || ssp::score_sv_workspace_bytes(L, total_frames) == 0, "ssp_gmm_score_shared: null workspace");
+  SSP_REQUIRE(((uintptr_t)workspace & (kWorkspaceAlign - 1)) == 0, "ssp_gmm_score_shared: workspace must be %d-byte aligned",
+              (int)kWorkspaceAlign);
   SSP_REQUIRE(n_utts >= 0 && total_frames >= 0, "ssp_gmm_score_shared: negative size");
   SSP_REQUIRE(workspace_bytes >= ssp::score_sv_workspace_bytes(L, total_frames), "ssp_gmm_score_shared: workspace of %lld bytes, need %lld",
               (long long)workspace_bytes, (long long)ssp::score_sv_workspace_bytes(L, total_frames));
@@ -139,6 +146,8 @@ extern "C" int ssp_gmm_stats(const float* feats, const int64_t* seg_offsets, int
               "ssp_gmm_stats: %d models for %lld segments (one model for all segments, or one per segment)", dims->n_models,
               (long long)n_segs);
   SSP_REQUIRE(seg_offsets && pack && frame_lse && out_n && out_f && out_s && out_loglik, "ssp_gmm_stats: null pointer");
+  SSP_REQUIRE(((uintptr_t)workspace & (kWorkspaceAlign - 1)) == 0, "ssp_gmm_stats: workspace must be %d-byte aligned",
+              (int)kWorkspaceAlign);
   SSP_REQUIRE(n_segs >= 0 && total_frames >= 0, "ssp_gmm_stats: negative size");
   if (n_segs == 0) return SSP_OK;
   cudaStream_t st = (cudaStream_t)stream;
@@ -182,6 +191,8 @@ extern "C" int ssp_gmm_posteriors(const float* feats, const int64_t* seg_offsets
               dims->n_models, (long long)n_segs);
   SSP_REQUIRE(out_resp || out_label, "ssp_gmm_posteriors: out_resp and out_label are both NULL (nothing to compute)");
   SSP_REQUIRE(seg_offsets && pack && (feats || total_frames == 0), "ssp_gmm_posteriors: null pointer");
+  SSP_REQUIRE(((uintptr_t)workspace & (kWorkspaceAlign - 1)) == 0, "ssp_gmm_posteriors: workspace must be %d-byte aligned",
+              (int)kWorkspaceAlign);
   SSP_REQUIRE(n_segs >= 0 && total_frames >= 0, "ssp_gmm_posteriors: negative size");
   if (n_segs == 0 || total_frames == 0) return SSP_OK;
   cudaStream_t st = (cudaStream_t)stream;

@@ -16,7 +16,7 @@ from __future__ import annotations
 import numpy as np
 
 from . import _lib
-from .mixture import concat_utterances
+from .mixture import concat_utterances, device_frames
 
 METRICS = {"euclidean": 0, "sqeuclidean": 1, "cityblock": 2}
 
@@ -117,12 +117,9 @@ def _ragged(seqs, dev, what):
     """list of (n_i, dim) / (n_i,) arrays, or a ``(device_feats, offsets)`` tuple -> (feats, offsets numpy, dim)."""
     torch = _lib.require_cuda()
     if isinstance(seqs, tuple) and len(seqs) == 2 and isinstance(seqs[0], torch.Tensor):
-        feats, offs = seqs
-        if feats.ndim != 2 or feats.dtype != torch.float32 or feats.device != dev:
-            raise ValueError(f"{what}: device features must be a 2-D float32 tensor on {dev}")
-        feats, offs = concat_utterances((feats, offs), dev)
-        if len(offs) < 2 or offs[0] != 0 or offs[-1] != len(feats) or np.any(np.diff(offs) < 1):
-            raise ValueError(f"{what}: offsets must start at 0, end at the frame count, and give every sequence a frame")
+        feats, offs = seqs[0], device_frames(seqs[0], seqs[1], dev, what)
+        if len(offs) < 2 or np.any(np.diff(offs) < 1):
+            raise ValueError(f"{what}: offsets must give every sequence a frame")
         return feats, offs, feats.shape[1]
     seqs = [_sequence(s, f"{what}[{k}]") for k, s in enumerate(seqs)]
     if not seqs:

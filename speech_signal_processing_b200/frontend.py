@@ -268,6 +268,8 @@ class FrontEnd:
         self.recipe = recipe
         self.delta_order, self.delta_n, self.cmvn = int(delta_order), int(delta_n), bool(cmvn)
         self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
+        if self.device.index is None:   # "cuda": the current device, named, so that tensors on it compare equal
+            self.device = torch.device("cuda", torch.cuda.current_device())
         fb = np.asarray(recipe.fbank, dtype=np.float64)
         if fb.shape[1] != recipe.nfft // 2 + 1:
             raise ValueError("filterbank must have nfft/2+1 columns")
@@ -351,6 +353,11 @@ class FrontEnd:
     # -- device entry: PCM already resident in HBM --------------------------------------------
     @_lib.on_device
     def extract_device(self, pcm, sample_offsets: np.ndarray, want_log_energy: bool = False, out=None):
+        """``pcm``: 1-D contiguous int16 / float32 tensor on ``self.device``; ``sample_offsets``: 1-D integer host array,
+        never decreasing, within ``[0, len(pcm)]`` (it need not start at 0); ``out``: ``(total frames, out_dim)``
+        contiguous float32 on the device, or None.  Anything else raises before a launch (a PCM dtype other than int16 /
+        float32 is a ``TypeError``, the rest ``ValueError``): the kernel reads ``pcm`` as packed samples and writes
+        ``out`` as packed rows."""
         torch = _lib.require_cuda()
         if pcm.dtype == torch.int16:
             pcm_dtype = 0
@@ -358,8 +365,16 @@ class FrontEnd:
             pcm_dtype = 1
         else:
             raise TypeError("PCM must be int16 or float32")
+        if pcm.dim() != 1 or not pcm.is_contiguous() or pcm.device != self.device:
+            raise ValueError(f"PCM must be a 1-D contiguous tensor on {self.device} (got {pcm.dim()}-D, stride "
+                             f"{tuple(pcm.stride())}, on {pcm.device})")
         cfg = self._cfg(pcm_dtype)
-        sample_offsets = np.asarray(sample_offsets, dtype=np.int64)
+        sample_offsets = np.asarray(sample_offsets)
+        if sample_offsets.ndim != 1 or sample_offsets.dtype.kind not in "iu" or len(sample_offsets) == 0:
+            raise ValueError("sample_offsets must be a non-empty 1-D integer array")
+        sample_offsets = sample_offsets.astype(np.int64, copy=False)
+        if sample_offsets[0] < 0 or sample_offsets[-1] > pcm.shape[0] or np.any(sample_offsets[1:] < sample_offsets[:-1]):
+            raise ValueError(f"sample_offsets must never decrease and stay within [0, {pcm.shape[0]}] (the PCM's samples)")
         n_utts = len(sample_offsets) - 1
         r = self.recipe
         nfr = self.frame_counts(np.diff(sample_offsets))
@@ -368,6 +383,10 @@ class FrontEnd:
         total = int(frame_offsets[-1])
         if out is None:
             out = torch.empty((total, self.out_dim), dtype=torch.float32, device=self.device)
+        elif (tuple(out.shape) != (total, self.out_dim) or out.dtype != torch.float32 or not out.is_contiguous()
+              or out.device != self.device):
+            raise ValueError(f"out must be a contiguous ({total}, {self.out_dim}) float32 tensor on {self.device} (got "
+                             f"{tuple(out.shape)} {out.dtype} on {out.device})")
         log_e = torch.empty(total, dtype=torch.float32, device=self.device) if want_log_energy else None
         if n_utts == 0 or total == 0:
             return out, frame_offsets, log_e

@@ -50,11 +50,45 @@ def _as_feats(x, device):
     return torch.as_tensor(np.ascontiguousarray(x, dtype=np.float32), device=device)
 
 
+def device_frames(feats, offsets, device, what="feats"):
+    """The one rule for frames a caller hands the GMM and DTW kernels on the device -> ``offsets`` as np.int64.
+
+    ``feats`` must be a 2-D float32 torch tensor on ``device`` with contiguous rows (a row range ``x[a:b]`` is fine, a
+    column slice or a transpose is not); ``offsets`` a 1-D integer host array that starts at 0, never decreases and ends
+    at ``feats.shape[0]`` (empty utterances are allowed).  Anything else raises ``ValueError`` before a launch: the
+    kernels read ``feats`` as packed float32 rows through the offsets, so another dtype or layout would be read as
+    wrong numbers, and bad offsets would send them past the buffer.  Nothing is converted: a float64 copy of an EM run's
+    frames would cost as much HBM as the frames themselves.  Checked on the host, with no device read-back."""
+    import torch
+
+    device = torch.device(device)
+    if device.type == "cuda" and device.index is None:
+        device = torch.device("cuda", torch.cuda.current_device())
+    if not isinstance(feats, torch.Tensor):
+        raise ValueError(f"{what}: expected a torch tensor on {device}, got {type(feats).__name__}")
+    if feats.dim() != 2 or feats.dtype != torch.float32:
+        raise ValueError(f"{what}: expected a 2-D float32 tensor, got {feats.dim()}-D {feats.dtype}")
+    if feats.device != device:
+        raise ValueError(f"{what}: the tensor is on {feats.device}, the kernels run on {device}")
+    if not feats.is_contiguous():
+        raise ValueError(f"{what}: rows must be contiguous (stride ({feats.shape[1]}, 1), got {tuple(feats.stride())}); "
+                         "pass .contiguous()")
+    offs = np.asarray(offsets)
+    if offs.ndim != 1 or offs.dtype.kind not in "iu" or len(offs) == 0:
+        raise ValueError(f"{what}: offsets must be a non-empty 1-D integer array (got {offs.ndim}-D {offs.dtype})")
+    offs = offs.astype(np.int64, copy=False)
+    if offs[0] != 0 or offs[-1] != feats.shape[0] or np.any(offs[1:] < offs[:-1]):
+        raise ValueError(f"{what}: offsets must start at 0, never decrease and end at the {feats.shape[0]} rows of the "
+                         f"tensor (got {offs[0]} .. {offs[-1]})")
+    return offs
+
+
 def concat_utterances(utts, device):
-    """list of (T_i, D) arrays -> (feats (sum T, D) cuda, frame_offsets np.int64)."""
+    """list of (T_i, D) arrays -> (feats (sum T, D) cuda, frame_offsets np.int64); a ``(feats, offsets)`` tuple of device
+    frames is passed through after :func:`device_frames` has checked it."""
     torch = _lib.require_cuda()
     if isinstance(utts, tuple) and len(utts) == 2 and isinstance(utts[0], torch.Tensor):
-        return utts[0].contiguous(), np.asarray(utts[1], dtype=np.int64)
+        return utts[0], device_frames(utts[0], utts[1], device)
     lens = np.array([len(u) for u in utts], dtype=np.int64)
     offs = np.zeros(len(utts) + 1, dtype=np.int64)
     np.cumsum(lens, out=offs[1:])
@@ -107,7 +141,7 @@ class ModelSet:
         single pass streams FP16 images of the models) or "auto"
         (:func:`resolve_precision`)."""
         torch = _lib.require_cuda()
-        frame_offsets = np.asarray(frame_offsets, dtype=np.int64)
+        frame_offsets = device_frames(feats, frame_offsets, self.device)
         n_utts, total = len(frame_offsets) - 1, int(frame_offsets[-1])
         precision = resolve_precision(precision, self.n_comp, self.n_feat)
         if feats.shape[1] != self.n_feat:
@@ -131,8 +165,10 @@ class ModelSet:
         ``seg_offsets``; ``reuse_images=True`` then skips the preparation pass that turns the frames into tensor-core
         operand images (EM iterations: the frames never change).  Default: a workspace owned by this model set."""
         torch = _lib.require_cuda()
-        seg_offsets = np.asarray(seg_offsets, dtype=np.int64)
+        seg_offsets = device_frames(feats, seg_offsets, self.device)
         n_segs, total = len(seg_offsets) - 1, int(seg_offsets[-1])
+        if feats.shape[1] != self.n_feat:
+            raise ValueError(f"X has {feats.shape[1]} features, but the models expect {self.n_feat}")
         if self.n_models != 1 and self.n_models != n_segs:
             raise ValueError("statistics are taken under one model for all segments (the UBM), or under one model per "
                              f"segment (got {self.n_models} models for {n_segs} segments)")
@@ -171,7 +207,7 @@ class ModelSet:
         FP32 CUDA-core kernels above.  ``workspace`` / ``reuse_images`` as in :meth:`stats`, whose workspace (and frame
         images) this call shares."""
         torch = _lib.require_cuda()
-        seg_offsets = np.asarray(seg_offsets, dtype=np.int64)
+        seg_offsets = device_frames(feats, seg_offsets, self.device)
         n_segs, total = len(seg_offsets) - 1, int(seg_offsets[-1])
         if self.n_models != 1 and self.n_models != n_segs:
             raise ValueError("posteriors are taken under one model for all segments, or under one model per segment "
@@ -274,7 +310,7 @@ class SharedModelSet:
         if precision not in ("tf32", "auto"):
             raise ValueError("the shared-variance kernel has one precision rung (11-bit operands, FP32-grade common part); expand() to a ModelSet for the "
                              "other precisions")
-        frame_offsets = np.asarray(frame_offsets, dtype=np.int64)
+        frame_offsets = device_frames(feats, frame_offsets, self.device)
         n_utts, total = len(frame_offsets) - 1, int(frame_offsets[-1])
         if feats.shape[1] != self.n_feat:
             raise ValueError(f"X has {feats.shape[1]} features, but the models expect {self.n_feat}")

@@ -78,6 +78,32 @@ def test_null_arguments_fail_without_touching_the_gpu(lib):
     assert lib.ssp_delta(None, 10, 13, 0, None, None) == -1
 
 
+@pytest.mark.parametrize("d", [13, 39, 40])
+def test_misaligned_workspace_fails_without_touching_the_gpu(lib, d):
+    """The statistics, posterior and shared-variance workspaces must be 16-byte aligned (the tensor-core kernels write
+    the frame images with 16-byte stores and stream them with cp.async.bulk).  A base 4, 8 or 12 bytes off is
+    SSP_EINVAL before any CUDA call; a 16-byte aligned one passes the check (no segments: nothing is launched).  The
+    pointers are made up: the calls return before anything dereferences them."""
+    from speech_signal_processing_b200 import _lib
+
+    dims = C.byref(_lib.GmmDims(1, 16, d))
+    p = 1 << 20                                   # stands in for every device buffer
+    for off, want in ((4, -1), (8, -1), (12, -1), (16, 0), (1024, 0)):
+        ws = p + off
+        assert lib.ssp_gmm_stats(p, p, 0, 0, p, dims, p, p, p, p, p, ws, 1 << 20, 0, None) == want, (d, off)
+        if want:
+            assert b"16-byte aligned" in lib.ssp_last_error()
+        assert lib.ssp_gmm_posteriors(p, p, 0, 0, p, dims, p, p, p, ws, 1 << 20, 0, None) == want, (d, off)
+        if want:
+            assert b"16-byte aligned" in lib.ssp_last_error()
+        if d <= 39:                               # the shared-variance kernel's widths
+            assert lib.ssp_gmm_score_shared(p, p, 0, 0, p, dims, p, p, ws, 1 << 20, None) == want, (d, off)
+            if want:
+                assert b"16-byte aligned" in lib.ssp_last_error()
+    # a NULL workspace stays legal where none is needed
+    assert lib.ssp_gmm_stats(p, p, 0, 0, p, dims, p, p, p, p, p, None, 0, 0, None) == 0
+
+
 def test_library_has_no_hidden_tuning_switches():
     """The kernels' tuning choices are constants in the sources.  The only environment variable the library reads is
     SSP_SV_GROUP_MB (the L2 group size of shared-variance scoring, which tests use to reach the multi-launch path), and no
