@@ -299,6 +299,48 @@ int ssp_gmm_posteriors(const float* feats, const int64_t* seg_offsets, int64_t n
 int64_t ssp_gmm_posteriors_workspace_bytes(const ssp_gmm_dims* dims, int64_t total_frames, int64_t n_segs);
 
 /*
+ * Top-C Gaussian selection (the first half of the fast scoring of Reynolds, Quatieri & Dunn 2000): for every frame the C
+ * components with the largest L_c(t) = log w_c + log N(x_t; c) under ONE model, in descending order, the lower index
+ * first on equal values.  D <= 39 (SSP_EUNSUP above), 1 <= C <= min(K, 64) (else SSP_EINVAL), dims->n_models == 1.
+ * FP32 grade: the logits are the 3 x BF16 tcgen05 products of ssp_gmm_posteriors.
+ * out_idx        device int32[total_frames * C]
+ * out_logit      device float[total_frames * C]: L_c(t) of the selected components
+ * workspace      device, ssp_gmm_top_components_workspace_bytes() bytes, 16-byte aligned (else SSP_EINVAL).  The layout of
+ *                the ssp_gmm_stats / ssp_gmm_posteriors workspace with a longer last section: the frame images sit at the
+ *                same place, so reuse_images works across the three calls on the same frames.
+ */
+int ssp_gmm_top_components(const float* feats, const int64_t* seg_offsets, int64_t n_segs, int64_t total_frames,
+                           const void* pack, const ssp_gmm_dims* dims, int32_t c, int32_t* out_idx, float* out_logit,
+                           void* workspace, int64_t workspace_bytes, int32_t reuse_images, void* stream);
+/* Scratch bytes ssp_gmm_top_components needs (0: unsupported dims or C). */
+int64_t ssp_gmm_top_components_workspace_bytes(const ssp_gmm_dims* dims, int64_t total_frames, int64_t n_segs, int32_t c);
+
+/*
+ * Top-C scoring of a model set that shares weights and variances (the second half of the fast scoring): with S_t the
+ * selection of ssp_gmm_top_components under the reference member r,
+ *   l_s(t) = log sum_{c in S_t} exp(L_s,c(t)),   L_s,c(t) = L_r,c(t) + a_s,c . x_t + b_s,c,
+ *   a_s,c = (mu_s,c - mu_r,c) / var_c,   b_s,c = -1/2 sum_d (mu_s,c - mu_r,c)(mu_s,c + mu_r,c) / var_c,
+ * scores[u, s] = mean of l_s(t) over the frames of utterance u (0 for an empty utterance).  With C = K this is the exact
+ * score.  The (a, b) table is the pack: FP32, component-major ([K][S][roundup(D + 1, 4)]); the weights cancel in L_s - L_r
+ * and are not part of it.  dims->n_models = S, weights / variances / means as in ssp_gmm_pack_shared, D <= 39.
+ * The frames are scored in chunks of ssp_gmm_topc_chunk_frames() frames: each chunk's (frame, slot) pairs are routed by
+ * component, the difference terms of a component for all models are FP32 FMAs, the log-sum-exp over the C slots is taken
+ * per (frame, model) in FP32 and the utterance sums are double.
+ * idx, logit     device int32 / float [total_frames * C] from ssp_gmm_top_components (entries outside [0, K) are skipped)
+ * out_scores     device double[n_utts * S]
+ * out_frame_lse  device float[S * total_frames] or NULL: l_s(t)
+ * workspace      device, ssp_gmm_score_topc_workspace_bytes() bytes, 16-byte aligned (else SSP_EINVAL)
+ */
+int64_t ssp_gmm_topc_pack_bytes(const ssp_gmm_dims* dims);
+int ssp_gmm_pack_topc(const double* variances, const double* means, const ssp_gmm_dims* dims, int32_t ref_model,
+                      void* out_pack, void* stream);
+int64_t ssp_gmm_topc_chunk_frames(void);
+int64_t ssp_gmm_score_topc_workspace_bytes(const ssp_gmm_dims* dims, int32_t c, int64_t total_frames);
+int ssp_gmm_score_topc(const float* feats, const int64_t* frame_offsets, int64_t n_utts, int64_t total_frames,
+                       const int32_t* idx, const float* logit, int32_t c, const void* pack, const ssp_gmm_dims* dims,
+                       double* out_scores, float* out_frame_lse, void* workspace, int64_t workspace_bytes, void* stream);
+
+/*
  * M-step on device (sklearn _gaussian_mixture.py:312-313,250-252,898): from (all-reduced)
  * statistics to weights/means/variances, double precision, for n_models models at once (arrays [n_models][K](xD)).
  * nk = N + 10*eps_of(stat_dtype); mu = F/nk; var = S/nk - mu^2 + reg_covar; w = nk/sum(nk).

@@ -216,3 +216,84 @@ extern "C" int ssp_gmm_posteriors(const float* feats, const int64_t* seg_offsets
   return ssp::launch_posteriors_simt(feats, seg_offsets, n_segs, total_frames, pack, L, out_resp, out_label, out_frame_lse,
                                      workspace, st);
 }
+
+extern "C" int64_t ssp_gmm_top_components_workspace_bytes(const ssp_gmm_dims* dims, int64_t total_frames, int64_t n_segs,
+                                                          int32_t c) {
+  ssp::PackLayout L;
+  if (!ssp::make_layout(dims, &L) || L.n_models != 1 || total_frames < 0 || n_segs < 0 || c < 1 || c > ssp::kTopcMaxC)
+    return 0;
+  return ssp::topc_tc_workspace_bytes(L, total_frames, n_segs, c);
+}
+
+extern "C" int ssp_gmm_top_components(const float* feats, const int64_t* seg_offsets, int64_t n_segs, int64_t total_frames,
+                                      const void* pack, const ssp_gmm_dims* dims, int32_t c, int32_t* out_idx, float* out_logit,
+                                      void* workspace, int64_t workspace_bytes, int32_t reuse_images, void* stream) {
+  ssp::PackLayout L;
+  SSP_REQUIRE(ssp::make_layout(dims, &L), "ssp_gmm_top_components: unsupported dims");
+  SSP_REQUIRE(dims->n_models == 1, "ssp_gmm_top_components: %d models (selection runs under one model)", dims->n_models);
+  if (!ssp::stats_tc_supported(L)) {
+    ssp::set_error("ssp_gmm_top_components: D = %d (the selection kernels take D <= %d)", L.D, ssp::kTopcMaxFeat);
+    return SSP_EUNSUP;
+  }
+  SSP_REQUIRE(c >= 1 && c <= L.K && c <= ssp::kTopcMaxC, "ssp_gmm_top_components: C = %d outside [1, min(K = %d, %d)]", c, L.K,
+              ssp::kTopcMaxC);
+  SSP_REQUIRE(seg_offsets && pack && out_idx && out_logit && (feats || total_frames == 0), "ssp_gmm_top_components: null pointer");
+  SSP_REQUIRE(((uintptr_t)workspace & (kWorkspaceAlign - 1)) == 0, "ssp_gmm_top_components: workspace must be %d-byte aligned",
+              (int)kWorkspaceAlign);
+  SSP_REQUIRE(n_segs >= 0 && total_frames >= 0, "ssp_gmm_top_components: negative size");
+  if (n_segs == 0 || total_frames == 0) return SSP_OK;
+  const int64_t need = ssp::topc_tc_workspace_bytes(L, total_frames, n_segs, c);
+  SSP_REQUIRE(workspace && workspace_bytes >= need,
+              "ssp_gmm_top_components: workspace of %lld bytes, need %lld (ssp_gmm_top_components_workspace_bytes)",
+              (long long)(workspace ? workspace_bytes : 0), (long long)need);
+  return ssp::launch_topc_tc(feats, seg_offsets, n_segs, total_frames, pack, L, c, out_idx, out_logit, workspace,
+                             reuse_images != 0, (cudaStream_t)stream);
+}
+
+static bool topc_dims_ok(const ssp_gmm_dims* dims) {
+  return dims && dims->n_models >= 1 && dims->n_comp >= 1 && dims->n_feat >= 1 && dims->n_feat <= ssp::kTopcMaxFeat;
+}
+
+extern "C" int64_t ssp_gmm_topc_pack_bytes(const ssp_gmm_dims* dims) {
+  return topc_dims_ok(dims) ? ssp::topc_pack_bytes(dims->n_models, dims->n_comp, dims->n_feat) : 0;
+}
+
+extern "C" int ssp_gmm_pack_topc(const double* variances, const double* means, const ssp_gmm_dims* dims, int32_t ref_model,
+                                 void* out_pack, void* stream) {
+  SSP_REQUIRE(topc_dims_ok(dims), "ssp_gmm_pack_topc: unsupported dims (need 1 <= D <= %d)", ssp::kTopcMaxFeat);
+  SSP_REQUIRE(variances && means && out_pack, "ssp_gmm_pack_topc: null pointer");
+  SSP_REQUIRE(((uintptr_t)out_pack & 15) == 0, "ssp_gmm_pack_topc: out_pack must be 16-byte aligned");
+  SSP_REQUIRE(ref_model >= 0 && ref_model < dims->n_models, "ssp_gmm_pack_topc: ref_model %d outside [0, %d)", ref_model,
+              dims->n_models);
+  return ssp::launch_pack_topc(variances, means, dims->n_models, dims->n_comp, dims->n_feat, ref_model, out_pack,
+                               (cudaStream_t)stream);
+}
+
+extern "C" int64_t ssp_gmm_topc_chunk_frames(void) { return ssp::kTopcChunkFrames; }
+
+extern "C" int64_t ssp_gmm_score_topc_workspace_bytes(const ssp_gmm_dims* dims, int32_t c, int64_t total_frames) {
+  if (!topc_dims_ok(dims) || c < 1 || c > dims->n_comp || c > ssp::kTopcMaxC || total_frames < 0) return 0;
+  return ssp::score_topc_workspace_bytes(dims->n_models, dims->n_comp, c, total_frames);
+}
+
+extern "C" int ssp_gmm_score_topc(const float* feats, const int64_t* frame_offsets, int64_t n_utts, int64_t total_frames,
+                                  const int32_t* idx, const float* logit, int32_t c, const void* pack, const ssp_gmm_dims* dims,
+                                  double* out_scores, float* out_frame_lse, void* workspace, int64_t workspace_bytes,
+                                  void* stream) {
+  SSP_REQUIRE(topc_dims_ok(dims), "ssp_gmm_score_topc: unsupported dims (need 1 <= D <= %d)", ssp::kTopcMaxFeat);
+  SSP_REQUIRE(c >= 1 && c <= dims->n_comp && c <= ssp::kTopcMaxC, "ssp_gmm_score_topc: C = %d outside [1, min(K = %d, %d)]", c,
+              dims->n_comp, ssp::kTopcMaxC);
+  SSP_REQUIRE(frame_offsets && pack && out_scores && ((feats && idx && logit) || total_frames == 0),
+              "ssp_gmm_score_topc: null pointer");
+  SSP_REQUIRE(((uintptr_t)pack & 15) == 0, "ssp_gmm_score_topc: pack must be 16-byte aligned");
+  SSP_REQUIRE(((uintptr_t)workspace & (kWorkspaceAlign - 1)) == 0, "ssp_gmm_score_topc: workspace must be %d-byte aligned",
+              (int)kWorkspaceAlign);
+  SSP_REQUIRE(n_utts >= 0 && total_frames >= 0, "ssp_gmm_score_topc: negative size");
+  const int64_t need = ssp::score_topc_workspace_bytes(dims->n_models, dims->n_comp, c, total_frames);
+  SSP_REQUIRE(need == 0 || (workspace && workspace_bytes >= need),
+              "ssp_gmm_score_topc: workspace of %lld bytes, need %lld (ssp_gmm_score_topc_workspace_bytes)",
+              (long long)(workspace ? workspace_bytes : 0), (long long)need);
+  if (n_utts == 0) return SSP_OK;
+  return ssp::launch_score_topc(feats, frame_offsets, n_utts, total_frames, idx, logit, c, pack, dims->n_models, dims->n_comp,
+                                dims->n_feat, out_scores, out_frame_lse, workspace, (cudaStream_t)stream);
+}

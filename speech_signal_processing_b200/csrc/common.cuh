@@ -220,6 +220,23 @@ int64_t stats_tc_workspace_bytes(const PackLayout& L, int64_t total_frames, int6
 int launch_posteriors_tc(const float* feats, const int64_t* seg_offsets, int64_t n_segs, int64_t total_frames, const void* pack,
                          const PackLayout& L, float* out_resp, int64_t* out_label, float* out_frame_lse, void* workspace,
                          bool reuse_images, cudaStream_t st);
+// top-C selection (gmm_em_tc.cu) and top-C scoring of shared-variance model sets (gmm_topc.cu)
+constexpr int kTopcMaxC = 64;
+constexpr int kTopcMaxFeat = 39;
+// frames per chunk of the top-C scoring: the chunk buffer holds kTopcChunkFrames * C * n_models FP32 values (82 MB at
+// C = 5 and 1001 models, L2-sized) and each component receives about kTopcChunkFrames * C / K routed pairs per chunk
+constexpr int64_t kTopcChunkFrames = 4096;
+inline int topc_row_floats(int D) { return (D + 1 + 3) / 4 * 4; }  // [a (D), b, 0..] per (component, model)
+int64_t topc_tc_workspace_bytes(const PackLayout& L, int64_t total_frames, int64_t n_segs, int c);
+int launch_topc_tc(const float* feats, const int64_t* seg_offsets, int64_t n_segs, int64_t total_frames, const void* pack,
+                   const PackLayout& L, int c, int32_t* out_idx, float* out_logit, void* workspace, bool reuse_images,
+                   cudaStream_t st);
+int64_t topc_pack_bytes(int S, int K, int D);
+int launch_pack_topc(const double* var, const double* mu, int S, int K, int D, int ref, void* pack, cudaStream_t st);
+int64_t score_topc_workspace_bytes(int S, int K, int C, int64_t T);
+int launch_score_topc(const float* feats, const int64_t* offsets, int64_t n_utts, int64_t T, const int32_t* idx,
+                      const float* logit, int C, const void* pack, int S, int K, int D, double* scores, float* frame_lse,
+                      void* workspace, cudaStream_t st);
 // workspace of the CUDA-core posterior path: per-segment sums of the scoring kernel, then the per-frame lse
 inline int64_t posteriors_simt_lse_offset(int64_t n_segs) { return (8 * n_segs + 255) / 256 * 256; }
 inline int64_t posteriors_simt_workspace_bytes(int64_t total_frames, int64_t n_segs) {

@@ -103,6 +103,9 @@ struct Args {
   float* out_resp;           // [total_frames][K] (posterior pass)
   int64_t* out_label;        // [total_frames]    (posterior pass)
   int resp_vec;              // out_resp rows are 16-byte aligned (K % 4 == 0 and an aligned base): float4 stores
+  int topc;                  // C of the selection pass: partial holds [2 n_tiles][C][P] (logit, component) lists
+  int32_t* out_idx;          // [total_frames][C] (selection pass)
+  float* out_logit;          // [total_frames][C] (selection pass)
 };
 
 // ------------------------------------------------------------------------------------------------ PTX helpers
@@ -295,7 +298,10 @@ __global__ void __launch_bounds__(256) em_prep_kernel(const Args a) {
 //   kEpiResp   (gmm_em_post_kernel)  gamma = 2^(L - lse2) -> out_resp[frame][comp], live frames and components only
 //   kEpiLabel  (gmm_em_post_kernel)  (max logit, lowest component reaching it) of each half tile -> partial, in the
 //                                    slots of the LSE partials (em_label_merge_kernel reduces them)
-constexpr int kEpiLse = 0, kEpiResp = 1, kEpiLabel = 2;
+//   kEpiTopC   (gmm_em_post_kernel)  the C largest (logit, component) of each half tile in descending order, the lower
+//                                    component first on equal logits -> C partial slots per half tile
+//                                    (em_topc_merge_kernel reduces them)
+constexpr int kEpiLse = 0, kEpiResp = 1, kEpiLabel = 2, kEpiTopC = 4;
 
 template <int kEpi>
 __device__ __forceinline__ void logit_pass(const Args& a) {
@@ -452,6 +458,28 @@ __device__ __forceinline__ void logit_pass(const Args& a) {
           }
           dst[i * IMG] = make_float2(bm, __int_as_float(comp0 + bi));
         }
+        if constexpr (kEpi == kEpiTopC) {
+          // C rounds of a selection: round j takes the best column strictly after the pick of round j - 1 in the order
+          // (logit descending, column ascending); once the live columns are used up, the rounds write (-3e38, column 64),
+          // which the merge never prefers to a real component (C <= K)
+          const int n_live = a.K - comp0;
+          float2* out = a.partial + (size_t)(2 * (tile0 + t) + half) * a.topc * a.P + i * IMG + row;
+          float pv = 3.0e38f;
+          int pi = -1;
+#pragma unroll 1
+          for (int j = 0; j < a.topc; ++j) {
+            float bm = -3.0e38f;
+            int bi = 64;
+#pragma unroll
+            for (int e = 0; e < 64; ++e) {
+              const float v = __uint_as_float(e < 32 ? ra[e] : rb[e - 32]);
+              if (e < n_live && (v < pv || (v == pv && e > pi)) && v > bm) { bm = v; bi = e; }
+            }
+            out[(size_t)j * a.P] = make_float2(bm, __int_as_float(comp0 + bi));
+            pv = bm;
+            pi = bi;
+          }
+        }
         if constexpr (kResp) {
           if (live) {
             float* out = a.out_resp + frame * a.K + comp0;
@@ -505,6 +533,69 @@ __global__ void __launch_bounds__(256) em_label_merge_kernel(const Args a) {
       if (q.x > bm) { bm = q.x; bi = q.y; }
     }
     a.out_label[__ldg(a.blk_t0 + b) + r] = __float_as_int(bi);
+  }
+}
+
+// top-C partials -> out_idx / out_logit: thread == padded frame.  The running list (C entries, sorted) lives in shared
+// memory, two buffers per thread that alternate as the merge target; the half-tile lists come in ascending component
+// order, so a list whose first entry does not beat the running list's last contributes nothing and is skipped.
+// Order: logit descending, the lower component first on equal logits.
+__device__ __forceinline__ bool topc_before(float2 x, float2 y) {
+  return x.x > y.x || (x.x == y.x && __float_as_int(x.y) < __float_as_int(y.y));
+}
+constexpr int kTopcMergeThreads = 128;
+__global__ void __launch_bounds__(kTopcMergeThreads) em_topc_merge_kernel(const Args a) {
+  extern __shared__ float2 lists[];  // [2][C][kTopcMergeThreads]
+  const int C = a.topc, tid = threadIdx.x;
+  const int64_t n_rows = ((a.blk_start[a.n_segs] + 1) & ~(int64_t)1) * BLK;
+  const int n_part = 2 * a.n_tiles;
+  const size_t lstride = (size_t)C * a.P;  // between the lists of two half tiles
+  for (int64_t p = (int64_t)blockIdx.x * kTopcMergeThreads + tid; p < n_rows; p += (int64_t)gridDim.x * kTopcMergeThreads) {
+    const int64_t b = p >> 6;
+    const int r = (int)(p & 63);
+    if (r >= __ldg(a.blk_nt + b)) continue;
+    float2* cur = lists + tid;
+    float2* nxt = lists + (size_t)C * kTopcMergeThreads + tid;
+    for (int j = 0; j < C; ++j) cur[j * kTopcMergeThreads] = __ldg(a.partial + (size_t)j * a.P + p);
+    for (int y = 1; y < n_part; ++y) {
+      const float2* src = a.partial + (size_t)y * lstride + p;
+      float2 hb = __ldg(src);
+      if (!topc_before(hb, cur[(C - 1) * kTopcMergeThreads])) continue;
+      int ia = 0, ib = 0;
+      for (int j = 0; j < C; ++j) {
+        const float2 ha = cur[ia * kTopcMergeThreads];
+        if (topc_before(hb, ha)) {
+          nxt[j * kTopcMergeThreads] = hb;
+          ++ib;
+          hb = ib < C ? __ldg(src + (size_t)ib * a.P) : make_float2(-3.4e38f, __int_as_float(0x7fffffff));
+        } else {
+          nxt[j * kTopcMergeThreads] = ha;
+          ++ia;
+        }
+      }
+      float2* tmp = cur;
+      cur = nxt;
+      nxt = tmp;
+    }
+    // log2 domain of the tiles -> natural log; two logits an ulp apart in log2 may round to one value, and the lower
+    // component then goes first (an insertion pass over the nearly sorted list)
+    for (int j = 0; j < C; ++j) {
+      float2 q = cur[j * kTopcMergeThreads];
+      q.x *= 0.69314718055994530942f;
+      int k = j;
+      for (; k > 0; --k) {
+        const float2 p = cur[(k - 1) * kTopcMergeThreads];
+        if (!topc_before(q, p)) break;
+        cur[k * kTopcMergeThreads] = p;
+      }
+      cur[k * kTopcMergeThreads] = q;
+    }
+    const int64_t frame = __ldg(a.blk_t0 + b) + r;
+    for (int j = 0; j < C; ++j) {
+      const float2 q = cur[j * kTopcMergeThreads];
+      a.out_idx[frame * C + j] = __float_as_int(q.y);
+      a.out_logit[frame * C + j] = q.x;
+    }
   }
 }
 
@@ -816,6 +907,14 @@ int64_t stats_tc_workspace_bytes(const PackLayout& L, int64_t total_frames, int6
   return stats_tc_supported(L) ? (int64_t)em::ws_layout(L, total_frames, n_segs).bytes : 0;
 }
 
+// the statistics / posterior workspace with its last section, the partials, C times as long
+int64_t topc_tc_workspace_bytes(const PackLayout& L, int64_t total_frames, int64_t n_segs, int c) {
+  if (!stats_tc_supported(L)) return 0;
+  const em::Ws w = em::ws_layout(L, total_frames, n_segs);
+  const size_t part = sizeof(float2) * 2 * (L.Kp / em::BN) * (size_t)w.P * (size_t)c;
+  return (int64_t)(w.o_partial + (part + 1023) / 1024 * 1024);
+}
+
 static int g_num_sms = 0;
 static int query_sms() {
   if (g_num_sms == 0) {
@@ -971,6 +1070,32 @@ int launch_posteriors_tc(const float* feats, const int64_t* seg_offsets, int64_t
     em_label_merge_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, st>>>(a);
     SSP_LAUNCH_CHECK("em_label_merge_kernel");
   }
+  return SSP_OK;
+}
+
+int launch_topc_tc(const float* feats, const int64_t* seg_offsets, int64_t n_segs, int64_t total_frames, const void* pack,
+                   const PackLayout& L, int c, int32_t* out_idx, float* out_logit, void* workspace, bool reuse_images,
+                   cudaStream_t st) {
+  using namespace em;
+  if (total_frames == 0) return SSP_OK;
+  const Ws w = ws_layout(L, total_frames, n_segs);
+  Args a = em_args(feats, seg_offsets, n_segs, total_frames, pack, L, w, workspace);
+  a.topc = c;
+  a.out_idx = out_idx;
+  a.out_logit = out_logit;
+  EmGrid g;
+  int rc = em_grid(a, w, n_segs, total_frames, "ssp_gmm_top_components", &g);
+  if (rc != SSP_OK) return rc;
+  rc = em_prepare_and_lse(a, w, g, reuse_images, false, st);
+  if (rc != SSP_OK) return rc;
+  SSP_CUDA_OK(cudaFuncSetAttribute(gmm_em_post_kernel<kEpiTopC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem_lse));
+  gmm_em_post_kernel<kEpiTopC><<<dim3((unsigned)g.gx_l, (unsigned)g.n_pairs, g.gz), THREADS, g.smem_lse, st>>>(a);
+  SSP_LAUNCH_CHECK("gmm_em_post_kernel<topc>");
+  const size_t smem = sizeof(float2) * 2 * (size_t)c * kTopcMergeThreads;
+  SSP_CUDA_OK(cudaFuncSetAttribute(em_topc_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const int64_t blocks = (w.P + kTopcMergeThreads - 1) / kTopcMergeThreads, cap = 8 * (int64_t)g_num_sms;
+  em_topc_merge_kernel<<<(unsigned)(blocks < cap ? blocks : cap), kTopcMergeThreads, smem, st>>>(a);
+  SSP_LAUNCH_CHECK("em_topc_merge_kernel");
   return SSP_OK;
 }
 

@@ -236,6 +236,52 @@ class ModelSet:
         self._keep = d_off
         return g, lab, lse
 
+    @_lib.on_device
+    def top_components(self, feats, seg_offsets, c, workspace=None, reuse_images=False):
+        """(idx (T, C) int32 cuda, logit (T, C) float32 cuda): the C components with the largest weighted
+        log-probability ``log w_c + log N(x_t; c)`` for every frame, in descending order and the lower index first on
+        equal values -- the Gaussian selection of top-C fast scoring (:meth:`SharedModelSet.score_top_c`).  One-model
+        sets, D <= 39, 1 <= c <= min(K, 64).  FP32 grade: the tensor-core logits of :meth:`posteriors`, whose workspace
+        (and frame images) this call shares; ``workspace`` / ``reuse_images`` as in :meth:`stats`."""
+        torch = _lib.require_cuda()
+        seg_offsets = device_frames(feats, seg_offsets, self.device)
+        n_segs, total = len(seg_offsets) - 1, int(seg_offsets[-1])
+        if self.n_models != 1:
+            raise ValueError(f"top_components selects under one model (got a set of {self.n_models})")
+        if feats.shape[1] != self.n_feat:
+            raise ValueError(f"X has {feats.shape[1]} features, but the models expect {self.n_feat}")
+        c = check_top_c(c, self.n_comp)
+        idx = torch.empty((total, c), dtype=torch.int32, device=self.device)
+        logit = torch.empty((total, c), dtype=torch.float32, device=self.device)
+        d_off = torch.as_tensor(seg_offsets, device=self.device)
+        ws_bytes = int(self.lib.ssp_gmm_top_components_workspace_bytes(C.byref(self.dims), total, n_segs, c))
+        if workspace is None:
+            workspace = getattr(self, "_ws", None)
+            if workspace is None:
+                workspace = self._ws = StatsWorkspace(self.device)
+            reuse_images = False
+        buf = workspace.reserve(ws_bytes)
+        rc = self.lib.ssp_gmm_top_components(_lib.ptr(feats), _lib.ptr(d_off), n_segs, total, _lib.ptr(self.pack),
+                                             C.byref(self.dims), c, _lib.ptr(idx), _lib.ptr(logit),
+                                             _lib.ptr(buf) if ws_bytes else None, ws_bytes,
+                                             int(bool(reuse_images) and workspace.valid), _lib.stream_ptr())
+        _lib.check(rc, "ssp_gmm_top_components")
+        if total:
+            workspace.valid = True
+        self._keep = d_off
+        return idx, logit
+
+
+# widest selection the top-C kernels keep per frame
+MAX_TOP_C = 64
+
+
+def check_top_c(c, n_comp):
+    """``c`` as an int in [1, min(n_comp, MAX_TOP_C)], else ``ValueError``."""
+    if isinstance(c, bool) or not isinstance(c, (int, np.integer)) or not 1 <= int(c) <= min(n_comp, MAX_TOP_C):
+        raise ValueError(f"top-C needs an integer C in [1, min(K = {n_comp}, {MAX_TOP_C})] (got {c!r})")
+    return int(c)
+
 
 class StatsWorkspace:
     """Scratch of ``ssp_gmm_stats`` and ``ssp_gmm_posteriors`` (operand images of the frames + log-sum-exp partials; the
@@ -325,6 +371,42 @@ class SharedModelSet:
                                            _lib.ptr(self._ws) if ws_bytes else None, ws_bytes, _lib.stream_ptr())
         _lib.check(rc, "ssp_gmm_score_shared")
         self._keep = d_off
+        return scores, lse
+
+    @_lib.on_device
+    def score_top_c(self, feats, frame_offsets, c=5, want_frame_lse=False):
+        """Top-C fast scoring (Reynolds, Quatieri & Dunn 2000): (scores (n_utts, n_models) cuda float64, frame_lse
+        (n_models, total) cuda float32 | None).  For every frame the C components the reference member ``ref_model`` (the
+        UBM) ranks highest are selected (:meth:`ModelSet.top_components`), and every model is scored over those C
+        components only: ``log sum_{c in S_t} w_c N(x_t; mu_s,c, var_c)``, averaged over the frames of each utterance (0 for
+        an empty one).  An approximation with its own definition: with ``c = n_comp`` it is the exact score.  Always FP32
+        grade (FP32-grade selection logits, FP32 difference terms, double utterance sums)."""
+        torch = _lib.require_cuda()
+        frame_offsets = device_frames(feats, frame_offsets, self.device)
+        n_utts, total = len(frame_offsets) - 1, int(frame_offsets[-1])
+        if feats.shape[1] != self.n_feat:
+            raise ValueError(f"X has {feats.shape[1]} features, but the models expect {self.n_feat}")
+        c = check_top_c(c, self.n_comp)
+        w, var, mu = self._params
+        if getattr(self, "_topc", None) is None:
+            # the reference member as a one-model set (selection) and the component-major (a, b) table (scoring)
+            ref = ModelSet(w[None], mu[self.ref_model][None], var[None], device=self.device)
+            pack = torch.empty(int(self.lib.ssp_gmm_topc_pack_bytes(C.byref(self.dims))), dtype=torch.uint8, device=self.device)
+            _lib.check(self.lib.ssp_gmm_pack_topc(_lib.ptr(var), _lib.ptr(mu), C.byref(self.dims), self.ref_model,
+                                                  _lib.ptr(pack), _lib.stream_ptr()), "ssp_gmm_pack_topc")
+            self._topc = (ref, pack)
+        ref, pack = self._topc
+        idx, logit = ref.top_components(feats, np.array([0, total], dtype=np.int64), c)
+        d_off = torch.as_tensor(frame_offsets, device=self.device)
+        scores = torch.empty((n_utts, self.n_models), dtype=torch.float64, device=self.device)
+        lse = torch.empty((self.n_models, total), dtype=torch.float32, device=self.device) if want_frame_lse else None
+        ws_bytes = int(self.lib.ssp_gmm_score_topc_workspace_bytes(C.byref(self.dims), c, total))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=self.device) if ws_bytes else None
+        rc = self.lib.ssp_gmm_score_topc(_lib.ptr(feats), _lib.ptr(d_off), n_utts, total, _lib.ptr(idx), _lib.ptr(logit), c,
+                                         _lib.ptr(pack), C.byref(self.dims), _lib.ptr(scores), _lib.ptr(lse), _lib.ptr(ws),
+                                         ws_bytes, _lib.stream_ptr())
+        _lib.check(rc, "ssp_gmm_score_topc")
+        self._keep = (d_off, idx, logit, ws)
         return scores, lse
 
     def expand(self) -> "ModelSet":

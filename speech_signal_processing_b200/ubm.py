@@ -22,8 +22,8 @@ import numpy as np
 from . import _lib
 from . import frontend as fe
 from .wavio import read_wav_batch
-from .mixture import (SINGLE_PASS_MIN_COMPONENTS, GaussianMixture, ModelSet, SharedModelSet, concat_utterances, fit_batch,
-                      resolve_precision)
+from .mixture import (SINGLE_PASS_MIN_COMPONENTS, GaussianMixture, ModelSet, SharedModelSet, check_top_c, concat_utterances,
+                      fit_batch, resolve_precision)
 
 
 def map_adapt(ubm: GaussianMixture, speaker_frames, relevance: float = 16.0, adapt=("means",), device=None):
@@ -77,7 +77,40 @@ def _base_params(model):
     return np.asarray(model.weights_), np.asarray(model.covariances_)
 
 
-def identify(utts, speakers, ubm=None, precision="auto", device=None):
+def _top_c_set(speakers, ubm, dev):
+    """(SharedModelSet whose reference member is the UBM, column of the UBM) for top-C scoring, or the refusal: no UBM is a
+    ``ValueError``, speakers that do not share the UBM's weights and variances a ``NotImplementedError``."""
+    if isinstance(speakers, SharedModelSet) and ubm is None:
+        k = getattr(speakers, "ubm_index", None)
+        if k is None:
+            raise ValueError("top_c scores against a UBM: pass ubm=, or a SharedModelSet from map_enrol")
+        if k != speakers.ref_model:
+            raise NotImplementedError("top_c selects by the reference member of the set, which must be its UBM "
+                                      f"(ref_model {speakers.ref_model}, ubm_index {k})")
+        return speakers, k
+    if ubm is None:
+        raise ValueError("top_c scores against a UBM: pass ubm=, or a SharedModelSet from map_enrol")
+    base = _base_params(ubm)
+    if base is None:
+        raise ValueError("ubm must be ONE model")
+    if isinstance(speakers, SharedModelSet):
+        w, var, mu = (t.cpu().numpy() for t in speakers._params)
+        sw, svar, smu = w[None], var[None], mu
+    elif isinstance(speakers, ModelSet):
+        sw, smu, svar = (t.cpu().numpy() for t in speakers._params)
+    else:
+        sw = np.stack([np.asarray(m.weights_) for m in speakers])
+        smu = np.stack([np.asarray(m.means_) for m in speakers])
+        svar = np.stack([np.asarray(m.covariances_) for m in speakers])
+    if not (SharedModelSet.shares_base(sw, svar) and np.array_equal(base[0], sw[0]) and np.array_equal(base[1], svar[0])):
+        raise NotImplementedError("top_c needs speaker models that share the UBM's weights and variances (mean-only MAP "
+                                  "enrolment): there is no component correspondence otherwise")
+    umu = ubm._params[1][0].cpu().numpy() if isinstance(ubm, ModelSet) else np.asarray(ubm.means_)
+    sms = SharedModelSet(base[0], base[1], np.concatenate([smu, umu[None]]), ref_model=-1, device=dev)
+    return sms, sms.n_models - 1
+
+
+def identify(utts, speakers, ubm=None, precision="auto", device=None, top_c=None):
     """LLR matrix and decisions for all (utterance, speaker) pairs (GMM_UBM.py:191-197).
 
     ``speakers``: :class:`ModelSet` / :class:`SharedModelSet`, or list of fitted GaussianMixture-likes.  ``ubm``: fitted
@@ -89,10 +122,24 @@ def identify(utts, speakers, ubm=None, precision="auto", device=None):
     ``precision``: "auto" (default) keeps every LLR within 1e-3 absolute of float64: one TF32 pass for models of
     >= 512 components (mean-only MAP sets then go through the shared-variance kernel), three passes (FP32-grade) for
     smaller ones, FP32 CUDA cores for D > 39.  "tf32" forces the single pass, "tf32x2" / "tf32x3" / "fp32" the others.
+
+    ``top_c``: None (default) scores exactly as above.  An integer C scores by top-C fast scoring
+    (:meth:`SharedModelSet.score_top_c`, Reynolds et al. 2000): every frame under every speaker over the C components the
+    UBM ranks highest for it, always at FP32 grade (``precision`` is ignored).  The speakers must share the UBM's weights
+    and variances: a :func:`map_enrol` set, or mean-only MAP models with a ``ubm`` of the same weights and variances
+    (``NotImplementedError`` otherwise); without a UBM it is a ``ValueError``.
     """
     torch = _lib.require_cuda()
     dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
     with torch.cuda.device(dev):
+        if top_c is not None:
+            sms, k = _top_c_set(speakers, ubm, dev)
+            check_top_c(top_c, sms.n_comp)
+            feats, offs = concat_utterances(utts, dev)
+            scores, _ = sms.score_top_c(feats, offs, c=top_c)
+            keep = [i for i in range(sms.n_models) if i != k]
+            pred = (scores[:, keep] - scores[:, k : k + 1]).cpu().numpy()
+            return pred, pred.argmax(axis=1)
         feats, offs = concat_utterances(utts, dev)
         if isinstance(speakers, SharedModelSet) and getattr(speakers, "ubm_index", None) is not None and ubm is None:
             # the UBM rides along as one of the mean sets (map_enrol): one launch scores everything
@@ -165,7 +212,7 @@ def split_for_overlap(frame_counts, head_fraction: float = 0.1, min_frames: int 
 
 
 def identify_pcm(host_pcm, sample_offsets, front_end, speakers, ubm_index=None, precision="auto", out=None,
-                 head_fraction: float = 0.1, min_split_frames: int = 4 * _WAVE_FRAMES):
+                 head_fraction: float = 0.1, min_split_frames: int = 4 * _WAVE_FRAMES, top_c=None):
     """Raw PCM on the host -> speaker decisions on the host, for one batch of utterances: the front-end of
     GMM_UBM.py:129 and the scoring / argmax of :191-197 as one call.
 
@@ -175,9 +222,18 @@ def identify_pcm(host_pcm, sample_offsets, front_end, speakers, ubm_index=None, 
     the argmax), or None.  The host-to-device copy is cut in two at an utterance boundary: the head (about a tenth of
     the frames, whole scoring waves) is copied on the current stream and goes straight into the front-end and scoring
     kernels while a side stream copies the rest, so all but the head's transfer is hidden behind compute.
+    ``top_c``: None scores exactly; an integer C scores by top-C fast scoring (:meth:`SharedModelSet.score_top_c`,
+    ``precision`` ignored), which needs a :class:`SharedModelSet` whose reference member is the UBM and ``ubm_index``
+    naming it (a :func:`map_enrol` set and its ``ubm_index``).
     Returns ``(decisions (N,) int64 host tensor, total_frames)``; the call returns after the decisions have landed."""
     torch = _lib.require_cuda()
     dev = front_end.device
+    if top_c is not None:
+        if ubm_index is None:
+            raise ValueError("top_c scores against a UBM: pass ubm_index")
+        if not isinstance(speakers, SharedModelSet) or int(ubm_index) % speakers.n_models != speakers.ref_model:
+            raise NotImplementedError("top_c needs a SharedModelSet whose reference member is the UBM (ubm_index)")
+        check_top_c(top_c, speakers.n_comp)
     if isinstance(host_pcm, np.ndarray):
         host_pcm = torch.from_numpy(np.ascontiguousarray(host_pcm))
     sample_offsets = np.asarray(sample_offsets, dtype=np.int64)
@@ -215,7 +271,10 @@ def identify_pcm(host_pcm, sample_offsets, front_end, speakers, ubm_index=None, 
         offs = sample_offsets[lo : hi + 1] - base
         feats, foffs, _ = front_end.extract_device(pcm, offs)
         total += int(foffs[-1])
-        scores, _ = speakers.score(feats, foffs, precision=precision)
+        if top_c is None:
+            scores, _ = speakers.score(feats, foffs, precision=precision)
+        else:
+            scores, _ = speakers.score_top_c(feats, foffs, c=top_c)
         if ubm_index is not None:
             k = int(ubm_index) % scores.shape[1]
             llr = scores - scores[:, k : k + 1]
