@@ -57,6 +57,16 @@ extern "C" const char* ssp_launch_log(void) {
 // aligned.  Every section inside a workspace starts at a multiple of 256 bytes from its base, so the base is what counts.
 static constexpr uintptr_t kWorkspaceAlign = 16;
 
+// The workspace argument of `fn`: 16-byte aligned (NULL passes), and at least `need` bytes where the call needs one (no
+// silent slower path: a short workspace is the caller's error).  `query` names the entry point that gives `need`.
+static int check_workspace(const char* fn, const void* workspace, int64_t workspace_bytes, int64_t need, const char* query) {
+  SSP_REQUIRE(((uintptr_t)workspace & (kWorkspaceAlign - 1)) == 0, "%s: workspace must be %d-byte aligned", fn,
+              (int)kWorkspaceAlign);
+  SSP_REQUIRE(need == 0 || (workspace && workspace_bytes >= need), "%s: workspace of %lld bytes, need %lld (%s)", fn,
+              (long long)(workspace ? workspace_bytes : 0), (long long)need, query);
+  return SSP_OK;
+}
+
 extern "C" int64_t ssp_gmm_pack_bytes(const ssp_gmm_dims* dims) {
   ssp::PackLayout L;
   if (!ssp::make_layout(dims, &L)) return 0;
@@ -119,13 +129,10 @@ extern "C" int ssp_gmm_score_shared(const float* feats, const int64_t* frame_off
   ssp::SvLayout L;
   SSP_REQUIRE(ssp::make_sv_layout(dims, &L), "ssp_gmm_score_shared: unsupported dims");
   SSP_REQUIRE(frame_offsets && pack && out_scores && (feats || total_frames == 0), "ssp_gmm_score_shared: null pointer");
-  SSP_REQUIRE(workspace || ssp::score_sv_workspace_bytes(L, total_frames) == 0, "ssp_gmm_score_shared: null workspace");
-  SSP_REQUIRE(((uintptr_t)workspace & (kWorkspaceAlign - 1)) == 0, "ssp_gmm_score_shared: workspace must be %d-byte aligned",
-              (int)kWorkspaceAlign);
   SSP_REQUIRE(n_utts >= 0 && total_frames >= 0, "ssp_gmm_score_shared: negative size");
-  SSP_REQUIRE(workspace_bytes >= ssp::score_sv_workspace_bytes(L, total_frames), "ssp_gmm_score_shared: workspace of %lld bytes, need %lld",
-              (long long)workspace_bytes, (long long)ssp::score_sv_workspace_bytes(L, total_frames));
-  if (n_utts == 0) return SSP_OK;
+  int rc = check_workspace("ssp_gmm_score_shared", workspace, workspace_bytes, ssp::score_sv_workspace_bytes(L, total_frames),
+                           "ssp_gmm_score_shared_workspace_bytes");
+  if (rc != SSP_OK || n_utts == 0) return rc;
   return ssp::launch_score_sv(feats, frame_offsets, n_utts, total_frames, pack, L, true, out_scores, out_frame_lse, workspace,
                               (cudaStream_t)stream);
 }
@@ -146,19 +153,15 @@ extern "C" int ssp_gmm_stats(const float* feats, const int64_t* seg_offsets, int
               "ssp_gmm_stats: %d models for %lld segments (one model for all segments, or one per segment)", dims->n_models,
               (long long)n_segs);
   SSP_REQUIRE(seg_offsets && pack && frame_lse && out_n && out_f && out_s && out_loglik, "ssp_gmm_stats: null pointer");
-  SSP_REQUIRE(((uintptr_t)workspace & (kWorkspaceAlign - 1)) == 0, "ssp_gmm_stats: workspace must be %d-byte aligned",
-              (int)kWorkspaceAlign);
   SSP_REQUIRE(n_segs >= 0 && total_frames >= 0, "ssp_gmm_stats: negative size");
-  if (n_segs == 0) return SSP_OK;
+  // only the tensor-core path takes a workspace (0 bytes otherwise)
+  int rc = check_workspace("ssp_gmm_stats", workspace, workspace_bytes,
+                           n_segs ? ssp::stats_tc_workspace_bytes(L, total_frames, n_segs) : 0, "ssp_gmm_stats_workspace_bytes");
+  if (rc != SSP_OK || n_segs == 0) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   // The tensor-core kernels serve every feature width they support (D <= 39); the FP32 CUDA-core kernels serve wider
   // features only.
   if (ssp::stats_tc_supported(L)) {
-    // no silent 10x slower path: a short workspace is the caller's error
-    const int64_t need = ssp::stats_tc_workspace_bytes(L, total_frames, n_segs);
-    SSP_REQUIRE(need == 0 || (workspace && workspace_bytes >= need),
-                "ssp_gmm_stats: workspace of %lld bytes, the tensor-core path needs %lld (ssp_gmm_stats_workspace_bytes)",
-                (long long)(workspace ? workspace_bytes : 0), (long long)need);
     return ssp::launch_stats_tc(feats, seg_offsets, n_segs, total_frames, pack, L, frame_lse, out_n, out_f, out_s, out_loglik,
                                 workspace, reuse_images != 0, st);
   }
@@ -168,7 +171,7 @@ extern "C" int ssp_gmm_stats(const float* feats, const int64_t* seg_offsets, int
   }
   // FP32 CUDA-core path (D > 39).  pass 1: per-frame log-likelihood and the per-segment sum of frame log-likelihoods (the EM
   // lower bound numerator, sklearn _base.py:558); pass 2: posteriors and N/F/S
-  int rc = ssp::launch_score_simt(feats, seg_offsets, n_segs, total_frames, pack, L, false, out_loglik, frame_lse, st);
+  rc = ssp::launch_score_simt(feats, seg_offsets, n_segs, total_frames, pack, L, false, out_loglik, frame_lse, st);
   if (rc != SSP_OK) return rc;
   return ssp::launch_stats_simt(feats, seg_offsets, n_segs, total_frames, pack, L, frame_lse, out_n, out_f, out_s, st);
 }
@@ -191,16 +194,14 @@ extern "C" int ssp_gmm_posteriors(const float* feats, const int64_t* seg_offsets
               dims->n_models, (long long)n_segs);
   SSP_REQUIRE(out_resp || out_label, "ssp_gmm_posteriors: out_resp and out_label are both NULL (nothing to compute)");
   SSP_REQUIRE(seg_offsets && pack && (feats || total_frames == 0), "ssp_gmm_posteriors: null pointer");
-  SSP_REQUIRE(((uintptr_t)workspace & (kWorkspaceAlign - 1)) == 0, "ssp_gmm_posteriors: workspace must be %d-byte aligned",
-              (int)kWorkspaceAlign);
   SSP_REQUIRE(n_segs >= 0 && total_frames >= 0, "ssp_gmm_posteriors: negative size");
-  if (n_segs == 0 || total_frames == 0) return SSP_OK;
+  const bool empty = n_segs == 0 || total_frames == 0;
+  int rc = check_workspace("ssp_gmm_posteriors", workspace, workspace_bytes,
+                           empty ? 0 : ssp_gmm_posteriors_workspace_bytes(dims, total_frames, n_segs),
+                           "ssp_gmm_posteriors_workspace_bytes");
+  if (rc != SSP_OK || empty) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   if (ssp::stats_tc_supported(L)) {
-    const int64_t need = ssp::stats_tc_workspace_bytes(L, total_frames, n_segs);
-    SSP_REQUIRE(workspace && workspace_bytes >= need,
-                "ssp_gmm_posteriors: workspace of %lld bytes, need %lld (ssp_gmm_posteriors_workspace_bytes)",
-                (long long)(workspace ? workspace_bytes : 0), (long long)need);
     return ssp::launch_posteriors_tc(feats, seg_offsets, n_segs, total_frames, pack, L, out_resp, out_label, out_frame_lse,
                                      workspace, reuse_images != 0, st);
   }
@@ -209,10 +210,6 @@ extern "C" int ssp_gmm_posteriors(const float* feats, const int64_t* seg_offsets
                    ssp::kMaxTrainModels);
     return SSP_EUNSUP;
   }
-  const int64_t need = ssp::posteriors_simt_workspace_bytes(total_frames, n_segs);
-  SSP_REQUIRE(workspace && workspace_bytes >= need,
-              "ssp_gmm_posteriors: workspace of %lld bytes, need %lld (ssp_gmm_posteriors_workspace_bytes)",
-              (long long)(workspace ? workspace_bytes : 0), (long long)need);
   return ssp::launch_posteriors_simt(feats, seg_offsets, n_segs, total_frames, pack, L, out_resp, out_label, out_frame_lse,
                                      workspace, st);
 }
@@ -238,14 +235,12 @@ extern "C" int ssp_gmm_top_components(const float* feats, const int64_t* seg_off
   SSP_REQUIRE(c >= 1 && c <= L.K && c <= ssp::kTopcMaxC, "ssp_gmm_top_components: C = %d outside [1, min(K = %d, %d)]", c, L.K,
               ssp::kTopcMaxC);
   SSP_REQUIRE(seg_offsets && pack && out_idx && out_logit && (feats || total_frames == 0), "ssp_gmm_top_components: null pointer");
-  SSP_REQUIRE(((uintptr_t)workspace & (kWorkspaceAlign - 1)) == 0, "ssp_gmm_top_components: workspace must be %d-byte aligned",
-              (int)kWorkspaceAlign);
   SSP_REQUIRE(n_segs >= 0 && total_frames >= 0, "ssp_gmm_top_components: negative size");
-  if (n_segs == 0 || total_frames == 0) return SSP_OK;
-  const int64_t need = ssp::topc_tc_workspace_bytes(L, total_frames, n_segs, c);
-  SSP_REQUIRE(workspace && workspace_bytes >= need,
-              "ssp_gmm_top_components: workspace of %lld bytes, need %lld (ssp_gmm_top_components_workspace_bytes)",
-              (long long)(workspace ? workspace_bytes : 0), (long long)need);
+  const bool empty = n_segs == 0 || total_frames == 0;
+  int rc = check_workspace("ssp_gmm_top_components", workspace, workspace_bytes,
+                           empty ? 0 : ssp::topc_tc_workspace_bytes(L, total_frames, n_segs, c),
+                           "ssp_gmm_top_components_workspace_bytes");
+  if (rc != SSP_OK || empty) return rc;
   return ssp::launch_topc_tc(feats, seg_offsets, n_segs, total_frames, pack, L, c, out_idx, out_logit, workspace,
                              reuse_images != 0, (cudaStream_t)stream);
 }
@@ -286,14 +281,11 @@ extern "C" int ssp_gmm_score_topc(const float* feats, const int64_t* frame_offse
   SSP_REQUIRE(frame_offsets && pack && out_scores && ((feats && idx && logit) || total_frames == 0),
               "ssp_gmm_score_topc: null pointer");
   SSP_REQUIRE(((uintptr_t)pack & 15) == 0, "ssp_gmm_score_topc: pack must be 16-byte aligned");
-  SSP_REQUIRE(((uintptr_t)workspace & (kWorkspaceAlign - 1)) == 0, "ssp_gmm_score_topc: workspace must be %d-byte aligned",
-              (int)kWorkspaceAlign);
   SSP_REQUIRE(n_utts >= 0 && total_frames >= 0, "ssp_gmm_score_topc: negative size");
-  const int64_t need = ssp::score_topc_workspace_bytes(dims->n_models, dims->n_comp, c, total_frames);
-  SSP_REQUIRE(need == 0 || (workspace && workspace_bytes >= need),
-              "ssp_gmm_score_topc: workspace of %lld bytes, need %lld (ssp_gmm_score_topc_workspace_bytes)",
-              (long long)(workspace ? workspace_bytes : 0), (long long)need);
-  if (n_utts == 0) return SSP_OK;
+  int rc = check_workspace("ssp_gmm_score_topc", workspace, workspace_bytes,
+                           ssp::score_topc_workspace_bytes(dims->n_models, dims->n_comp, c, total_frames),
+                           "ssp_gmm_score_topc_workspace_bytes");
+  if (rc != SSP_OK || n_utts == 0) return rc;
   return ssp::launch_score_topc(feats, frame_offsets, n_utts, total_frames, idx, logit, c, pack, dims->n_models, dims->n_comp,
                                 dims->n_feat, out_scores, out_frame_lse, workspace, (cudaStream_t)stream);
 }

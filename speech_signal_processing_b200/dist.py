@@ -112,9 +112,7 @@ def map_enrol_sharded(comm: Comm, ubm, speaker_frames, relevance: float = 16.0):
         mu = torch.empty((0, k, d), dtype=torch.float64, device=umu.device)
     counts = [shard_range(n_spk, r, comm.world_size) for r in range(comm.world_size)]
     means = comm.gather_rows(mu, [b - a for a, b in counts])
-    sms = SharedModelSet(uw[0], uvar[0], torch.cat([means, umu]), ref_model=-1, device=umu.device)
-    sms.ubm_index = n_spk
-    return sms
+    return SharedModelSet.with_ubm(uw[0], uvar[0], means, umu, device=umu.device)
 
 
 def identify_sharded(comm: Comm, utts, speakers, ubm=None, precision="auto"):

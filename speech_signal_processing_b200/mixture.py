@@ -100,6 +100,32 @@ def concat_utterances(utts, device):
     return host.to(device, non_blocking=True), offs
 
 
+def _as_params(a, device):
+    """A model parameter (numpy or torch) as a contiguous float64 tensor on ``device``."""
+    torch = _lib.require_cuda()
+    if isinstance(a, torch.Tensor):
+        return a.to(device=device, dtype=torch.float64).contiguous()
+    return torch.as_tensor(np.ascontiguousarray(a, dtype=np.float64), device=device)
+
+
+def stacked_params(models):
+    """(weights (S,K), means (S,K,D), covariances (S,K,D)) numpy of a list of fitted GaussianMixture-likes."""
+    return (np.stack([np.asarray(m.weights_) for m in models]), np.stack([np.asarray(m.means_) for m in models]),
+            np.stack([np.asarray(m.covariances_) for m in models]))
+
+
+def _upload_frames(ms, feats, offsets):
+    """What every call of a model set ``ms`` starts with: :func:`device_frames`, the feature-width check and the upload of
+    the offsets, which ``ms`` keeps alive until its next call so that the stream has consumed them before they are
+    freed.  Returns (offsets on the device, number of segments, total frames)."""
+    torch = _lib.require_cuda()
+    offsets = device_frames(feats, offsets, ms.device)
+    if feats.shape[1] != ms.n_feat:
+        raise ValueError(f"X has {feats.shape[1]} features, but the models expect {ms.n_feat}")
+    ms._keep = torch.as_tensor(offsets, device=ms.device)
+    return ms._keep, len(offsets) - 1, int(offsets[-1])
+
+
 class ModelSet:
     """``n_models`` diagonal GMMs with the same (K, D), packed once in HBM for the scoring kernels."""
 
@@ -107,13 +133,7 @@ class ModelSet:
         torch = _lib.require_cuda()
         self.lib = _lib.load()
         self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
-
-        def dev(a):
-            if isinstance(a, torch.Tensor):
-                return a.to(device=self.device, dtype=torch.float64).contiguous()
-            return torch.as_tensor(np.ascontiguousarray(a, dtype=np.float64), device=self.device)
-
-        w, mu, var = dev(weights), dev(means), dev(variances)
+        w, mu, var = (_as_params(a, self.device) for a in (weights, means, variances))
         if mu.dim() == 2:
             w, mu, var = w[None], mu[None], var[None]
         if mu.dim() != 3 or var.shape != mu.shape or w.shape != mu.shape[:2]:
@@ -124,6 +144,7 @@ class ModelSet:
         if nbytes <= 0:
             raise ValueError(f"unsupported GMM dims K={self.n_comp} D={self.n_feat} (need 1 <= D <= 80)")
         self.pack = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+        self._ws = StatsWorkspace(self.device)  # the calls given no workspace of their own
         self.repack(w, mu, var)
 
     @_lib.on_device
@@ -133,6 +154,18 @@ class ModelSet:
         _lib.check(self.lib.ssp_gmm_pack_models(_lib.ptr(w), _lib.ptr(mu), _lib.ptr(var), C.byref(self.dims),
                                                 _lib.ptr(self.pack), _lib.stream_ptr()), "ssp_gmm_pack_models")
 
+    def _image_frames(self, fn, name, total, ws_bytes, workspace, reuse_images, *args):
+        """``fn(*args, workspace, ws_bytes, reuse_images, stream)``: one of the calls that turn the frames into operand
+        images in a :class:`StatsWorkspace`.  Without a ``workspace`` the set's own serves and its images are rebuilt (its
+        frames may be another call's).  The workspace holds valid images only after a call that imaged frames."""
+        if workspace is None:
+            workspace, reuse_images = self._ws, False
+        buf = workspace.reserve(ws_bytes)
+        _lib.check(fn(*args, _lib.ptr(buf) if ws_bytes else None, ws_bytes, int(bool(reuse_images) and workspace.valid),
+                      _lib.stream_ptr()), name)
+        if total:
+            workspace.valid = True
+
     # ---------------------------------------------------------------------------------------
     @_lib.on_device
     def score(self, feats, frame_offsets, precision="auto", want_frame_lse=False):
@@ -141,19 +174,14 @@ class ModelSet:
         single pass streams FP16 images of the models) or "auto"
         (:func:`resolve_precision`)."""
         torch = _lib.require_cuda()
-        frame_offsets = device_frames(feats, frame_offsets, self.device)
-        n_utts, total = len(frame_offsets) - 1, int(frame_offsets[-1])
         precision = resolve_precision(precision, self.n_comp, self.n_feat)
-        if feats.shape[1] != self.n_feat:
-            raise ValueError(f"X has {feats.shape[1]} features, but the models expect {self.n_feat}")
-        d_off = torch.as_tensor(frame_offsets, device=self.device)
+        d_off, n_utts, total = _upload_frames(self, feats, frame_offsets)
         scores = torch.empty((n_utts, self.n_models), dtype=torch.float64, device=self.device)
         lse = torch.empty((self.n_models, total), dtype=torch.float32, device=self.device) if want_frame_lse else None
         rc = self.lib.ssp_gmm_score(_lib.ptr(feats), _lib.ptr(d_off), n_utts, total, _lib.ptr(self.pack),
                                     C.byref(self.dims), PRECISIONS[precision], _lib.ptr(scores), _lib.ptr(lse),
                                     _lib.stream_ptr())
         _lib.check(rc, "ssp_gmm_score")
-        self._keep = d_off
         return scores, lse
 
     @_lib.on_device
@@ -165,10 +193,7 @@ class ModelSet:
         ``seg_offsets``; ``reuse_images=True`` then skips the preparation pass that turns the frames into tensor-core
         operand images (EM iterations: the frames never change).  Default: a workspace owned by this model set."""
         torch = _lib.require_cuda()
-        seg_offsets = device_frames(feats, seg_offsets, self.device)
-        n_segs, total = len(seg_offsets) - 1, int(seg_offsets[-1])
-        if feats.shape[1] != self.n_feat:
-            raise ValueError(f"X has {feats.shape[1]} features, but the models expect {self.n_feat}")
+        d_off, n_segs, total = _upload_frames(self, feats, seg_offsets)
         if self.n_models != 1 and self.n_models != n_segs:
             raise ValueError("statistics are taken under one model for all segments (the UBM), or under one model per "
                              f"segment (got {self.n_models} models for {n_segs} segments)")
@@ -178,20 +203,10 @@ class ModelSet:
         s = torch.zeros((n_segs, k, d), dtype=torch.float64, device=self.device)
         ll = torch.zeros(n_segs, dtype=torch.float64, device=self.device)
         lse = torch.empty(max(total, 1), dtype=torch.float32, device=self.device)
-        d_off = torch.as_tensor(seg_offsets, device=self.device)
-        ws_bytes = int(self.lib.ssp_gmm_stats_workspace_bytes(C.byref(self.dims), total, n_segs))
-        if workspace is None:
-            workspace = getattr(self, "_ws", None)
-            if workspace is None:
-                workspace = self._ws = StatsWorkspace(self.device)
-            reuse_images = False
-        buf = workspace.reserve(ws_bytes)
-        rc = self.lib.ssp_gmm_stats(_lib.ptr(feats), _lib.ptr(d_off), n_segs, total, _lib.ptr(self.pack),
-                                    C.byref(self.dims), _lib.ptr(lse), _lib.ptr(n), _lib.ptr(f), _lib.ptr(s), _lib.ptr(ll),
-                                    _lib.ptr(buf) if ws_bytes else None, ws_bytes, int(bool(reuse_images) and workspace.valid),
-                                    _lib.stream_ptr())
-        _lib.check(rc, "ssp_gmm_stats")
-        workspace.valid = True
+        self._image_frames(self.lib.ssp_gmm_stats, "ssp_gmm_stats", total,
+                           int(self.lib.ssp_gmm_stats_workspace_bytes(C.byref(self.dims), total, n_segs)), workspace,
+                           reuse_images, _lib.ptr(feats), _lib.ptr(d_off), n_segs, total, _lib.ptr(self.pack),
+                           C.byref(self.dims), _lib.ptr(lse), _lib.ptr(n), _lib.ptr(f), _lib.ptr(s), _lib.ptr(ll))
         self._keep = (d_off, lse)
         return n, f, s, ll
 
@@ -207,33 +222,19 @@ class ModelSet:
         FP32 CUDA-core kernels above.  ``workspace`` / ``reuse_images`` as in :meth:`stats`, whose workspace (and frame
         images) this call shares."""
         torch = _lib.require_cuda()
-        seg_offsets = device_frames(feats, seg_offsets, self.device)
-        n_segs, total = len(seg_offsets) - 1, int(seg_offsets[-1])
+        d_off, n_segs, total = _upload_frames(self, feats, seg_offsets)
         if self.n_models != 1 and self.n_models != n_segs:
             raise ValueError("posteriors are taken under one model for all segments, or under one model per segment "
                              f"(got {self.n_models} models for {n_segs} segments)")
-        if feats.shape[1] != self.n_feat:
-            raise ValueError(f"X has {feats.shape[1]} features, but the models expect {self.n_feat}")
         if not (resp or labels):
             raise ValueError("posteriors: ask for resp, labels or both")
         g = torch.empty((total, self.n_comp), dtype=torch.float32, device=self.device) if resp else None
         lab = torch.empty(total, dtype=torch.int64, device=self.device) if labels else None
         lse = torch.empty(total, dtype=torch.float32, device=self.device) if resp else None
-        d_off = torch.as_tensor(seg_offsets, device=self.device)
-        ws_bytes = int(self.lib.ssp_gmm_posteriors_workspace_bytes(C.byref(self.dims), total, n_segs))
-        if workspace is None:
-            workspace = getattr(self, "_ws", None)
-            if workspace is None:
-                workspace = self._ws = StatsWorkspace(self.device)
-            reuse_images = False
-        buf = workspace.reserve(ws_bytes)
-        rc = self.lib.ssp_gmm_posteriors(_lib.ptr(feats), _lib.ptr(d_off), n_segs, total, _lib.ptr(self.pack),
-                                         C.byref(self.dims), _lib.ptr(g), _lib.ptr(lab), _lib.ptr(lse),
-                                         _lib.ptr(buf) if ws_bytes else None, ws_bytes,
-                                         int(bool(reuse_images) and workspace.valid), _lib.stream_ptr())
-        _lib.check(rc, "ssp_gmm_posteriors")
-        workspace.valid = True
-        self._keep = d_off
+        self._image_frames(self.lib.ssp_gmm_posteriors, "ssp_gmm_posteriors", total,
+                           int(self.lib.ssp_gmm_posteriors_workspace_bytes(C.byref(self.dims), total, n_segs)), workspace,
+                           reuse_images, _lib.ptr(feats), _lib.ptr(d_off), n_segs, total, _lib.ptr(self.pack),
+                           C.byref(self.dims), _lib.ptr(g), _lib.ptr(lab), _lib.ptr(lse))
         return g, lab, lse
 
     @_lib.on_device
@@ -244,31 +245,16 @@ class ModelSet:
         sets, D <= 39, 1 <= c <= min(K, 64).  FP32 grade: the tensor-core logits of :meth:`posteriors`, whose workspace
         (and frame images) this call shares; ``workspace`` / ``reuse_images`` as in :meth:`stats`."""
         torch = _lib.require_cuda()
-        seg_offsets = device_frames(feats, seg_offsets, self.device)
-        n_segs, total = len(seg_offsets) - 1, int(seg_offsets[-1])
+        d_off, n_segs, total = _upload_frames(self, feats, seg_offsets)
         if self.n_models != 1:
             raise ValueError(f"top_components selects under one model (got a set of {self.n_models})")
-        if feats.shape[1] != self.n_feat:
-            raise ValueError(f"X has {feats.shape[1]} features, but the models expect {self.n_feat}")
         c = check_top_c(c, self.n_comp)
         idx = torch.empty((total, c), dtype=torch.int32, device=self.device)
         logit = torch.empty((total, c), dtype=torch.float32, device=self.device)
-        d_off = torch.as_tensor(seg_offsets, device=self.device)
-        ws_bytes = int(self.lib.ssp_gmm_top_components_workspace_bytes(C.byref(self.dims), total, n_segs, c))
-        if workspace is None:
-            workspace = getattr(self, "_ws", None)
-            if workspace is None:
-                workspace = self._ws = StatsWorkspace(self.device)
-            reuse_images = False
-        buf = workspace.reserve(ws_bytes)
-        rc = self.lib.ssp_gmm_top_components(_lib.ptr(feats), _lib.ptr(d_off), n_segs, total, _lib.ptr(self.pack),
-                                             C.byref(self.dims), c, _lib.ptr(idx), _lib.ptr(logit),
-                                             _lib.ptr(buf) if ws_bytes else None, ws_bytes,
-                                             int(bool(reuse_images) and workspace.valid), _lib.stream_ptr())
-        _lib.check(rc, "ssp_gmm_top_components")
-        if total:
-            workspace.valid = True
-        self._keep = d_off
+        self._image_frames(self.lib.ssp_gmm_top_components, "ssp_gmm_top_components", total,
+                           int(self.lib.ssp_gmm_top_components_workspace_bytes(C.byref(self.dims), total, n_segs, c)),
+                           workspace, reuse_images, _lib.ptr(feats), _lib.ptr(d_off), n_segs, total, _lib.ptr(self.pack),
+                           C.byref(self.dims), c, _lib.ptr(idx), _lib.ptr(logit))
         return idx, logit
 
 
@@ -284,9 +270,9 @@ def check_top_c(c, n_comp):
 
 
 class StatsWorkspace:
-    """Scratch of ``ssp_gmm_stats`` and ``ssp_gmm_posteriors`` (operand images of the frames + log-sum-exp partials; the
-    two calls lay it out alike).  ``valid`` says that it holds the images of the frames it was last used with; growing it
-    invalidates them."""
+    """Grow-only device scratch of the GMM calls that take a workspace.  ``ssp_gmm_stats``, ``ssp_gmm_posteriors`` and
+    ``ssp_gmm_top_components`` lay it out alike (operand images of the frames + log-sum-exp partials): ``valid`` says that
+    it holds the images of the frames it was last used with; growing it invalidates them."""
 
     def __init__(self, device):
         self.device, self.buf, self.valid = device, None, False
@@ -315,13 +301,7 @@ class SharedModelSet:
         torch = _lib.require_cuda()
         self.lib = _lib.load()
         self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
-
-        def dev(a):
-            if isinstance(a, torch.Tensor):
-                return a.to(device=self.device, dtype=torch.float64).contiguous()
-            return torch.as_tensor(np.ascontiguousarray(a, dtype=np.float64), device=self.device)
-
-        w, var, mu = dev(weights), dev(variances), dev(means)
+        w, var, mu = (_as_params(a, self.device) for a in (weights, variances, means))
         if mu.dim() == 2:
             mu = mu[None]
         if w.dim() != 1 or var.dim() != 2 or mu.dim() != 3 or mu.shape[1:] != var.shape or w.shape[0] != var.shape[0]:
@@ -338,7 +318,20 @@ class SharedModelSet:
                                                     self.ref_model, _lib.ptr(self.pack), _lib.stream_ptr()),
                        "ssp_gmm_pack_shared")
         self._params = (w, var, mu)
-        self._ws = None
+        self._ws = None    # score's scratch, made when the scoring first needs one (more than one L2 group of models)
+        self._topc = None
+
+    @classmethod
+    def with_ubm(cls, weights, variances, speaker_means, ubm_means, device=None):
+        """Speakers (S,K,D means) and their UBM (K,D means) with the same weights and variances as one set: the UBM is
+        model S, the reference member, and ``ubm_index`` names it."""
+        torch = _lib.require_cuda()
+        dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
+        speaker_means, ubm_means = _as_params(speaker_means, dev), _as_params(ubm_means, dev)
+        sms = cls(weights, variances, torch.cat([speaker_means, ubm_means.reshape(1, *speaker_means.shape[1:])]),
+                  ref_model=-1, device=dev)
+        sms.ubm_index = sms.n_models - 1
+        return sms
 
     @staticmethod
     def shares_base(weights, variances) -> bool:
@@ -356,21 +349,17 @@ class SharedModelSet:
         if precision not in ("tf32", "auto"):
             raise ValueError("the shared-variance kernel has one precision rung (11-bit operands, FP32-grade common part); expand() to a ModelSet for the "
                              "other precisions")
-        frame_offsets = device_frames(feats, frame_offsets, self.device)
-        n_utts, total = len(frame_offsets) - 1, int(frame_offsets[-1])
-        if feats.shape[1] != self.n_feat:
-            raise ValueError(f"X has {feats.shape[1]} features, but the models expect {self.n_feat}")
-        d_off = torch.as_tensor(frame_offsets, device=self.device)
+        d_off, n_utts, total = _upload_frames(self, feats, frame_offsets)
         scores = torch.empty((n_utts, self.n_models), dtype=torch.float64, device=self.device)
         lse = torch.empty((self.n_models, total), dtype=torch.float32, device=self.device) if want_frame_lse else None
         ws_bytes = int(self.lib.ssp_gmm_score_shared_workspace_bytes(C.byref(self.dims), total))
-        if ws_bytes and (self._ws is None or self._ws.numel() < ws_bytes):
-            self._ws = torch.empty(ws_bytes, dtype=torch.uint8, device=self.device)
+        if ws_bytes and self._ws is None:
+            self._ws = StatsWorkspace(self.device)
+        ws = self._ws.reserve(ws_bytes) if ws_bytes else None
         rc = self.lib.ssp_gmm_score_shared(_lib.ptr(feats), _lib.ptr(d_off), n_utts, total, _lib.ptr(self.pack),
                                            C.byref(self.dims), _lib.ptr(scores), _lib.ptr(lse),
-                                           _lib.ptr(self._ws) if ws_bytes else None, ws_bytes, _lib.stream_ptr())
+                                           _lib.ptr(ws) if ws_bytes else None, ws_bytes, _lib.stream_ptr())
         _lib.check(rc, "ssp_gmm_score_shared")
-        self._keep = d_off
         return scores, lse
 
     @_lib.on_device
@@ -382,31 +371,28 @@ class SharedModelSet:
         an empty one).  An approximation with its own definition: with ``c = n_comp`` it is the exact score.  Always FP32
         grade (FP32-grade selection logits, FP32 difference terms, double utterance sums)."""
         torch = _lib.require_cuda()
-        frame_offsets = device_frames(feats, frame_offsets, self.device)
-        n_utts, total = len(frame_offsets) - 1, int(frame_offsets[-1])
-        if feats.shape[1] != self.n_feat:
-            raise ValueError(f"X has {feats.shape[1]} features, but the models expect {self.n_feat}")
+        d_off, n_utts, total = _upload_frames(self, feats, frame_offsets)
         c = check_top_c(c, self.n_comp)
         w, var, mu = self._params
-        if getattr(self, "_topc", None) is None:
-            # the reference member as a one-model set (selection) and the component-major (a, b) table (scoring)
+        if self._topc is None:
+            # the reference member as a one-model set (selection), the component-major (a, b) table (scoring) and the
+            # scoring's scratch
             ref = ModelSet(w[None], mu[self.ref_model][None], var[None], device=self.device)
             pack = torch.empty(int(self.lib.ssp_gmm_topc_pack_bytes(C.byref(self.dims))), dtype=torch.uint8, device=self.device)
             _lib.check(self.lib.ssp_gmm_pack_topc(_lib.ptr(var), _lib.ptr(mu), C.byref(self.dims), self.ref_model,
                                                   _lib.ptr(pack), _lib.stream_ptr()), "ssp_gmm_pack_topc")
-            self._topc = (ref, pack)
-        ref, pack = self._topc
+            self._topc = (ref, pack, StatsWorkspace(self.device))
+        ref, pack, scratch = self._topc
         idx, logit = ref.top_components(feats, np.array([0, total], dtype=np.int64), c)
-        d_off = torch.as_tensor(frame_offsets, device=self.device)
         scores = torch.empty((n_utts, self.n_models), dtype=torch.float64, device=self.device)
         lse = torch.empty((self.n_models, total), dtype=torch.float32, device=self.device) if want_frame_lse else None
         ws_bytes = int(self.lib.ssp_gmm_score_topc_workspace_bytes(C.byref(self.dims), c, total))
-        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=self.device) if ws_bytes else None
+        ws = scratch.reserve(ws_bytes)
         rc = self.lib.ssp_gmm_score_topc(_lib.ptr(feats), _lib.ptr(d_off), n_utts, total, _lib.ptr(idx), _lib.ptr(logit), c,
-                                         _lib.ptr(pack), C.byref(self.dims), _lib.ptr(scores), _lib.ptr(lse), _lib.ptr(ws),
-                                         ws_bytes, _lib.stream_ptr())
+                                         _lib.ptr(pack), C.byref(self.dims), _lib.ptr(scores), _lib.ptr(lse),
+                                         _lib.ptr(ws) if ws_bytes else None, ws_bytes, _lib.stream_ptr())
         _lib.check(rc, "ssp_gmm_score_topc")
-        self._keep = (d_off, idx, logit, ws)
+        self._keep = (d_off, idx, logit)
         return scores, lse
 
     def expand(self) -> "ModelSet":
@@ -421,12 +407,27 @@ def score_matrix(utts, models, precision="auto", device=None):
     (or anything with ``weights_/means_/covariances_``) or a :class:`ModelSet`.  Returns float64 numpy."""
     torch = _lib.require_cuda()
     dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
-    ms = models if isinstance(models, ModelSet) else ModelSet(
-        np.stack([np.asarray(m.weights_) for m in models]), np.stack([np.asarray(m.means_) for m in models]),
-        np.stack([np.asarray(m.covariances_) for m in models]), device=dev)
+    ms = models if isinstance(models, ModelSet) else ModelSet(*stacked_params(models), device=dev)
     feats, offs = concat_utterances(utts, dev)
     scores, _ = ms.score(feats, offs, precision=precision)
     return scores.cpu().numpy()
+
+
+def _nk_eps(X):
+    """sklearn's floor on the component counts of the M-step: 10 eps of the input's dtype (float32 input keeps
+    float32, anything else is taken as float64)."""
+    torch = _lib.require_cuda()
+    f32 = (isinstance(X, torch.Tensor) and X.dtype == torch.float32) or (isinstance(X, np.ndarray) and X.dtype == np.float32)
+    return 10.0 * float(np.finfo(np.float32 if f32 else np.float64).eps)
+
+
+def _check_sample_counts(counts, k):
+    """sklearn's refusal of a model fitted to fewer than 2 or fewer than ``k`` frames."""
+    for cnt in counts:
+        if cnt < 2:
+            raise ValueError(f"Found array with {cnt} sample(s) while a minimum of 2 is required.")
+        if cnt < k:
+            raise ValueError(f"Expected n_samples >= n_components but got n_components = {k}, n_samples = {cnt}")
 
 
 class GaussianMixture:
@@ -496,36 +497,89 @@ class GaussianMixture:
             self._ms = ModelSet(self.weights_, self.means_, self.covariances_)
         return self._ms
 
-    def _set_params_from_device(self, w, mu, var):
-        self.weights_ = w.cpu().numpy()
-        self.means_ = mu.cpu().numpy()
-        self.covariances_ = var.cpu().numpy()
+    def _rng(self):
+        return self.random_state if isinstance(self.random_state, np.random.RandomState) else np.random.RandomState(self.random_state)
+
+    def _set_fitted(self, weights, means, covariances, converged, n_iter, lower_bound):
+        self.weights_, self.means_, self.covariances_ = (np.asarray(a, dtype=np.float64) for a in (weights, means, covariances))
         self.precisions_cholesky_ = 1.0 / np.sqrt(self.covariances_)
         self.precisions_ = self.precisions_cholesky_ ** 2
+        self.converged_, self.n_iter_, self.lower_bound_ = bool(converged), int(n_iter), float(lower_bound)
+        self._ms = None
+
+    def _finish_em(self, weights, means, covariances, converged, n_iter, lower_bound, bounds):
+        """sklearn's end of ``fit``: the non-convergence warning, the refusal of ill-defined covariances, the fitted
+        attributes."""
+        if not converged and self.max_iter > 0:
+            warnings.warn("Best performing initialization did not converge. Try different init parameters, or "
+                          "increase max_iter, tol, or check for degenerate data.", UserWarning)
+        if not np.all(np.isfinite(covariances)) or np.any(covariances <= 0):
+            raise ValueError("Fitting the mixture model failed because some components have ill-defined empirical "
+                             "covariance (for instance caused by singleton or collapsed samples). Try to decrease the "
+                             "number of components, increase reg_covar, or scale the input data.")
+        self._set_fitted(weights, means, covariances, converged, n_iter, lower_bound)
+        self.lower_bounds_ = bounds
 
     # ------------------------------------------------------------------ EM
-    def _em_iteration(self, ms, feats, seg, n_total, nk_eps, w, mu, var, workspace=None):
-        """One E+M step on device.  Returns the lower bound (mean frame log-likelihood under the
-        parameters the E-step used)."""
+    def _em_step(self, ms, feats, seg, workspace, nk_eps, w, mu, var, timed=False):
+        """One E+M step on device: the statistics of segment s under model s (``ssp_gmm_stats``), summed over the ranks of
+        ``comm`` in ONE all-reduce of ``[N, F, S, loglik, frames]``, then the M-step of every model into (w, mu, var).
+        Returns (N, loglik) on the device and the frames of every segment on the host, all summed over the ranks."""
         torch = _lib.require_cuda()
+        counts = np.diff(seg).astype(np.float64)
         n, f, s, ll = ms.stats(feats, seg, workspace=workspace, reuse_images=True)
-        if self.comm is not None and self.comm.world_size > 1:
-            k, d = ms.n_comp, ms.n_feat
-            cnt = torch.tensor([float(feats.shape[0])], dtype=torch.float64, device=feats.device)
-            flat = torch.cat([n.reshape(-1), f.reshape(-1), s.reshape(-1), ll.reshape(-1), cnt])
-            timing = getattr(self, "allreduce_events", None)  # bench.py: a list to append (start, end) CUDA events to
+        reduce = self.comm is not None and self.comm.world_size > 1
+        if reduce:
+            parts = (n, f, s, ll, torch.as_tensor(counts, device=feats.device))
+            flat = torch.cat([t.reshape(-1) for t in parts])
+            # bench.py: a list to append (start, end) CUDA events of the EM loop's all-reduce to
+            timing = getattr(self, "allreduce_events", None) if timed else None
             if timing is not None:
                 timing.append((torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)))
                 timing[-1][0].record()
             flat = self.comm.allreduce_sum(flat)
             if timing is not None:
                 timing[-1][1].record()
-            n, f, s = flat[:k].reshape(1, k), flat[k : k + k * d].reshape(1, k, d), flat[k + k * d : k + 2 * k * d].reshape(1, k, d)
-            ll, n_total = flat[k + 2 * k * d : k + 2 * k * d + 1], float(flat[-1].item())
-        rc = ms.lib.ssp_gmm_mstep(_lib.ptr(n), _lib.ptr(f), _lib.ptr(s), 1, ms.n_comp, ms.n_feat, float(self.reg_covar),
-                                  float(nk_eps), _lib.ptr(w), _lib.ptr(mu), _lib.ptr(var), _lib.stream_ptr())
+            n, f, s, ll, counts = (v.view(t.shape) for v, t in zip(flat.split([t.numel() for t in parts]), parts))
+        rc = ms.lib.ssp_gmm_mstep(_lib.ptr(n), _lib.ptr(f), _lib.ptr(s), ms.n_models, ms.n_comp, ms.n_feat,
+                                  float(self.reg_covar), float(nk_eps), _lib.ptr(w), _lib.ptr(mu), _lib.ptr(var),
+                                  _lib.stream_ptr())
         _lib.check(rc, "ssp_gmm_mstep")
-        return float(ll.item()) / n_total, n
+        return n, ll, counts.cpu().numpy() if reduce else counts
+
+    def _em(self, feats, seg, workspace, w, mu, var, nk_eps):
+        """The EM loop of :meth:`fit` (S = 1) and :func:`fit_batch`: S models from (w (S,K), mu, var (S,K,D)), segment s
+        of ``feats`` under model s, each to its own convergence as :func:`fit_batch` describes; the lower bound is the mean
+        frame log-likelihood under the parameters the E-step used.  Returns (w, mu, var, lower bound (S,), bounds of
+        every iteration (S lists), converged (S,), n_iter (S,))."""
+        torch = _lib.require_cuda()
+        ms = ModelSet(w, mu, var, device=feats.device)
+        lower = np.full(ms.n_models, -np.inf)
+        bounds = [[] for _ in range(ms.n_models)]
+        converged = np.zeros(ms.n_models, dtype=bool)
+        n_iter = np.zeros(ms.n_models, dtype=np.int64)
+        for it in range(1, self.max_iter + 1):
+            active = ~converged
+            if not active.any():
+                break
+            ms.repack(w, mu, var)
+            if active.all():  # the M-step in place
+                _, ll, cnt = self._em_step(ms, feats, seg, workspace, nk_eps, w, mu, var, timed=True)
+            else:
+                w_new, mu_new, var_new = torch.empty_like(w), torch.empty_like(mu), torch.empty_like(var)
+                _, ll, cnt = self._em_step(ms, feats, seg, workspace, nk_eps, w_new, mu_new, var_new, timed=True)
+                keep = torch.as_tensor(active, device=feats.device)
+                w = torch.where(keep[:, None], w_new, w)
+                mu = torch.where(keep[:, None, None], mu_new, mu)
+                var = torch.where(keep[:, None, None], var_new, var)
+            now = ll.cpu().numpy() / cnt          # the one host synchronisation of the iteration (a second with comm)
+            for i in np.nonzero(active)[0]:
+                bounds[i].append(float(now[i]))
+                n_iter[i] = it
+                if abs(now[i] - lower[i]) < self.tol:
+                    converged[i] = True
+                lower[i] = now[i]
+        return w, mu, var, lower, bounds, converged, n_iter
 
     def _kmeans_init(self, feats, seg, rs, w, mu, var, nk_eps, iters=10, workspace=None):
         """Lloyd iterations as hard EM: equal weights, one small shared variance, so posteriors are
@@ -575,13 +629,7 @@ class GaussianMixture:
         ms = ModelSet(w, mu, sharp, device=feats.device)
         for it in range(iters + 1):
             ms.repack(w, mu, sharp)
-            n, f, s, _ = ms.stats(feats, seg, workspace=workspace, reuse_images=True)
-            if comm is not None:
-                flat = reduced(torch.cat([n.reshape(-1), f.reshape(-1), s.reshape(-1)]))
-                n, f, s = flat[:k].reshape(1, k), flat[k : k + k * d].reshape(1, k, d), flat[k + k * d :].reshape(1, k, d)
-            rc = ms.lib.ssp_gmm_mstep(_lib.ptr(n), _lib.ptr(f), _lib.ptr(s), 1, k, d, float(self.reg_covar), float(nk_eps),
-                                      _lib.ptr(w), _lib.ptr(mu), _lib.ptr(var), _lib.stream_ptr())
-            _lib.check(rc, "ssp_gmm_mstep")
+            n, _, _ = self._em_step(ms, feats, seg, workspace, nk_eps, w, mu, var)
             empty = (n[0] < 0.5).nonzero().flatten()
             if it == iters:
                 # clusters still empty after the last Lloyd step would enter EM with mean 0 / var reg_covar; sklearn's
@@ -641,49 +689,22 @@ class GaussianMixture:
         torch = _lib.require_cuda()
         self._check()
         dev = torch.device(f"cuda:{torch.cuda.current_device()}")
-        x_dtype = X.dtype if isinstance(X, np.ndarray) and X.dtype in (np.float32, np.float64) else np.float64
-        if isinstance(X, torch.Tensor):
-            x_dtype = np.float32 if X.dtype == torch.float32 else np.float64
         feats = _as_feats(X, dev)
-        n_frames, d = feats.shape
-        k = self.n_components
-        if n_frames < 2:
-            raise ValueError(f"Found array with {n_frames} sample(s) while a minimum of 2 is required.")
-        if n_frames < k:
-            raise ValueError("Expected n_samples >= n_components "
-                             f"but got n_components = {k}, n_samples = {n_frames}")
-        nk_eps = 10.0 * float(np.finfo(x_dtype).eps)
-        seg = np.array([0, n_frames], dtype=np.int64)
-        rs = self.random_state if isinstance(self.random_state, np.random.RandomState) else np.random.RandomState(self.random_state)
+        seg = np.array([0, feats.shape[0]], dtype=np.int64)
+        _check_sample_counts(np.diff(seg), self.n_components)
+        nk_eps = _nk_eps(X)
+        rs = self._rng()
 
         do_init = not (self.warm_start and hasattr(self, "converged_"))
         best = None
         workspace = StatsWorkspace(dev)  # the frames' operand images are built by the first statistics call and reused
         for _init in range(self.n_init if do_init else 1):
             w, mu, var = self._initial_parameters(feats, seg, rs, nk_eps, do_init, workspace)
-            ms = ModelSet(w, mu, var, device=dev)
-            lower, bounds, converged, n_iter = -np.inf, [], False, 0
-            for n_iter in range(1, self.max_iter + 1):
-                prev = lower
-                ms.repack(w, mu, var)
-                lower, _ = self._em_iteration(ms, feats, seg, float(n_frames), nk_eps, w, mu, var, workspace)
-                bounds.append(lower)
-                if abs(lower - prev) < self.tol:
-                    converged = True
-                    break
-            if best is None or lower > best[0] or best[0] == -np.inf:
-                best = (lower, w.clone(), mu.clone(), var.clone(), n_iter, converged, bounds)
+            w, mu, var, lower, bounds, converged, n_iter = self._em(feats, seg, workspace, w, mu, var, nk_eps)
+            if best is None or lower[0] > best[0] or best[0] == -np.inf:
+                best = (lower[0], w[0], mu[0], var[0], n_iter[0], converged[0], bounds[0])
         lower, w, mu, var, n_iter, converged, bounds = best
-        if not converged and self.max_iter > 0:
-            warnings.warn("Best performing initialization did not converge. Try different init parameters, or "
-                          "increase max_iter, tol, or check for degenerate data.", UserWarning)
-        self._set_params_from_device(w[0], mu[0], var[0])
-        if not np.all(np.isfinite(self.covariances_)) or np.any(self.covariances_ <= 0):
-            raise ValueError("Fitting the mixture model failed because some components have ill-defined empirical "
-                             "covariance (for instance caused by singleton or collapsed samples). Try to decrease the "
-                             "number of components, increase reg_covar, or scale the input data.")
-        self.converged_, self.n_iter_, self.lower_bound_, self.lower_bounds_ = converged, n_iter, lower, bounds
-        self._ms = None
+        self._finish_em(w.cpu().numpy(), mu.cpu().numpy(), var.cpu().numpy(), converged, n_iter, lower, bounds)
         return feats, workspace
 
     # ------------------------------------------------------------------ scoring
@@ -750,12 +771,7 @@ class GaussianMixture:
     @classmethod
     def from_params(cls, weights, means, covariances, **kw):
         gm = cls(n_components=len(weights), **kw)
-        gm.weights_ = np.asarray(weights, dtype=np.float64)
-        gm.means_ = np.asarray(means, dtype=np.float64)
-        gm.covariances_ = np.asarray(covariances, dtype=np.float64)
-        gm.precisions_cholesky_ = 1.0 / np.sqrt(gm.covariances_)
-        gm.precisions_ = gm.precisions_cholesky_ ** 2
-        gm.converged_, gm.n_iter_, gm.lower_bound_ = True, 0, -np.inf
+        gm._set_fitted(weights, means, covariances, True, 0, -np.inf)
         return gm
 
     @classmethod
@@ -813,65 +829,19 @@ def fit_batch(X_list, n_components=1, **kwargs):
     d, k = feats.shape[1], n_components
     if 2 * d + 2 > 80:  # per-segment models need the tensor-core statistics kernels
         return [gm.fit(x) for gm, x in zip(gms, X_list)]
-    counts = np.diff(seg)
-    for cnt in counts:
-        if cnt < 2:
-            raise ValueError(f"Found array with {cnt} sample(s) while a minimum of 2 is required.")
-        if cnt < k:
-            raise ValueError(f"Expected n_samples >= n_components but got n_components = {k}, n_samples = {cnt}")
-    x_dtypes = [np.float32 if (isinstance(x, torch.Tensor) and x.dtype == torch.float32) or
-                (isinstance(x, np.ndarray) and x.dtype == np.float32) else np.float64 for x in X_list]
-    nk_eps = 10.0 * float(np.finfo(x_dtypes[0]).eps)
+    _check_sample_counts(np.diff(seg), k)
+    nk_eps = _nk_eps(X_list[0])
     # ---- initial parameters, per model (same code and RNG use as fit())
     w = torch.empty((n_models, k), dtype=torch.float64, device=dev)
     mu = torch.empty((n_models, k, d), dtype=torch.float64, device=dev)
     var = torch.empty((n_models, k, d), dtype=torch.float64, device=dev)
     for i, gm in enumerate(gms):
-        rs = gm.random_state if isinstance(gm.random_state, np.random.RandomState) else np.random.RandomState(gm.random_state)
         fi = feats[int(seg[i]) : int(seg[i + 1])]
-        wi, mi, vi = gm._initial_parameters(fi, np.array([0, fi.shape[0]], dtype=np.int64), rs, nk_eps, True, StatsWorkspace(dev))
+        wi, mi, vi = gm._initial_parameters(fi, np.array([0, fi.shape[0]], dtype=np.int64), gm._rng(), nk_eps, True, StatsWorkspace(dev))
         w[i], mu[i], var[i] = wi[0], mi[0], vi[0]
     # ---- batched EM
-    ms = ModelSet(w, mu, var, device=dev)
-    workspace = StatsWorkspace(dev)
-    t_counts = torch.as_tensor(counts.astype(np.float64), device=dev)
-    w_new, mu_new, var_new = torch.empty_like(w), torch.empty_like(mu), torch.empty_like(var)
-    lower = np.full(n_models, -np.inf)
-    bounds = [[] for _ in range(n_models)]
-    converged = np.zeros(n_models, dtype=bool)
-    n_iter = np.zeros(n_models, dtype=np.int64)
-    for it in range(1, g0.max_iter + 1):
-        active = ~converged
-        if not active.any():
-            break
-        ms.repack(w, mu, var)
-        n, f, s, ll = ms.stats(feats, seg, workspace=workspace, reuse_images=True)
-        rc = ms.lib.ssp_gmm_mstep(_lib.ptr(n), _lib.ptr(f), _lib.ptr(s), n_models, k, d, float(g0.reg_covar), float(nk_eps),
-                                  _lib.ptr(w_new), _lib.ptr(mu_new), _lib.ptr(var_new), _lib.stream_ptr())
-        _lib.check(rc, "ssp_gmm_mstep")
-        now = (ll / t_counts).cpu().numpy()          # the one host synchronisation of the iteration
-        keep = torch.as_tensor(active, device=dev)
-        w = torch.where(keep[:, None], w_new, w)
-        mu = torch.where(keep[:, None, None], mu_new, mu)
-        var = torch.where(keep[:, None, None], var_new, var)
-        for i in np.nonzero(active)[0]:
-            bounds[i].append(float(now[i]))
-            n_iter[i] = it
-            if abs(now[i] - lower[i]) < g0.tol:
-                converged[i] = True
-            lower[i] = now[i]
+    w, mu, var, lower, bounds, converged, n_iter = g0._em(feats, seg, StatsWorkspace(dev), w, mu, var, nk_eps)
     hw, hmu, hvar = w.cpu().numpy(), mu.cpu().numpy(), var.cpu().numpy()
     for i, gm in enumerate(gms):
-        if not converged[i] and gm.max_iter > 0:
-            warnings.warn("Best performing initialization did not converge. Try different init parameters, or "
-                          "increase max_iter, tol, or check for degenerate data.", UserWarning)
-        gm.weights_, gm.means_, gm.covariances_ = hw[i], hmu[i], hvar[i]
-        gm.precisions_cholesky_ = 1.0 / np.sqrt(gm.covariances_)
-        gm.precisions_ = gm.precisions_cholesky_ ** 2
-        if not np.all(np.isfinite(gm.covariances_)) or np.any(gm.covariances_ <= 0):
-            raise ValueError("Fitting the mixture model failed because some components have ill-defined empirical "
-                             "covariance (for instance caused by singleton or collapsed samples). Try to decrease the "
-                             "number of components, increase reg_covar, or scale the input data.")
-        gm.converged_, gm.n_iter_, gm.lower_bound_, gm.lower_bounds_ = bool(converged[i]), int(n_iter[i]), float(lower[i]), bounds[i]
-        gm._ms = None
+        gm._finish_em(hw[i], hmu[i], hvar[i], converged[i], n_iter[i], lower[i], bounds[i])
     return gms

@@ -23,7 +23,7 @@ from . import _lib
 from . import frontend as fe
 from .wavio import read_wav_batch
 from .mixture import (SINGLE_PASS_MIN_COMPONENTS, GaussianMixture, ModelSet, SharedModelSet, check_top_c, concat_utterances,
-                      fit_batch, resolve_precision)
+                      fit_batch, resolve_precision, stacked_params)
 
 
 def map_adapt(ubm: GaussianMixture, speaker_frames, relevance: float = 16.0, adapt=("means",), device=None):
@@ -62,9 +62,7 @@ def map_enrol(ubm: GaussianMixture, speaker_frames, relevance: float = 16.0, dev
     dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
     _, mu, _ = map_adapt(ubm, speaker_frames, relevance=relevance, adapt=("means",), device=dev)
     uw, umu, uvar = ubm._model_set()._params
-    sms = SharedModelSet(uw[0], uvar[0], torch.cat([mu, umu]), ref_model=-1, device=dev)
-    sms.ubm_index = sms.n_models - 1
-    return sms
+    return SharedModelSet.with_ubm(uw[0], uvar[0], mu, umu, device=dev)
 
 
 def _base_params(model):
@@ -75,6 +73,29 @@ def _base_params(model):
         w, _, var = model._params
         return w[0].cpu().numpy(), var[0].cpu().numpy()
     return np.asarray(model.weights_), np.asarray(model.covariances_)
+
+
+def _shares_base(weights, variances, ubm=None) -> bool:
+    """True if every speaker of the (S,K) / (S,K,D) numpy stacks carries the same weights and variances -- and, given a
+    ``ubm``, those are KNOWN to be the UBM's (mean-only MAP models adapted from it)."""
+    if not SharedModelSet.shares_base(weights, variances):
+        return False
+    if ubm is None:
+        return True
+    base = _base_params(ubm)
+    return base is not None and np.array_equal(base[0], weights[0]) and np.array_equal(base[1], variances[0])
+
+
+def _ubm_means(ubm):
+    return ubm._params[1] if isinstance(ubm, ModelSet) else np.asarray(ubm.means_)
+
+
+def _llr(scores, k):
+    """(pred (N, S) numpy, argmax (N,)) from the scores of a set whose column ``k`` is the UBM: every other column minus
+    column ``k``."""
+    keep = [i for i in range(scores.shape[1]) if i != k]
+    pred = (scores[:, keep] - scores[:, k : k + 1]).cpu().numpy()
+    return pred, pred.argmax(axis=1)
 
 
 def _top_c_set(speakers, ubm, dev):
@@ -90,8 +111,7 @@ def _top_c_set(speakers, ubm, dev):
         return speakers, k
     if ubm is None:
         raise ValueError("top_c scores against a UBM: pass ubm=, or a SharedModelSet from map_enrol")
-    base = _base_params(ubm)
-    if base is None:
+    if isinstance(ubm, ModelSet) and ubm.n_models != 1:
         raise ValueError("ubm must be ONE model")
     if isinstance(speakers, SharedModelSet):
         w, var, mu = (t.cpu().numpy() for t in speakers._params)
@@ -99,15 +119,36 @@ def _top_c_set(speakers, ubm, dev):
     elif isinstance(speakers, ModelSet):
         sw, smu, svar = (t.cpu().numpy() for t in speakers._params)
     else:
-        sw = np.stack([np.asarray(m.weights_) for m in speakers])
-        smu = np.stack([np.asarray(m.means_) for m in speakers])
-        svar = np.stack([np.asarray(m.covariances_) for m in speakers])
-    if not (SharedModelSet.shares_base(sw, svar) and np.array_equal(base[0], sw[0]) and np.array_equal(base[1], svar[0])):
+        sw, smu, svar = stacked_params(speakers)
+    if not _shares_base(sw, svar, ubm):
         raise NotImplementedError("top_c needs speaker models that share the UBM's weights and variances (mean-only MAP "
                                   "enrolment): there is no component correspondence otherwise")
-    umu = ubm._params[1][0].cpu().numpy() if isinstance(ubm, ModelSet) else np.asarray(ubm.means_)
-    sms = SharedModelSet(base[0], base[1], np.concatenate([smu, umu[None]]), ref_model=-1, device=dev)
-    return sms, sms.n_models - 1
+    sms = SharedModelSet.with_ubm(sw[0], svar[0], smu, _ubm_means(ubm), device=dev)
+    return sms, sms.ubm_index
+
+
+def _exact_set(speakers, ubm, precision, dev):
+    """(model set that scores ``speakers`` exactly at ``precision``, column of the UBM in it or None -- then the UBM, if
+    any, is scored on its own)."""
+    if isinstance(speakers, SharedModelSet) and getattr(speakers, "ubm_index", None) is not None and ubm is None:
+        return speakers, speakers.ubm_index   # map_enrol: the UBM rides along as one of the mean sets
+    if isinstance(speakers, SharedModelSet):
+        return (speakers if precision in ("tf32", "auto") else speakers.expand()), None
+    if isinstance(speakers, ModelSet):
+        return speakers, None
+    sw, smu, svar = stacked_params(speakers)
+    single_pass = precision == "tf32" or (precision == "auto" and sw.shape[1] >= SINGLE_PASS_MIN_COMPONENTS)
+    # mean-only MAP speakers (e.g. unpickled models adapted from this UBM): shared-variance kernel, with the UBM as one
+    # more mean set
+    if single_pass and smu.shape[2] <= 39 and _shares_base(sw, svar, ubm):
+        try:
+            if ubm is None:
+                return SharedModelSet(sw[0], svar[0], smu, device=dev), None
+            sms = SharedModelSet.with_ubm(sw[0], svar[0], smu, _ubm_means(ubm), device=dev)
+            return sms, sms.ubm_index
+        except NotImplementedError:   # parameters outside the FP16 range of that kernel: general kernel below
+            pass
+    return ModelSet(sw, smu, svar, device=dev), None
 
 
 def identify(utts, speakers, ubm=None, precision="auto", device=None, top_c=None):
@@ -136,49 +177,11 @@ def identify(utts, speakers, ubm=None, precision="auto", device=None, top_c=None
             sms, k = _top_c_set(speakers, ubm, dev)
             check_top_c(top_c, sms.n_comp)
             feats, offs = concat_utterances(utts, dev)
-            scores, _ = sms.score_top_c(feats, offs, c=top_c)
-            keep = [i for i in range(sms.n_models) if i != k]
-            pred = (scores[:, keep] - scores[:, k : k + 1]).cpu().numpy()
-            return pred, pred.argmax(axis=1)
+            return _llr(sms.score_top_c(feats, offs, c=top_c)[0], k)
         feats, offs = concat_utterances(utts, dev)
-        if isinstance(speakers, SharedModelSet) and getattr(speakers, "ubm_index", None) is not None and ubm is None:
-            # the UBM rides along as one of the mean sets (map_enrol): one launch scores everything
-            scores, _ = speakers.score(feats, offs)
-            k = speakers.ubm_index
-            keep = [i for i in range(speakers.n_models) if i != k]
-            pred = (scores[:, keep] - scores[:, k : k + 1]).cpu().numpy()
-            return pred, pred.argmax(axis=1)
-        if isinstance(speakers, (ModelSet, SharedModelSet)):
-            ms = speakers
-        else:
-            sw = np.stack([np.asarray(m.weights_) for m in speakers])
-            smu = np.stack([np.asarray(m.means_) for m in speakers])
-            svar = np.stack([np.asarray(m.covariances_) for m in speakers])
-            single_pass = precision == "tf32" or (precision == "auto" and sw.shape[1] >= SINGLE_PASS_MIN_COMPONENTS)
-            base = _base_params(ubm) if ubm is not None else None
-            # mean-only MAP speakers (e.g. unpickled models adapted from this UBM): shared-variance kernel, with the UBM
-            # as one more mean set -- only when the UBM (if any) is KNOWN to carry the same weights and variances
-            if (single_pass and smu.shape[2] <= 39 and SharedModelSet.shares_base(sw, svar)
-                    and (ubm is None or (base is not None and np.array_equal(base[0], sw[0]) and np.array_equal(base[1], svar[0])))):
-                if ubm is None:
-                    means = smu
-                elif isinstance(ubm, ModelSet):
-                    means = np.concatenate([smu, ubm._params[1].cpu().numpy()])
-                else:
-                    means = np.concatenate([smu, np.asarray(ubm.means_)[None]])
-                try:
-                    sms = SharedModelSet(sw[0], svar[0], means, ref_model=-1, device=dev)
-                except NotImplementedError:   # parameters outside the FP16 range of that kernel: general kernel below
-                    sms = None
-                if sms is not None:
-                    scores, _ = sms.score(feats, offs)
-                    if ubm is not None:
-                        scores = scores[:, :-1] - scores[:, -1:]
-                    pred = scores.cpu().numpy()
-                    return pred, pred.argmax(axis=1)
-            ms = ModelSet(sw, smu, svar, device=dev)
-        if isinstance(ms, SharedModelSet) and precision not in ("tf32", "auto"):
-            ms = ms.expand()
+        ms, k = _exact_set(speakers, ubm, precision, dev)
+        if k is not None:   # one launch scores speakers and UBM
+            return _llr(ms.score(feats, offs)[0], k)
         scores, _ = ms.score(feats, offs, precision=precision)
         if ubm is not None:
             ums = ubm if isinstance(ubm, ModelSet) else ModelSet(ubm.weights_, ubm.means_, ubm.covariances_, device=dev)
