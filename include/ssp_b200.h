@@ -341,6 +341,27 @@ int ssp_gmm_score_topc(const float* feats, const int64_t* frame_offsets, int64_t
                        double* out_scores, float* out_frame_lse, void* workspace, int64_t workspace_bytes, void* stream);
 
 /*
+ * Top-C scoring of a model set MAP-adapted from its reference member r in weights and variances too (component c of
+ * every model is component c of r): as ssp_gmm_score_topc, with
+ *   L_s,c(t) = L_r,c(t) + k_s,c + a_s,c . y + b_s,c . y^2,   y = x_t - mu_r,c,   delta = mu_s,c - mu_r,c,
+ *   a = delta / var_s,c,   b = -1/2 (1/var_s,c - 1/var_r,c),
+ *   k = log(w_s,c / w_r,c) - 1/2 sum_d log(var_s,c / var_r,c) - 1/2 sum_d delta^2 / var_s,c.
+ * A model (or component) with the reference's parameters has a row of zeros and scores L_r,c(t) bit for bit.
+ * The pack: the table [K][S][roundup(2D + 1, 4)] FP32 rows [a (D), b (D), k, 0..] computed in double, then the reference
+ * means [K][roundup(D, 4)] in FP32; ssp_gmm_topc_adapted_pack_bytes() bytes, 16-byte aligned.  weights [S][K], means and
+ * variances [S][K][D] double (positive, finite weights and variances: the table takes their logarithms), D <= 39,
+ * ref_model in [0, S).  ssp_gmm_score_topc_adapted takes the arguments of ssp_gmm_score_topc, with this pack, and its
+ * workspace from ssp_gmm_score_topc_workspace_bytes().
+ */
+int64_t ssp_gmm_topc_adapted_pack_bytes(const ssp_gmm_dims* dims);
+int ssp_gmm_pack_topc_adapted(const double* weights, const double* means, const double* variances, const ssp_gmm_dims* dims,
+                              int32_t ref_model, void* out_pack, void* stream);
+int ssp_gmm_score_topc_adapted(const float* feats, const int64_t* frame_offsets, int64_t n_utts, int64_t total_frames,
+                               const int32_t* idx, const float* logit, int32_t c, const void* pack, const ssp_gmm_dims* dims,
+                               double* out_scores, float* out_frame_lse, void* workspace, int64_t workspace_bytes,
+                               void* stream);
+
+/*
  * M-step on device (sklearn _gaussian_mixture.py:312-313,250-252,898): from (all-reduced)
  * statistics to weights/means/variances, double precision, for n_models models at once (arrays [n_models][K](xD)).
  * nk = N + 10*eps_of(stat_dtype); mu = F/nk; var = S/nk - mu^2 + reg_covar; w = nk/sum(nk).

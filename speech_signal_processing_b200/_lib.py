@@ -80,6 +80,9 @@ PROTOTYPES = {
     "ssp_gmm_topc_chunk_frames": (_I64, []),
     "ssp_gmm_score_topc_workspace_bytes": (_I64, [C.POINTER(GmmDims), _I32, _I64]),
     "ssp_gmm_score_topc": (C.c_int, [_P, _P, _I64, _I64, _P, _P, _I32, _P, C.POINTER(GmmDims), _P, _P, _P, _I64, _P]),
+    "ssp_gmm_topc_adapted_pack_bytes": (_I64, [C.POINTER(GmmDims)]),
+    "ssp_gmm_pack_topc_adapted": (C.c_int, [_P, _P, _P, C.POINTER(GmmDims), _I32, _P, _P]),
+    "ssp_gmm_score_topc_adapted": (C.c_int, [_P, _P, _I64, _I64, _P, _P, _I32, _P, C.POINTER(GmmDims), _P, _P, _P, _I64, _P]),
     "ssp_gmm_mstep": (C.c_int, [_P, _P, _P, _I32, _I32, _I32, C.c_double, C.c_double, _P, _P, _P, _P]),
     "ssp_gmm_map_adapt": (C.c_int, [_P, _P, _P, _P, _I64, _P, _P, _P, _I32, _I32, C.c_double, _I32, _P, _P, _P, _P]),
     "ssp_dtw_max_len": (_I64, [_I32]),

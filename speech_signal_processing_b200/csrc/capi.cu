@@ -264,6 +264,21 @@ extern "C" int ssp_gmm_pack_topc(const double* variances, const double* means, c
                                (cudaStream_t)stream);
 }
 
+extern "C" int64_t ssp_gmm_topc_adapted_pack_bytes(const ssp_gmm_dims* dims) {
+  return topc_dims_ok(dims) ? ssp::topc_adapted_pack_bytes(dims->n_models, dims->n_comp, dims->n_feat) : 0;
+}
+
+extern "C" int ssp_gmm_pack_topc_adapted(const double* weights, const double* means, const double* variances,
+                                         const ssp_gmm_dims* dims, int32_t ref_model, void* out_pack, void* stream) {
+  SSP_REQUIRE(topc_dims_ok(dims), "ssp_gmm_pack_topc_adapted: unsupported dims (need 1 <= D <= %d)", ssp::kTopcMaxFeat);
+  SSP_REQUIRE(weights && means && variances && out_pack, "ssp_gmm_pack_topc_adapted: null pointer");
+  SSP_REQUIRE(((uintptr_t)out_pack & 15) == 0, "ssp_gmm_pack_topc_adapted: out_pack must be 16-byte aligned");
+  SSP_REQUIRE(ref_model >= 0 && ref_model < dims->n_models, "ssp_gmm_pack_topc_adapted: ref_model %d outside [0, %d)",
+              ref_model, dims->n_models);
+  return ssp::launch_pack_topc_adapted(weights, means, variances, dims->n_models, dims->n_comp, dims->n_feat, ref_model,
+                                       out_pack, (cudaStream_t)stream);
+}
+
 extern "C" int64_t ssp_gmm_topc_chunk_frames(void) { return ssp::kTopcChunkFrames; }
 
 extern "C" int64_t ssp_gmm_score_topc_workspace_bytes(const ssp_gmm_dims* dims, int32_t c, int64_t total_frames) {
@@ -271,21 +286,37 @@ extern "C" int64_t ssp_gmm_score_topc_workspace_bytes(const ssp_gmm_dims* dims, 
   return ssp::score_topc_workspace_bytes(dims->n_models, dims->n_comp, c, total_frames);
 }
 
-extern "C" int ssp_gmm_score_topc(const float* feats, const int64_t* frame_offsets, int64_t n_utts, int64_t total_frames,
-                                  const int32_t* idx, const float* logit, int32_t c, const void* pack, const ssp_gmm_dims* dims,
-                                  double* out_scores, float* out_frame_lse, void* workspace, int64_t workspace_bytes,
-                                  void* stream) {
-  SSP_REQUIRE(topc_dims_ok(dims), "ssp_gmm_score_topc: unsupported dims (need 1 <= D <= %d)", ssp::kTopcMaxFeat);
-  SSP_REQUIRE(c >= 1 && c <= dims->n_comp && c <= ssp::kTopcMaxC, "ssp_gmm_score_topc: C = %d outside [1, min(K = %d, %d)]", c,
+// ssp_gmm_score_topc (adapted == false) and ssp_gmm_score_topc_adapted: the same checks, the same workspace
+static int score_topc(const char* fn, bool adapted, const float* feats, const int64_t* frame_offsets, int64_t n_utts,
+                      int64_t total_frames, const int32_t* idx, const float* logit, int32_t c, const void* pack,
+                      const ssp_gmm_dims* dims, double* out_scores, float* out_frame_lse, void* workspace,
+                      int64_t workspace_bytes, void* stream) {
+  SSP_REQUIRE(topc_dims_ok(dims), "%s: unsupported dims (need 1 <= D <= %d)", fn, ssp::kTopcMaxFeat);
+  SSP_REQUIRE(c >= 1 && c <= dims->n_comp && c <= ssp::kTopcMaxC, "%s: C = %d outside [1, min(K = %d, %d)]", fn, c,
               dims->n_comp, ssp::kTopcMaxC);
-  SSP_REQUIRE(frame_offsets && pack && out_scores && ((feats && idx && logit) || total_frames == 0),
-              "ssp_gmm_score_topc: null pointer");
-  SSP_REQUIRE(((uintptr_t)pack & 15) == 0, "ssp_gmm_score_topc: pack must be 16-byte aligned");
-  SSP_REQUIRE(n_utts >= 0 && total_frames >= 0, "ssp_gmm_score_topc: negative size");
-  int rc = check_workspace("ssp_gmm_score_topc", workspace, workspace_bytes,
+  SSP_REQUIRE(frame_offsets && pack && out_scores && ((feats && idx && logit) || total_frames == 0), "%s: null pointer", fn);
+  SSP_REQUIRE(((uintptr_t)pack & 15) == 0, "%s: pack must be 16-byte aligned", fn);
+  SSP_REQUIRE(n_utts >= 0 && total_frames >= 0, "%s: negative size", fn);
+  int rc = check_workspace(fn, workspace, workspace_bytes,
                            ssp::score_topc_workspace_bytes(dims->n_models, dims->n_comp, c, total_frames),
                            "ssp_gmm_score_topc_workspace_bytes");
   if (rc != SSP_OK || n_utts == 0) return rc;
   return ssp::launch_score_topc(feats, frame_offsets, n_utts, total_frames, idx, logit, c, pack, dims->n_models, dims->n_comp,
-                                dims->n_feat, out_scores, out_frame_lse, workspace, (cudaStream_t)stream);
+                                dims->n_feat, adapted, out_scores, out_frame_lse, workspace, (cudaStream_t)stream);
+}
+
+extern "C" int ssp_gmm_score_topc(const float* feats, const int64_t* frame_offsets, int64_t n_utts, int64_t total_frames,
+                                  const int32_t* idx, const float* logit, int32_t c, const void* pack, const ssp_gmm_dims* dims,
+                                  double* out_scores, float* out_frame_lse, void* workspace, int64_t workspace_bytes,
+                                  void* stream) {
+  return score_topc("ssp_gmm_score_topc", false, feats, frame_offsets, n_utts, total_frames, idx, logit, c, pack, dims,
+                    out_scores, out_frame_lse, workspace, workspace_bytes, stream);
+}
+
+extern "C" int ssp_gmm_score_topc_adapted(const float* feats, const int64_t* frame_offsets, int64_t n_utts,
+                                          int64_t total_frames, const int32_t* idx, const float* logit, int32_t c,
+                                          const void* pack, const ssp_gmm_dims* dims, double* out_scores,
+                                          float* out_frame_lse, void* workspace, int64_t workspace_bytes, void* stream) {
+  return score_topc("ssp_gmm_score_topc_adapted", true, feats, frame_offsets, n_utts, total_frames, idx, logit, c, pack, dims,
+                    out_scores, out_frame_lse, workspace, workspace_bytes, stream);
 }

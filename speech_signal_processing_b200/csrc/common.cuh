@@ -227,16 +227,24 @@ constexpr int kTopcMaxFeat = 39;
 // C = 5 and 1001 models, L2-sized) and each component receives about kTopcChunkFrames * C / K routed pairs per chunk
 constexpr int64_t kTopcChunkFrames = 4096;
 inline int topc_row_floats(int D) { return (D + 1 + 3) / 4 * 4; }  // [a (D), b, 0..] per (component, model)
+// adapted sets (weights and variances per model too): [a (D), b (D), k, 0..] per (component, model), then the reference
+// means [K][roundup(D, 4)]
+inline int topc_adapted_row_floats(int D) { return (2 * D + 1 + 3) / 4 * 4; }
+inline int topc_ref_floats(int D) { return (D + 3) / 4 * 4; }
 int64_t topc_tc_workspace_bytes(const PackLayout& L, int64_t total_frames, int64_t n_segs, int c);
 int launch_topc_tc(const float* feats, const int64_t* seg_offsets, int64_t n_segs, int64_t total_frames, const void* pack,
                    const PackLayout& L, int c, int32_t* out_idx, float* out_logit, void* workspace, bool reuse_images,
                    cudaStream_t st);
 int64_t topc_pack_bytes(int S, int K, int D);
 int launch_pack_topc(const double* var, const double* mu, int S, int K, int D, int ref, void* pack, cudaStream_t st);
+int64_t topc_adapted_pack_bytes(int S, int K, int D);
+int launch_pack_topc_adapted(const double* w, const double* mu, const double* var, int S, int K, int D, int ref, void* pack,
+                             cudaStream_t st);
 int64_t score_topc_workspace_bytes(int S, int K, int C, int64_t T);
+// adapted: `pack` is a ssp_gmm_pack_topc_adapted table, else a ssp_gmm_pack_topc one
 int launch_score_topc(const float* feats, const int64_t* offsets, int64_t n_utts, int64_t T, const int32_t* idx,
-                      const float* logit, int C, const void* pack, int S, int K, int D, double* scores, float* frame_lse,
-                      void* workspace, cudaStream_t st);
+                      const float* logit, int C, const void* pack, int S, int K, int D, bool adapted, double* scores,
+                      float* frame_lse, void* workspace, cudaStream_t st);
 // workspace of the CUDA-core posterior path: per-segment sums of the scoring kernel, then the per-frame lse
 inline int64_t posteriors_simt_lse_offset(int64_t n_segs) { return (8 * n_segs + 255) / 256 * 256; }
 inline int64_t posteriors_simt_workspace_bytes(int64_t total_frames, int64_t n_segs) {

@@ -14,6 +14,15 @@
 //                                     sums in double
 // At a chunk of 4096 frames a component receives about 4096 C / K routed pairs (20 at C = 5, K = 1024): too few rows
 // for a 128-row tcgen05 tile, so the product runs on the CUDA cores, where the difference term is FP32-exact.
+//
+// Model sets MAP-adapted in weights and variances too (ssp_gmm_score_topc_adapted) keep the component correspondence
+// with the reference and differ from it by a quadratic form.  The product block of component c centres its frames on
+// mu_r,c (y = x - mu_r,c, delta = mu_s,c - mu_r,c), and topc_adapted_product_kernel computes
+//   L_s,c(t) = L_r,c(t) + a . y + b . y^2 + k,   a = delta / var_s,   b = -1/2 (1/var_s - 1/var_r),
+//   k = log(w_s / w_r) - 1/2 sum_d log(var_s / var_r) - 1/2 sum_d delta^2 / var_s
+// with the frames routed to c being the ones that selected it, |y| is of the order of sigma, and a member (or component)
+// with the reference's parameters has a row of zeros, so its value is L_r,c(t) bit for bit.  Routing, combine and
+// finalize are the same kernels for both forms.
 #include <algorithm>
 
 #include "common.cuh"
@@ -44,6 +53,31 @@ __global__ void __launch_bounds__(256) topc_pack_kernel(const double* __restrict
   }
   row[D] = (float)(-0.5 * b);
   for (int d = D + 1; d < DA; ++d) row[d] = 0.f;
+}
+
+// pack[c][s][0 .. DA) = a_s,c (D values), b_s,c (D values), k_s,c, zeros; after the K * S rows, mur[c][0 .. DR) = mu_r,c
+// in FP32, zero padded (the centring of the product's staging).  One thread per (component, model), double inside.
+__global__ void __launch_bounds__(256) topc_adapted_pack_kernel(const double* __restrict__ w, const double* __restrict__ mu,
+                                                                const double* __restrict__ var, int S, int K, int D, int DA,
+                                                                int DR, int ref, float* __restrict__ pack) {
+  const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
+  if (i >= (int64_t)K * S) return;
+  const int c = (int)(i / S), s = (int)(i % S);
+  const int64_t os = ((int64_t)s * K + c) * D, orf = ((int64_t)ref * K + c) * D;
+  float* row = pack + i * DA;
+  double k = log(w[(int64_t)s * K + c] / w[(int64_t)ref * K + c]);
+  for (int d = 0; d < D; ++d) {
+    const double delta = mu[os + d] - mu[orf + d], vs = var[os + d], vr = var[orf + d];
+    row[d] = (float)(delta / vs);
+    row[D + d] = (float)(-0.5 * (1.0 / vs - 1.0 / vr));
+    k -= 0.5 * (log(vs / vr) + delta * delta / vs);
+  }
+  row[2 * D] = (float)k;
+  for (int d = 2 * D + 1; d < DA; ++d) row[d] = 0.f;
+  if (s == 0) {
+    float* m = pack + (int64_t)K * S * DA + (int64_t)c * DR;
+    for (int d = 0; d < DR; ++d) m[d] = d < D ? (float)mu[orf + d] : 0.f;
+  }
 }
 
 // ------------------------------------------------------------------------------------------------ routing
@@ -164,6 +198,66 @@ __global__ void __launch_bounds__(kThreads) topc_product_kernel(const Product p)
   }
 }
 
+// The adapted form: as topc_product_kernel, with the row (a, b, k) of topc_adapted_pack_kernel and the routed frames
+// staged as [y, y^2, 1, 0..], y = x - mu_r,c (mur: the FP32 reference means after the table)
+template <int NQ>  // roundup(2D + 1, 4) / 4
+__global__ void __launch_bounds__(kThreads) topc_adapted_product_kernel(const Product p, const float* __restrict__ mur) {
+  constexpr int DA = 4 * NQ;
+  __shared__ __align__(16) float sx[kBatch][DA];
+  __shared__ float sl[kBatch];
+  __shared__ int32_t sq[kBatch];
+  const int c = blockIdx.x, tid = threadIdx.x;
+  const int n = p.cnt[c];
+  if (n == 0) return;
+  const int start = p.off[c] - n;
+  const int s = blockIdx.y * kThreads + tid;
+  const bool live = s < p.S;
+  const float* m = mur + (int64_t)c * ((p.D + 3) / 4 * 4);
+  float4 a[NQ];
+  {
+    const float4* row = reinterpret_cast<const float4*>(p.pack + ((int64_t)c * p.S + (live ? s : 0)) * DA);
+#pragma unroll
+    for (int q = 0; q < NQ; ++q) a[q] = __ldg(row + q);
+  }
+  for (int b0 = 0; b0 < n; b0 += kBatch) {
+    const int nb = min(kBatch, n - b0);
+    __syncthreads();
+    if (tid < nb) {
+      const int q = __ldg(p.list + start + b0 + tid);
+      sq[tid] = q;
+      sl[tid] = __ldg(p.logit + p.t0 * p.C + q);
+    }
+    for (int e = tid; e < nb * DA; e += kThreads) {
+      const int i = e / DA, d = e % DA;
+      float val = d == 2 * p.D ? 1.f : 0.f;
+      if (d < 2 * p.D) {
+        const int j = d < p.D ? d : d - p.D;
+        const int64_t t = p.t0 + __ldg(p.list + start + b0 + i) / p.C;
+        const float y = __ldg(p.feats + t * p.D + j) - __ldg(m + j);
+        val = d < p.D ? y : y * y;
+      }
+      sx[i][d] = val;
+    }
+    __syncthreads();
+    if (live) {
+#pragma unroll 2
+      for (int i = 0; i < nb; ++i) {
+        const float4* x = reinterpret_cast<const float4*>(sx[i]);
+        float acc0 = 0.f, acc1 = 0.f;
+#pragma unroll
+        for (int q = 0; q < NQ; ++q) {
+          const float4 xv = x[q];
+          acc0 = fmaf(a[q].x, xv.x, acc0);
+          acc1 = fmaf(a[q].y, xv.y, acc1);
+          acc0 = fmaf(a[q].z, xv.z, acc0);
+          acc1 = fmaf(a[q].w, xv.w, acc1);
+        }
+        __stcg(p.v + (int64_t)sq[i] * p.S + s, sl[i] + (acc0 + acc1));
+      }
+    }
+  }
+}
+
 // ------------------------------------------------------------------------------------------------ combine
 // grid = (model tiles, frame groups of kCombineFrames); thread == model, walking the group's frames in order and carrying
 // the running sum of the current utterance until it changes
@@ -246,11 +340,24 @@ int launch_pack_topc(const double* var, const double* mu, int S, int K, int D, i
   return SSP_OK;
 }
 
+int64_t topc_adapted_pack_bytes(int S, int K, int D) {
+  return ((int64_t)K * S * topc_adapted_row_floats(D) + (int64_t)K * topc_ref_floats(D)) * (int64_t)sizeof(float);
+}
+
+int launch_pack_topc_adapted(const double* w, const double* mu, const double* var, int S, int K, int D, int ref, void* pack,
+                             cudaStream_t st) {
+  const int64_t n = (int64_t)K * S;
+  topc::topc_adapted_pack_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(w, mu, var, S, K, D, topc_adapted_row_floats(D),
+                                                                              topc_ref_floats(D), ref, (float*)pack);
+  SSP_LAUNCH_CHECK("topc_adapted_pack_kernel");
+  return SSP_OK;
+}
+
 int64_t score_topc_workspace_bytes(int S, int K, int C, int64_t T) { return (int64_t)topc::ws_layout(K, S, C, T).bytes; }
 
 int launch_score_topc(const float* feats, const int64_t* offsets, int64_t n_utts, int64_t T, const int32_t* idx,
-                      const float* logit, int C, const void* pack, int S, int K, int D, double* scores, float* frame_lse,
-                      void* workspace, cudaStream_t st) {
+                      const float* logit, int C, const void* pack, int S, int K, int D, bool adapted, double* scores,
+                      float* frame_lse, void* workspace, cudaStream_t st) {
   using namespace topc;
   SSP_CUDA_OK(cudaMemsetAsync(scores, 0, sizeof(double) * n_utts * S, st));
   if (T > 0) {
@@ -275,7 +382,8 @@ int launch_score_topc(const float* feats, const int64_t* offsets, int64_t n_utts
     topc_scatter_kernel<<<g_pairs, 256, 0, st>>>(r);
     SSP_LAUNCH_CHECK("topc_scatter_kernel");
     float* v = (float*)(base + w.o_v);
-    const int DA = topc_row_floats(D);
+    const int DA = adapted ? topc_adapted_row_floats(D) : topc_row_floats(D);
+    const float* mur = (const float*)pack + (int64_t)K * S * DA;   // adapted: the reference means after the table
     const unsigned m_tiles = (unsigned)((S + kThreads - 1) / kThreads);
     for (int64_t ch = 0; ch < w.n_chunks; ++ch) {
       const int64_t t0 = ch * kTopcChunkFrames, t1 = std::min<int64_t>(T, t0 + kTopcChunkFrames);
@@ -293,15 +401,29 @@ int launch_score_topc(const float* feats, const int64_t* offsets, int64_t n_utts
       p.D = D;
       p.v = v;
       const dim3 grid((unsigned)K, m_tiles);
+      if (adapted) {
+#define SSP_TOPC_PRODUCT(nq) \
+  case nq: topc_adapted_product_kernel<nq><<<grid, kThreads, 0, st>>>(p, mur); break;
+        switch (DA / 4) {
+          SSP_TOPC_PRODUCT(1) SSP_TOPC_PRODUCT(2) SSP_TOPC_PRODUCT(3) SSP_TOPC_PRODUCT(4) SSP_TOPC_PRODUCT(5)
+          SSP_TOPC_PRODUCT(6) SSP_TOPC_PRODUCT(7) SSP_TOPC_PRODUCT(8) SSP_TOPC_PRODUCT(9) SSP_TOPC_PRODUCT(10)
+          SSP_TOPC_PRODUCT(11) SSP_TOPC_PRODUCT(12) SSP_TOPC_PRODUCT(13) SSP_TOPC_PRODUCT(14) SSP_TOPC_PRODUCT(15)
+          SSP_TOPC_PRODUCT(16) SSP_TOPC_PRODUCT(17) SSP_TOPC_PRODUCT(18) SSP_TOPC_PRODUCT(19) SSP_TOPC_PRODUCT(20)
+          default: SSP_REQUIRE(false, "ssp_gmm_score_topc_adapted: feature width %d", D);
+        }
+#undef SSP_TOPC_PRODUCT
+        SSP_LAUNCH_CHECK("topc_adapted_product_kernel");
+      } else {
 #define SSP_TOPC_PRODUCT(nq) \
   case nq: topc_product_kernel<nq><<<grid, kThreads, 0, st>>>(p); break;
-      switch (DA / 4) {
-        SSP_TOPC_PRODUCT(1) SSP_TOPC_PRODUCT(2) SSP_TOPC_PRODUCT(3) SSP_TOPC_PRODUCT(4) SSP_TOPC_PRODUCT(5)
-        SSP_TOPC_PRODUCT(6) SSP_TOPC_PRODUCT(7) SSP_TOPC_PRODUCT(8) SSP_TOPC_PRODUCT(9) SSP_TOPC_PRODUCT(10)
-        default: SSP_REQUIRE(false, "ssp_gmm_score_topc: feature width %d", D);
-      }
+        switch (DA / 4) {
+          SSP_TOPC_PRODUCT(1) SSP_TOPC_PRODUCT(2) SSP_TOPC_PRODUCT(3) SSP_TOPC_PRODUCT(4) SSP_TOPC_PRODUCT(5)
+          SSP_TOPC_PRODUCT(6) SSP_TOPC_PRODUCT(7) SSP_TOPC_PRODUCT(8) SSP_TOPC_PRODUCT(9) SSP_TOPC_PRODUCT(10)
+          default: SSP_REQUIRE(false, "ssp_gmm_score_topc: feature width %d", D);
+        }
 #undef SSP_TOPC_PRODUCT
-      SSP_LAUNCH_CHECK("topc_product_kernel");
+        SSP_LAUNCH_CHECK("topc_product_kernel");
+      }
       Combine q;
       q.v = v;
       q.idx = idx;

@@ -145,12 +145,44 @@ class ModelSet:
             raise ValueError(f"unsupported GMM dims K={self.n_comp} D={self.n_feat} (need 1 <= D <= 80)")
         self.pack = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
         self._ws = StatsWorkspace(self.device)  # the calls given no workspace of their own
+        self.ubm_index = None   # set by with_ubm
         self.repack(w, mu, var)
+
+    @classmethod
+    def with_ubm(cls, weights, means, variances, ubm, device=None):
+        """Speakers MAP-adapted from ``ubm`` in any of weights, means and variances (``weights`` (S,K), ``means`` and
+        ``variances`` (S,K,D), e.g. :func:`~speech_signal_processing_b200.ubm.map_adapt`) and the UBM as one set: the UBM
+        is model S and ``ubm_index`` names it.  That declares that component c of every speaker is component c of the UBM,
+        which :meth:`score_top_c` needs, and lets ``identify`` score the UBM in the same launch as the speakers.  ``ubm``:
+        a fitted GaussianMixture-like or a one-model :class:`ModelSet`.  Weights and variances must be positive and finite
+        (``ValueError`` otherwise, before anything is launched): the top-C table takes their logarithms, and a variance
+        MAP at relevance 0 gives a component of one frame a zero variance."""
+        torch = _lib.require_cuda()
+        dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
+        if isinstance(ubm, ModelSet):
+            if ubm.n_models != 1:
+                raise ValueError(f"ubm must be ONE model (got a ModelSet of {ubm.n_models})")
+            ubm_params = ubm._params
+        else:
+            ubm_params = (ubm.weights_, ubm.means_, ubm.covariances_)
+        w, mu, var = (_as_params(a, dev) for a in (weights, means, variances))
+        uw, umu, uvar = (_as_params(a, dev) for a in ubm_params)
+        if mu.dim() != 3 or var.shape != mu.shape or w.shape != mu.shape[:2] or umu.numel() != mu.shape[1] * mu.shape[2] \
+                or uvar.numel() != umu.numel() or uw.numel() != mu.shape[1]:
+            raise ValueError("expected weights (S,K), means (S,K,D), variances (S,K,D) and a UBM of the same K and D")
+        w, mu, var = (torch.cat([a, u.reshape(1, *a.shape[1:])]) for a, u in ((w, uw), (mu, umu), (var, uvar)))
+        for name, a in (("weights", w), ("variances", var)):
+            if not bool((torch.isfinite(a) & (a > 0)).all().item()):
+                raise ValueError(f"{name} must be positive and finite (the speakers' and the UBM's)")
+        ms = cls(w, mu, var, device=dev)
+        ms.ubm_index = ms.n_models - 1
+        return ms
 
     @_lib.on_device
     def repack(self, w, mu, var):
         """Re-derive the packed operands from (device, float64) parameters -- one tiny kernel."""
         self._params = (w, mu, var)
+        self._topc = None   # score_top_c's UBM set and table are rebuilt from the new parameters
         _lib.check(self.lib.ssp_gmm_pack_models(_lib.ptr(w), _lib.ptr(mu), _lib.ptr(var), C.byref(self.dims),
                                                 _lib.ptr(self.pack), _lib.stream_ptr()), "ssp_gmm_pack_models")
 
@@ -257,6 +289,38 @@ class ModelSet:
                            C.byref(self.dims), c, _lib.ptr(idx), _lib.ptr(logit))
         return idx, logit
 
+    @_lib.on_device
+    def score_top_c(self, feats, frame_offsets, c=5, want_frame_lse=False):
+        """Top-C fast scoring (Reynolds, Quatieri & Dunn 2000) of a set from :meth:`with_ubm`, whose speakers are
+        MAP-adapted from the UBM in weights and variances as well as means: (scores (n_utts, n_models) cuda float64,
+        frame_lse (n_models, total) cuda float32 | None).  For every frame the C components the UBM (``ubm_index``) ranks
+        highest are selected (:meth:`top_components`), and every model is scored over those C components only:
+        ``log sum_{c in S_t} w_s,c N(x_t; mu_s,c, var_s,c)``, averaged over the frames of each utterance (0 for an empty
+        one).  With ``c = n_comp`` it is the exact score.  Always FP32 grade: FP32-grade selection logits, the difference
+        from the UBM as FP32 FMAs on frames centred on the UBM's component mean, double utterance sums.  A set without
+        ``ubm_index`` is a ``ValueError``, D > 39 a ``NotImplementedError``; neither launches anything."""
+        if self.ubm_index is None:
+            raise ValueError("top-C scoring selects under the UBM: build the set with ModelSet.with_ubm (ubm_index)")
+        return _score_top_c(self, feats, frame_offsets, c, want_frame_lse, self.lib.ssp_gmm_score_topc_adapted,
+                            "ssp_gmm_score_topc_adapted")
+
+    def _topc_tables(self):
+        """(the UBM as a one-model set (selection), the ``ssp_gmm_pack_topc_adapted`` table, the scoring's scratch), made
+        on first use and dropped by :meth:`repack`."""
+        torch = _lib.require_cuda()
+        if self._topc is None:
+            nbytes = int(self.lib.ssp_gmm_topc_adapted_pack_bytes(C.byref(self.dims)))
+            if nbytes <= 0:
+                raise NotImplementedError(f"top-C scoring takes D <= 39 (got D = {self.n_feat})")
+            w, mu, var = self._params
+            k = self.ubm_index
+            ref = ModelSet(w[k][None], mu[k][None], var[k][None], device=self.device)
+            pack = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+            _lib.check(self.lib.ssp_gmm_pack_topc_adapted(_lib.ptr(w), _lib.ptr(mu), _lib.ptr(var), C.byref(self.dims), k,
+                                                          _lib.ptr(pack), _lib.stream_ptr()), "ssp_gmm_pack_topc_adapted")
+            self._topc = (ref, pack, StatsWorkspace(self.device))
+        return self._topc
+
 
 # widest selection the top-C kernels keep per frame
 MAX_TOP_C = 64
@@ -267,6 +331,26 @@ def check_top_c(c, n_comp):
     if isinstance(c, bool) or not isinstance(c, (int, np.integer)) or not 1 <= int(c) <= min(n_comp, MAX_TOP_C):
         raise ValueError(f"top-C needs an integer C in [1, min(K = {n_comp}, {MAX_TOP_C})] (got {c!r})")
     return int(c)
+
+
+def _score_top_c(ms, feats, frame_offsets, c, want_frame_lse, score_fn, name):
+    """The top-C call of :class:`SharedModelSet` and :class:`ModelSet`: the selection under the set's UBM, then
+    ``score_fn`` (``ssp_gmm_score_topc`` / ``ssp_gmm_score_topc_adapted``) on the table of ``ms._topc_tables()``."""
+    torch = _lib.require_cuda()
+    d_off, n_utts, total = _upload_frames(ms, feats, frame_offsets)
+    c = check_top_c(c, ms.n_comp)
+    ref, pack, scratch = ms._topc_tables()
+    idx, logit = ref.top_components(feats, np.array([0, total], dtype=np.int64), c)
+    scores = torch.empty((n_utts, ms.n_models), dtype=torch.float64, device=ms.device)
+    lse = torch.empty((ms.n_models, total), dtype=torch.float32, device=ms.device) if want_frame_lse else None
+    ws_bytes = int(ms.lib.ssp_gmm_score_topc_workspace_bytes(C.byref(ms.dims), c, total))
+    ws = scratch.reserve(ws_bytes)
+    rc = score_fn(_lib.ptr(feats), _lib.ptr(d_off), n_utts, total, _lib.ptr(idx), _lib.ptr(logit), c, _lib.ptr(pack),
+                  C.byref(ms.dims), _lib.ptr(scores), _lib.ptr(lse), _lib.ptr(ws) if ws_bytes else None, ws_bytes,
+                  _lib.stream_ptr())
+    _lib.check(rc, name)
+    ms._keep = (d_off, idx, logit)
+    return scores, lse
 
 
 class StatsWorkspace:
@@ -370,30 +454,20 @@ class SharedModelSet:
         components only: ``log sum_{c in S_t} w_c N(x_t; mu_s,c, var_c)``, averaged over the frames of each utterance (0 for
         an empty one).  An approximation with its own definition: with ``c = n_comp`` it is the exact score.  Always FP32
         grade (FP32-grade selection logits, FP32 difference terms, double utterance sums)."""
+        return _score_top_c(self, feats, frame_offsets, c, want_frame_lse, self.lib.ssp_gmm_score_topc, "ssp_gmm_score_topc")
+
+    def _topc_tables(self):
+        """(the reference member as a one-model set (selection), the component-major (a, b) table (scoring), the
+        scoring's scratch), made on first use."""
         torch = _lib.require_cuda()
-        d_off, n_utts, total = _upload_frames(self, feats, frame_offsets)
-        c = check_top_c(c, self.n_comp)
-        w, var, mu = self._params
         if self._topc is None:
-            # the reference member as a one-model set (selection), the component-major (a, b) table (scoring) and the
-            # scoring's scratch
+            w, var, mu = self._params
             ref = ModelSet(w[None], mu[self.ref_model][None], var[None], device=self.device)
             pack = torch.empty(int(self.lib.ssp_gmm_topc_pack_bytes(C.byref(self.dims))), dtype=torch.uint8, device=self.device)
             _lib.check(self.lib.ssp_gmm_pack_topc(_lib.ptr(var), _lib.ptr(mu), C.byref(self.dims), self.ref_model,
                                                   _lib.ptr(pack), _lib.stream_ptr()), "ssp_gmm_pack_topc")
             self._topc = (ref, pack, StatsWorkspace(self.device))
-        ref, pack, scratch = self._topc
-        idx, logit = ref.top_components(feats, np.array([0, total], dtype=np.int64), c)
-        scores = torch.empty((n_utts, self.n_models), dtype=torch.float64, device=self.device)
-        lse = torch.empty((self.n_models, total), dtype=torch.float32, device=self.device) if want_frame_lse else None
-        ws_bytes = int(self.lib.ssp_gmm_score_topc_workspace_bytes(C.byref(self.dims), c, total))
-        ws = scratch.reserve(ws_bytes)
-        rc = self.lib.ssp_gmm_score_topc(_lib.ptr(feats), _lib.ptr(d_off), n_utts, total, _lib.ptr(idx), _lib.ptr(logit), c,
-                                         _lib.ptr(pack), C.byref(self.dims), _lib.ptr(scores), _lib.ptr(lse),
-                                         _lib.ptr(ws) if ws_bytes else None, ws_bytes, _lib.stream_ptr())
-        _lib.check(rc, "ssp_gmm_score_topc")
-        self._keep = (d_off, idx, logit)
-        return scores, lse
+        return self._topc
 
     def expand(self) -> "ModelSet":
         """The same models as a general :class:`ModelSet` (weights and variances replicated)."""

@@ -53,13 +53,19 @@ def map_adapt(ubm: GaussianMixture, speaker_frames, relevance: float = 16.0, ada
     return ow, omu, ovar
 
 
-def map_enrol(ubm: GaussianMixture, speaker_frames, relevance: float = 16.0, device=None) -> SharedModelSet:
-    """Mean-only MAP enrolment straight into the form the shared-variance scoring kernel wants: a
-    :class:`SharedModelSet` of the S adapted mean sets plus the UBM's own means as model S (``ubm_index``), all with the
-    UBM's weights and variances.  ``identify(utts, map_enrol(...))`` then gives the LLR matrix of GMM_UBM.py:191-197
-    with one kernel launch and a per-speaker contraction of D + 2 instead of 2D + 2."""
+def map_enrol(ubm: GaussianMixture, speaker_frames, relevance: float = 16.0, adapt=("means",), device=None):
+    """MAP enrolment straight into a model set that carries the UBM as model S (``ubm_index``).
+
+    The default, mean-only enrolment gives the form the shared-variance scoring kernel wants: a :class:`SharedModelSet`
+    of the S adapted mean sets plus the UBM's own means, all with the UBM's weights and variances.
+    ``identify(utts, map_enrol(...))`` then gives the LLR matrix of GMM_UBM.py:191-197 with one kernel launch and a
+    per-speaker contraction of D + 2 instead of 2D + 2.  An ``adapt`` that includes ``"weights"`` or ``"variances"``
+    gives ``ModelSet.with_ubm(*map_adapt(...), ubm)``: the general scoring kernel, and top-C scoring through
+    :meth:`ModelSet.score_top_c`."""
     torch = _lib.require_cuda()
     dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
+    if "weights" in adapt or "variances" in adapt:
+        return ModelSet.with_ubm(*map_adapt(ubm, speaker_frames, relevance=relevance, adapt=adapt, device=dev), ubm, device=dev)
     _, mu, _ = map_adapt(ubm, speaker_frames, relevance=relevance, adapt=("means",), device=dev)
     uw, umu, uvar = ubm._model_set()._params
     return SharedModelSet.with_ubm(uw[0], uvar[0], mu, umu, device=dev)
@@ -99,8 +105,12 @@ def _llr(scores, k):
 
 
 def _top_c_set(speakers, ubm, dev):
-    """(SharedModelSet whose reference member is the UBM, column of the UBM) for top-C scoring, or the refusal: no UBM is a
-    ``ValueError``, speakers that do not share the UBM's weights and variances a ``NotImplementedError``."""
+    """(set that selects by its UBM member, column of the UBM) for top-C scoring: a :class:`ModelSet` from
+    :meth:`ModelSet.with_ubm` (speakers adapted in weights and variances too) or a :class:`SharedModelSet` whose
+    reference member is the UBM; or the refusal: no UBM is a ``ValueError``, speakers that do not share the UBM's weights
+    and variances a ``NotImplementedError``."""
+    if isinstance(speakers, ModelSet) and speakers.ubm_index is not None and ubm is None:
+        return speakers, speakers.ubm_index
     if isinstance(speakers, SharedModelSet) and ubm is None:
         k = getattr(speakers, "ubm_index", None)
         if k is None:
@@ -130,8 +140,8 @@ def _top_c_set(speakers, ubm, dev):
 def _exact_set(speakers, ubm, precision, dev):
     """(model set that scores ``speakers`` exactly at ``precision``, column of the UBM in it or None -- then the UBM, if
     any, is scored on its own)."""
-    if isinstance(speakers, SharedModelSet) and getattr(speakers, "ubm_index", None) is not None and ubm is None:
-        return speakers, speakers.ubm_index   # map_enrol: the UBM rides along as one of the mean sets
+    if isinstance(speakers, (SharedModelSet, ModelSet)) and getattr(speakers, "ubm_index", None) is not None and ubm is None:
+        return speakers, speakers.ubm_index   # map_enrol / with_ubm: the UBM rides along as one of the models
     if isinstance(speakers, SharedModelSet):
         return (speakers if precision in ("tf32", "auto") else speakers.expand()), None
     if isinstance(speakers, ModelSet):
@@ -158,17 +168,21 @@ def identify(utts, speakers, ubm=None, precision="auto", device=None, top_c=None
     GaussianMixture-like, single-model :class:`ModelSet`, or None.  Returns ``(pred (N,S) float64 numpy, argmax (N,)
     int64)``; ``pred`` is always the LLR ``speaker score - UBM score`` when a UBM is given, whichever kernel serves the
     call.  The UBM term is constant per utterance, so decisions depend on the speaker scores only (SURVEY F9); it is
-    evaluated ONCE per utterance, not once per speaker.
+    evaluated ONCE per utterance, not once per speaker.  A set with a ``ubm_index`` (:func:`map_enrol`,
+    :meth:`ModelSet.with_ubm`) given without ``ubm`` carries its UBM: it is scored in the same launch as the speakers and
+    ``pred`` is the LLR against it.
 
     ``precision``: "auto" (default) keeps every LLR within 1e-3 absolute of float64: one TF32 pass for models of
     >= 512 components (mean-only MAP sets then go through the shared-variance kernel), three passes (FP32-grade) for
     smaller ones, FP32 CUDA cores for D > 39.  "tf32" forces the single pass, "tf32x2" / "tf32x3" / "fp32" the others.
 
     ``top_c``: None (default) scores exactly as above.  An integer C scores by top-C fast scoring
-    (:meth:`SharedModelSet.score_top_c`, Reynolds et al. 2000): every frame under every speaker over the C components the
-    UBM ranks highest for it, always at FP32 grade (``precision`` is ignored).  The speakers must share the UBM's weights
-    and variances: a :func:`map_enrol` set, or mean-only MAP models with a ``ubm`` of the same weights and variances
-    (``NotImplementedError`` otherwise); without a UBM it is a ``ValueError``.
+    (:meth:`SharedModelSet.score_top_c` / :meth:`ModelSet.score_top_c`, Reynolds et al. 2000): every frame under every
+    speaker over the C components the UBM ranks highest for it, always at FP32 grade (``precision`` is ignored).  The
+    speakers must be known to be adapted from the UBM: a :func:`map_enrol` set (any ``adapt``), a
+    :meth:`ModelSet.with_ubm` set, or mean-only MAP models with a ``ubm`` of the same weights and variances
+    (``NotImplementedError`` otherwise: a list of models whose weights or variances differ from the UBM's may have been
+    trained independently, and then there is no component correspondence); without a UBM it is a ``ValueError``.
     """
     torch = _lib.require_cuda()
     dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
@@ -180,8 +194,9 @@ def identify(utts, speakers, ubm=None, precision="auto", device=None, top_c=None
             return _llr(sms.score_top_c(feats, offs, c=top_c)[0], k)
         feats, offs = concat_utterances(utts, dev)
         ms, k = _exact_set(speakers, ubm, precision, dev)
-        if k is not None:   # one launch scores speakers and UBM
-            return _llr(ms.score(feats, offs)[0], k)
+        if k is not None:   # one launch scores speakers and UBM (a SharedModelSet has its one precision rung)
+            scores, _ = ms.score(feats, offs) if isinstance(ms, SharedModelSet) else ms.score(feats, offs, precision=precision)
+            return _llr(scores, k)
         scores, _ = ms.score(feats, offs, precision=precision)
         if ubm is not None:
             ums = ubm if isinstance(ubm, ModelSet) else ModelSet(ubm.weights_, ubm.means_, ubm.covariances_, device=dev)
@@ -225,17 +240,20 @@ def identify_pcm(host_pcm, sample_offsets, front_end, speakers, ubm_index=None, 
     the argmax), or None.  The host-to-device copy is cut in two at an utterance boundary: the head (about a tenth of
     the frames, whole scoring waves) is copied on the current stream and goes straight into the front-end and scoring
     kernels while a side stream copies the rest, so all but the head's transfer is hidden behind compute.
-    ``top_c``: None scores exactly; an integer C scores by top-C fast scoring (:meth:`SharedModelSet.score_top_c`,
-    ``precision`` ignored), which needs a :class:`SharedModelSet` whose reference member is the UBM and ``ubm_index``
-    naming it (a :func:`map_enrol` set and its ``ubm_index``).
+    ``top_c``: None scores exactly; an integer C scores by top-C fast scoring (:meth:`SharedModelSet.score_top_c` /
+    :meth:`ModelSet.score_top_c`, ``precision`` ignored), which needs ``ubm_index`` to name the set's UBM: the reference
+    member of a :class:`SharedModelSet`, or the ``ubm_index`` of a :class:`ModelSet` (a :func:`map_enrol` set and its
+    ``ubm_index``, whatever it adapted).
     Returns ``(decisions (N,) int64 host tensor, total_frames)``; the call returns after the decisions have landed."""
     torch = _lib.require_cuda()
     dev = front_end.device
     if top_c is not None:
         if ubm_index is None:
             raise ValueError("top_c scores against a UBM: pass ubm_index")
-        if not isinstance(speakers, SharedModelSet) or int(ubm_index) % speakers.n_models != speakers.ref_model:
-            raise NotImplementedError("top_c needs a SharedModelSet whose reference member is the UBM (ubm_index)")
+        ubm_member = speakers.ref_model if isinstance(speakers, SharedModelSet) else getattr(speakers, "ubm_index", None)
+        if ubm_member is None or int(ubm_index) % speakers.n_models != ubm_member:
+            raise NotImplementedError("top_c needs a SharedModelSet whose reference member is the UBM, or a ModelSet whose "
+                                      "ubm_index is the UBM (ubm_index)")
         check_top_c(top_c, speakers.n_comp)
     if isinstance(host_pcm, np.ndarray):
         host_pcm = torch.from_numpy(np.ascontiguousarray(host_pcm))
